@@ -1,7 +1,7 @@
 """ORACLE (test infrastructure): expose the CPU restatement under the module names the
-reference imports (icocnn.ico_conv, icocnn.utils.ico_geometry, mesh.utils) so that
-/root/reference/models.py and losses.py can be imported UNCHANGED on top of it
-(only possible in the build container; /root/reference does not travel to the GPU box).
+reference imports (icocnn.ico_conv, icocnn.utils.ico_geometry, mesh.utils) so that the
+original project's models.py and losses.py can be imported UNCHANGED on top of it
+(only where a checkout of it is given by the environment variable GENICONET_REFERENCE).
 """
 import importlib
 import sys
@@ -33,10 +33,13 @@ def restore_modules(saved):
             sys.modules[k] = v
 
 
-def import_reference(name, ref_root='/root/reference'):
-    """Import /root/reference/<name>.py (models / losses) over the oracle modules."""
+def import_reference(name, ref_root=None):
+    """Import <ref_root>/<name>.py (models / losses; default root: $GENICONET_REFERENCE) over the oracle modules."""
     import importlib.util
     import os
+    ref_root = ref_root or os.environ.get('GENICONET_REFERENCE')
+    if not ref_root:
+        raise RuntimeError('import_reference: no checkout of the original project given (ref_root or GENICONET_REFERENCE)')
     path = os.path.join(ref_root, name + '.py')
     if not os.path.exists(path):
         raise FileNotFoundError(path)

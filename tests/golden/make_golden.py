@@ -1,11 +1,11 @@
-"""Generates tests/golden/*.json.  Run in the BUILD container only (needs /root/reference):
+"""Generates tests/golden/*.json from a checkout of the original GenIcoNet project:
 
-    python tests/golden/make_golden.py
+    GENICONET_REFERENCE=<checkout> python tests/golden/make_golden.py
 
 The reference's own models.py and losses.py are imported UNCHANGED on top of the oracle's icocnn / mesh
 modules (oracle/install.py); weights are the name-keyed deterministic fill of tests/oracle_models.py, inputs come
 from seeded CPU generators.  The stored numbers therefore pin "reference graph + reference loss code over the
-oracle layers"; the GPU tests reproduce them through the CUDA path without needing /root/reference.
+oracle layers"; the GPU tests reproduce them through the CUDA path without needing the checkout.
 """
 import json
 import os
@@ -43,7 +43,7 @@ def params_for(name):
 
 
 def build():
-    """The fixture as a dict (needs /root/reference)."""
+    """The fixture as a dict (needs GENICONET_REFERENCE)."""
     torch.set_num_threads(8)
     models = import_reference('models')
     saved = install_oracle_modules()

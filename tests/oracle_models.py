@@ -1,5 +1,5 @@
-"""Test tool: the ico2ico / ico2ico_vae graphs over the ORACLE layers (CPU), so model-level parity can be checked on the GPU
-box where /root/reference does not exist.  A thin adapter over oracle/models_ref.py: nothing here imports the product
+"""Test tool: the ico2ico / ico2ico_vae graphs over the ORACLE layers (CPU), so model-level parity can be checked without
+a checkout of the original project.  A thin adapter over oracle/models_ref.py: nothing here imports the product
 package (the CPU arm of bench.py runs through this file and must not load libgeniconet_b200.so)."""
 from oracle import models_ref
 

@@ -1,5 +1,6 @@
-"""Test infrastructure: import modules of the reference checkout (/root/reference, build container only) UNCHANGED, with
-stand-ins for the third-party packages that are absent here.  Nothing under geniconet_b200/ imports this.
+"""Test infrastructure: import modules of a checkout of the original GenIcoNet project UNCHANGED, with stand-ins for its
+third-party packages.  The checkout is not part of this repository: the tests that need it run when the environment variable
+GENICONET_REFERENCE names its directory and skip otherwise.  Nothing under geniconet_b200/ imports this.
 
 Stand-ins (each only as far as the imported reference code touches it):
   natsort.natsorted      digit runs compare as integers (natsort's default algorithm), written independently of
@@ -15,11 +16,12 @@ import re
 import sys
 import types
 
-REF_ROOT = '/root/reference'
+REF_ROOT = os.environ.get('GENICONET_REFERENCE', '')
+SKIP_REASON = 'needs a checkout of the original GenIcoNet project (GENICONET_REFERENCE)'
 
 
 def available():
-    return os.path.isdir(REF_ROOT)
+    return bool(REF_ROOT) and os.path.isdir(REF_ROOT)
 
 
 def _natsorted(seq, key=None):

@@ -5,6 +5,8 @@ import os
 import subprocess
 import sys
 
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -47,7 +49,62 @@ def test_reference_arm_other_ranks_exit_quietly():
 def test_our_arm_has_no_cpu_path():
     import torch
     if torch.cuda.is_available():
-        import pytest
         pytest.skip('a CUDA device is present')
     r = _run(['--steps', '1', '--warmup', '1', '--no-cpu-baseline'])
     assert r.returncode != 0 and 'no CUDA device' in (r.stderr + r.stdout)
+
+
+def test_steps_must_be_positive():
+    r = _run(['--steps', '0', '--no-cpu-baseline'])
+    assert r.returncode != 0 and '--steps must be at least 1' in r.stderr
+    r = _run(['--impl', 'reference', '--dump-outputs', 'unused'])
+    assert r.returncode != 0 and '--dump-outputs' in r.stderr
+
+
+def test_reference_arm_times_the_requested_steps():
+    r = _run(['--impl', 'reference', '--cpu-batch', '1', '--level', '3', '--steps', '6', '--warmup', '2'])
+    assert r.returncode == 0, r.stderr[-2000:]
+    d = json.loads(r.stdout.strip().splitlines()[-1])
+    assert d['steps'] == 6 and d['warmup'] == 2
+
+
+def _dump(tmp_path, tag, *extra):
+    import numpy as np
+    out = tmp_path / tag
+    r = _run(['--steps', '3', '--warmup', '1', '--no-cpu-baseline', '--no-kernel-table', '--dump-outputs', str(out)] + list(extra))
+    assert r.returncode == 0, r.stderr[-2000:]
+    assert json.loads(r.stdout.strip().splitlines()[-1])['steps'] == 3
+    assert sum(f.stat().st_size for f in out.iterdir()) <= (64 << 20) + 256 * len(list(out.iterdir()))     # + .npy headers
+    return {f.name[:-4]: np.load(f) for f in out.iterdir()}
+
+
+@pytest.mark.gpu
+def test_dump_outputs_holds_the_last_timed_step(tmp_path):
+    """--dump-outputs: inputs, loss, output, parameters and gradients of the last timed step as float32 .npy files; two runs with
+    the same arguments dump the same inputs and (up to reordered float sums) the same results."""
+    import numpy as np
+    from geniconet_b200 import models as gm
+    a, b = _dump(tmp_path, 'a'), _dump(tmp_path, 'b')
+    assert sorted(a) == sorted(b) and all(v.dtype == np.float32 and np.isfinite(v).all() for v in a.values())
+    names = [n for n, _ in gm.ico2ico(gm.default_params('ico2ico')).named_parameters()]
+    assert sorted(k for k in a if k.startswith('param.')) == sorted('param.' + n for n in names)
+    assert sorted(k for k in a if k.startswith('grad.')) == sorted('grad.' + n for n in names)
+    assert a['loss'].shape == (1,) and a['output'].shape == (36, 3, 160, 64) and a['input.x'].shape == (36, 3, 160, 64)
+    assert np.abs(a['grad.encoder.0.weight']).max() > 0
+    for k in ('input.x', 'input.target'):
+        assert np.array_equal(a[k], b[k]), k
+    for k in a:
+        assert np.allclose(a[k], b[k], rtol=1e-4, atol=1e-6 * max(1.0, float(np.abs(a[k]).max()))), k
+
+
+@pytest.mark.gpu
+def test_dump_outputs_samples_large_arrays(tmp_path):
+    """ico2ico_vae at batch 72: the arrays exceed the 64 MB budget, so the reconstruction and the input are stored as seeded samples."""
+    v = _dump(tmp_path, 'vae', '--model', 'ico2ico_vae', '--batch', '72')
+    assert {'loss', 'output', 'mu', 'logvar', 'input.x', 'input.target'} <= set(v)
+    # the reconstruction (72 x 3 x 160 x 64) is above every cap the budget allows: it is sampled down to the cap, and no array is
+    # larger than that cap; the input has the same size, so it is sampled to the same number of elements
+    cap = v['output'].size
+    assert v['output'].ndim == 1 and cap < 72 * 3 * 160 * 64
+    assert v['input.x'].ndim == 1 and v['input.x'].size == cap
+    assert all(a.size <= cap for a in v.values()) and v['mu'].size == v['logvar'].size

@@ -1,82 +1,64 @@
-"""The data / checkpoint / helper mirrors (geniconet_b200/data.py, checkpoint.py, ico_utils.py) against the reference's OWN code:
-/root/reference/data.py, run.py and ico_utils.py imported unchanged (tests/reference_imports.py supplies stand-ins for the absent
-third-party packages).  Build container only: /root/reference does not travel to the GPU box."""
-import copy
+"""The data / checkpoint / helper mirrors (geniconet_b200/data.py, checkpoint.py, ico_utils.py) against what the original
+project's own data.py, run.py, ico_utils.py and generate.py return on the same seeded inputs, stored in
+tests/golden/reference_vectors.json (tests/golden/make_reference_vectors.py)."""
+import json
 import os
 
 import numpy as np
 import pytest
 import torch
 
-import reference_imports as ri
 from geniconet_b200 import checkpoint as ck
 from geniconet_b200 import data as gd
-from geniconet_b200 import ico_utils as iu
 from geniconet_b200 import models as gm
+from golden.make_reference_vectors import BEST_LOSSES, NORMALS_LEVEL, NORMALS_SAMPLE, POLE_SEED, digest
 from test_datapath import LEVEL, N, P, _make_modelnet, _params
 
-pytestmark = pytest.mark.skipif(not ri.available(), reason='the reference checkout exists only in the build container')
-
-
-def _same(a, b):
-    if isinstance(a, (tuple, list)):
-        return len(a) == len(b) and all(_same(u, v) for u, v in zip(a, b))
-    if isinstance(a, np.ndarray) or isinstance(b, np.ndarray):
-        return np.array_equal(np.asarray(a), np.asarray(b))
-    if isinstance(a, torch.Tensor):
-        return torch.equal(a, b)
-    return a == b
+GOLD = json.load(open(os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden', 'reference_vectors.json')))
 
 
 def test_datasets_match_reference_data_py(tmp_path):
     root = str(tmp_path)
     _make_modelnet(root)                                   # chair/bed x train/test, names that need natural ordering
-    with ri.reference_modules('data') as rd:
-        for process in ('train', 'test'):
-            params = _params(root, process=process)
-            for inst in ('trn', 'val'):
-                assert gd.listFiles(params, 'ico', inst) == rd.listFiles(params, 'ico', inst)
-            f0 = gd.listFiles(params, 'ico', 'trn')[0]
-            assert _same(gd.loadIcoFile(params, f0), rd.loadIcoFile(params, f0))
-            for cls in ('createico2icoDataset', 'createico2ico_vaeDataset'):
-                ours, ref = getattr(gd, cls)(params, 'val'), getattr(rd, cls)(copy.deepcopy(params), 'val')
-                assert len(ours) == len(ref) == 6
-                for i in range(len(ours)):
-                    assert _same(ours[i], ref[i]), (cls, process, i)
-        # encodings: written through the reference's save_to_file convention ('arr_0'), read back by both
-        params = _params(root, process='test')
-        enc_ours, enc_ref = gd.createico2encDataset(params, 'val'), rd.createico2encDataset(copy.deepcopy(params), 'val')
-        assert len(enc_ours) == len(enc_ref)
-        for i in range(len(enc_ours)):
-            assert _same(enc_ours[i], enc_ref[i])
-            np.savez_compressed(enc_ours[i][1], np.full((2, 3), float(i), dtype=np.float32))
-        assert _same(gd.loadEncFile(params, enc_ours[2][1]), rd.loadEncFile(params, enc_ours[2][1]))
-        flat = dict(params, ico=dict(params['ico'], dataPthLvl=1, dataPth=os.path.join(root, 'ico', 'chair', 'test')),
-                    enc=dict(params['enc'], dataPth=params['enc']['dataPth']))
-        dec_ours, dec_ref = gd.createenc2icoDataset(flat, 'val'), rd.createenc2ico_vaeDataset(copy.deepcopy(flat), 'val')
-        assert len(dec_ours) == len(dec_ref) and len(dec_ours) >= 1
-        for i in range(len(dec_ours)):
-            assert _same(dec_ours[i], dec_ref[i])
-        with pytest.raises(ValueError):
-            rd.loadEncFile(params, 'x.bin')
-        with pytest.raises(ValueError):
-            gd.loadEncFile(params, 'x.bin')
+    want = GOLD['data']
+    for process in ('train', 'test'):
+        params = _params(root, process=process)
+        for inst in ('trn', 'val'):
+            assert digest(gd.listFiles(params, 'ico', inst), root) == want[process]['listFiles'][inst]
+        f0 = gd.listFiles(params, 'ico', 'trn')[0]
+        assert digest(gd.loadIcoFile(params, f0), root) == want[process]['loadIcoFile']
+        for cls in ('createico2icoDataset', 'createico2ico_vaeDataset'):
+            ours = getattr(gd, cls)(params, 'val')
+            assert len(ours) == len(want[process][cls]) == 6
+            for i in range(len(ours)):
+                assert digest(ours[i], root) == want[process][cls][i], (cls, process, i)
+    # encodings: written with the original's save_to_file convention ('arr_0'), read back
+    params = _params(root, process='test')
+    enc = gd.createico2encDataset(params, 'val')
+    assert [digest(enc[i], root) for i in range(len(enc))] == want['createico2encDataset']
+    for i in range(len(enc)):
+        np.savez_compressed(enc[i][1], np.full((2, 3), float(i), dtype=np.float32))
+    assert digest(gd.loadEncFile(params, enc[2][1]), root) == want['loadEncFile']
+    flat = dict(params, ico=dict(params['ico'], dataPthLvl=1, dataPth=os.path.join(root, 'ico', 'chair', 'test')))
+    dec = gd.createenc2icoDataset(flat, 'val')
+    assert len(dec) >= 1 and [digest(dec[i], root) for i in range(len(dec))] == want['createenc2ico_vaeDataset']
+    with pytest.raises(ValueError):
+        gd.loadEncFile(params, 'x.bin')
 
 
 def test_pole_rule_matches_reference_ico_utils():
-    with ri.reference_modules('ico_utils') as ru:
-        # the reference's pole rule on the CPU (ico_utils.py:10-24) against the plan the CUDA kernel walks (gin_pole_vertices_fwd)
-        from geniconet_b200 import _lib
-        g = torch.Generator().manual_seed(0)
-        x = torch.randn(2, 3, 5 * N, 2 * N, generator=g)
-        v_ref = ru.output2vertices(LEVEL, x)
-        blob = _lib.plan_blob(_lib.PLAN_LOSS, LEVEL)
-        assert int(blob[3]) == P and int(blob[4]) == P + 2                       # GinLossPlanHdr: magic, kind, level, P, V, total, ring, pole, flag
-        ring = np.asarray(blob[int(blob[7]):int(blob[7]) + 10]).reshape(2, 5)    # pole_off: the five pixels averaged into each pole
-        flat = x.reshape(2, 3, -1)
-        assert torch.equal(v_ref[:, :P], flat.transpose(1, 2))
-        for pole in (0, 1):
-            assert torch.allclose(v_ref[:, P + pole], flat[:, :, torch.as_tensor(ring[pole]).long()].mean(-1), atol=1e-7)
+    # the original's pole rule (ico_utils.py:10-24) on the CPU against the plan the CUDA kernel walks (gin_pole_vertices_fwd)
+    from geniconet_b200 import _lib
+    x = torch.randn(2, 3, 5 * N, 2 * N, generator=torch.Generator().manual_seed(POLE_SEED))
+    v_ref = torch.tensor(GOLD['pole']['vertices'])
+    blob = _lib.plan_blob(_lib.PLAN_LOSS, LEVEL)
+    assert int(blob[3]) == P and int(blob[4]) == P + 2                       # GinLossPlanHdr: magic, kind, level, P, V, total, ring, pole, flag
+    ring = np.asarray(blob[int(blob[7]):int(blob[7]) + 10]).reshape(2, 5)    # pole_off: the five pixels averaged into each pole
+    flat = x.reshape(2, 3, -1)
+    assert tuple(v_ref.shape) == (2, P + 2, 3)
+    assert torch.equal(v_ref[:, :P], flat.transpose(1, 2))
+    for pole in (0, 1):
+        assert torch.allclose(v_ref[:, P + pole], flat[:, :, torch.as_tensor(ring[pole]).long()].mean(-1), atol=1e-7)
 
 
 def _model(seed):
@@ -85,57 +67,47 @@ def _model(seed):
 
 
 def test_checkpoints_interoperate_with_reference_run_py(tmp_path):
-    with ri.reference_modules('run') as rr:
-        # 1. written by the reference's saveModel, read by ours
-        p_ref = _params(str(tmp_path / 'a'))
-        m0 = _model(0)
-        opt0 = torch.optim.Adam(m0.parameters(), lr=1e-3)
-        rr.saveModel(p_ref, m0, opt0, 'B4', 'ico2ico', 0.25, {'k': 1})
-        m1 = _model(1)
-        epoch, best, misc = [0], [np.inf], []
-        assert ck.loadModel(p_ref, m1, epoch, 'ico2ico', torch.optim.Adam(m1.parameters(), lr=1e-3), best, misc) is True
-        assert epoch == [4] and best == [0.25] and misc == [{'k': 1}]
-        assert all(torch.equal(a, b) for a, b in zip(m0.state_dict().values(), m1.state_dict().values()))
-        # 2. written by ours, read by the reference's loadModel (same files, same dict keys)
-        p_our = _params(str(tmp_path / 'b'))
-        ck.saveModel(p_our, m0, opt0, 'B9', 'ico2ico', 0.5, None)
-        m2 = _model(2)
-        epoch, best, misc = [0], [np.inf], []
-        assert rr.loadModel(p_our, m2, epoch, 'ico2ico', torch.optim.Adam(m2.parameters(), lr=1e-3), best, misc) is True
-        assert epoch == [9] and best == [0.5] and misc == [None]
-        assert all(torch.equal(a, b) for a, b in zip(m0.state_dict().values(), m2.state_dict().values()))
-        assert p_our['out']['dataPth'].endswith('out_EB9')
-        # 3. the same sequence of validation losses leaves the same files behind (best-model rotation, run.py:317-328)
-        pa, pb = _params(str(tmp_path / 'c')), _params(str(tmp_path / 'd'))
-        ba, bb = [np.inf], [np.inf]
-        for e, loss in enumerate([1.0, 0.9, 0.95, 0.8, 0.7, 0.6, 0.65, 0.5, 0.4, 0.3], start=1):
-            rr.saveBestModel(pa, m0, opt0, e, 'ico2ico', ba, [loss])
-            ck.saveBestModel(pb, m0, opt0, e, 'ico2ico', bb, [loss])
-        la = sorted(os.listdir(os.path.join(pa['logDir'], 'savedModel')))
-        lb = sorted(os.listdir(os.path.join(pb['logDir'], 'savedModel')))
-        assert la == lb and ba == bb and len(la) == 6
-        # 4. no file: both say False; loadMultiModel: both raise on a missing file, both fill from two checkpoints
-        assert rr.loadModel(_params(str(tmp_path / 'e')), m2, [3], 'ico2ico') is False
-        assert ck.loadModel(_params(str(tmp_path / 'e')), m2, [3], 'ico2ico') is False
-        ck.saveModel(p_our, _model(5), opt0, 2, 'other', 0.0, None)
-        ma, mb = _model(6), _model(7)
-        assert rr.loadMultiModel(p_our, ma, ['B9', 2], ['ico2ico', 'other']) and ck.loadMultiModel(p_our, mb, ['B9', 2], ['ico2ico', 'other'])
-        assert all(torch.equal(a, b) for a, b in zip(ma.state_dict().values(), mb.state_dict().values()))
-        for fn in (rr.loadMultiModel, ck.loadMultiModel):
-            with pytest.raises(ValueError):
-                fn(p_our, ma, [77], ['ico2ico'])
+    want = GOLD['checkpoint']
+    # 1. the files and dict keys the original's saveModel writes, and their values
+    p = _params(str(tmp_path / 'a'))
+    m0 = _model(0)
+    opt0 = torch.optim.Adam(m0.parameters(), lr=1e-3)
+    ck.saveModel(p, m0, opt0, 'B4', 'ico2ico', 0.25, {'k': 1})
+    files = sorted(os.path.relpath(os.path.join(d, f), p['logDir']) for d, _, fs in os.walk(p['logDir']) for f in fs)
+    assert files == want['saveModel_files']
+    saved = torch.load(os.path.join(p['logDir'], files[0]), weights_only=False)
+    assert sorted(saved) == want['saveModel_keys'] and {k: saved[k] for k in ('epoch', 'loss', 'misc')} == want['saveModel_values']
+    # 2. a file with exactly those keys and values (what the original writes) loads into ours
+    m1 = _model(1)
+    epoch, best, misc = [0], [np.inf], []
+    assert ck.loadModel(p, m1, epoch, 'ico2ico', torch.optim.Adam(m1.parameters(), lr=1e-3), best, misc) is True
+    assert epoch == [4] and best == [0.25] and misc == [{'k': 1}]
+    assert all(torch.equal(a, b) for a, b in zip(m0.state_dict().values(), m1.state_dict().values()))
+    assert os.path.basename(p['out']['dataPth']) == want['out_dataPth']
+    # 3. the same sequence of validation losses leaves the same files behind (best-model rotation, run.py:317-328)
+    pb, bb = _params(str(tmp_path / 'd')), [np.inf]
+    for e, loss in enumerate(BEST_LOSSES, start=1):
+        ck.saveBestModel(pb, m0, opt0, e, 'ico2ico', bb, [loss])
+    assert sorted(os.listdir(os.path.join(pb['logDir'], 'savedModel'))) == want['best_files'] and bb == [want['best_loss']]
+    # 4. no file: False; loadMultiModel: raises on a missing file, fills from two checkpoints
+    assert ck.loadModel(_params(str(tmp_path / 'e')), m1, [3], 'ico2ico') is False
+    ck.saveModel(p, _model(5), opt0, 2, 'other', 0.0, None)
+    ma = _model(6)
+    assert ck.loadMultiModel(p, ma, ['B4', 2], ['ico2ico', 'other'])
+    with pytest.raises(ValueError):
+        ck.loadMultiModel(p, ma, [77], ['ico2ico'])
 
 
 def test_target_normals_against_reference_generate_py():
     """generate.py:20-43 mesh_vertexnormals made the dataset's normal targets.  Its fancy-index `+=` keeps one face per corner slot
-    (numpy does not accumulate repeated indices), which data.vertex_normals(reference_semantics=True) reproduces exactly; the
+    (numpy does not accumulate repeated indices), which data.vertex_normals(reference_semantics=True) reproduces; the
     default (true area-weighted accumulation, what the loss kernels compute for the OUTPUT mesh) differs measurably."""
-    verts = gd.synthetic_mesh(3, 5)[1][:3].T.numpy().astype(np.float64)
-    faces = gd._topology(3)[1]
-    with ri.reference_modules('generate') as rg:
-        n_ref = rg.mesh_vertexnormals(verts, faces)
-        c_ref, s_ref = rg.get_normalize_unitsphere(verts)
-    assert np.array_equal(gd.vertex_normals(verts, faces, reference_semantics=True), n_ref)
+    want = GOLD['normals']
+    verts = gd.synthetic_mesh(NORMALS_LEVEL, NORMALS_SAMPLE)[1][:3].T.numpy().astype(np.float64)
+    faces = gd._topology(NORMALS_LEVEL)[1]
+    n_ref, c_ref, s_ref = np.asarray(want['normals']), np.asarray(want['center']), want['scale']
+    assert n_ref.shape == (10 * 4 ** NORMALS_LEVEL + 2, 3)
+    assert np.allclose(gd.vertex_normals(verts, faces, reference_semantics=True), n_ref, rtol=0, atol=1e-12)
     n_true = gd.vertex_normals(verts, faces)
     angle = np.degrees(np.arccos(np.clip((n_ref * n_true).sum(1), -1.0, 1.0)))
     assert 0.5 < angle.mean() < 10.0 and np.allclose(np.linalg.norm(n_true, axis=1), 1.0)

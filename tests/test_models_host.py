@@ -8,6 +8,7 @@ import pytest
 import torch
 
 import oracle_models as om
+import reference_imports as ri
 from geniconet_b200 import models as gm
 
 HERE = os.path.dirname(os.path.abspath(__file__))
@@ -71,8 +72,15 @@ def test_our_graph_over_oracle_reproduces_reference_golden():
     loss.backward()
     assert abs(loss.item() - g['loss']) <= 1e-5 * abs(g['loss'])
     assert torch.allclose(_sample(y), torch.tensor(g['output_sample']), rtol=1e-4, atol=1e-5)
+    # a conv bias ahead of a BatchNorm has a gradient that is mathematically zero: its stored norm (<= 2e-7 of the largest) is
+    # summation noise that changes with the host's CPU and thread count, so it is held below the noise level, not matched
+    noise = 1e-5 * max(g['grad_norms'].values())
     for k, p in m.named_parameters():
-        assert abs(p.grad.norm().item() - g['grad_norms'][k]) <= 1e-3 * g['grad_norms'][k] + 1e-9, k
+        want, got = g['grad_norms'][k], p.grad.norm().item()
+        if want < noise:
+            assert got < noise, k
+        else:
+            assert abs(got - want) <= 1e-3 * want + 1e-9, k
     for a, b in zip(parts, g['last_losses'][:3]):
         assert abs(a.item() - b) <= 1e-5 * max(1.0, abs(b))
 
@@ -114,8 +122,8 @@ def test_reference_files_import_over_the_shim_packages():
     from geniconet_b200.ico_conv import IcoConvS2S
     assert icocnn.ico_conv.IcoConvS2S is IcoConvS2S
     assert ig.get_ico_faces(5).max() + 1 == 10242 and ig.get_ico_faces(5).shape == (20480, 3)
-    ref_models = '/root/reference/models.py'
-    if os.path.exists(ref_models):                       # build container only
+    ref_models = os.path.join(ri.REF_ROOT, 'models.py')
+    if ri.available():                                   # with a checkout of the original project only
         import importlib.util
         spec = importlib.util.spec_from_file_location('_ref_models_over_product', ref_models)
         mod = importlib.util.module_from_spec(spec)
@@ -127,28 +135,29 @@ def test_reference_files_import_over_the_shim_packages():
 
 
 def test_reference_losses_construct_over_the_mesh_shim():
-    """The reference's UNMODIFIED losses.py over the product's `icocnn` / `mesh` shim packages: losses.py:39-40 registers the
-    adjacency matrix as a buffer, so compute_adjacency_matrix_sparse must hand back a real tensor (build container only)."""
-    ref_losses = '/root/reference/losses.py'
-    if not os.path.exists(ref_losses):
-        pytest.skip('needs /root/reference')
-    import importlib.util
-    import mesh.utils                                     # noqa: F401  (the product shim, not the oracle)
-    spec = importlib.util.spec_from_file_location('_ref_losses_over_product', ref_losses)
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)
+    """The original losses.py over the product's `icocnn` / `mesh` shim packages: losses.py:39-40 registers
+    compute_adjacency_matrix_sparse(get_ico_faces(5)) as a buffer, so the shim must hand back a real sparse tensor with the shape and
+    non-zeros the original's buffer has (tests/golden/reference_vectors.json)."""
+    import mesh.utils as shim                             # the product shim, not the oracle
+    import icocnn.utils.ico_geometry as ig
     import geniconet_b200.mesh_utils as mu
-    assert mod.compute_vertex_normals is mu.compute_vertex_normals and mod.compute_laplacian_batch is mu.compute_laplacian_batch
-    for crit in (mod.P2P_Loss(5, 1., 0., 0.), mod.P2PKLD_Loss(5, 0.6, 0.2, 0.2, 1.0)):
-        adj = dict(crit.named_buffers())['adj_mat']
-        assert adj.is_sparse and tuple(adj.shape) == (10242, 10242) and adj._nnz() == 2 * 30 * 4 ** 5      # one entry per directed edge
-        assert tuple(crit.ico_faces.shape) == (20480, 3)
-        crit.to('cpu')                                    # run.py:456 moves the criterion with .to(device)
-        # no CPU path: the forward must refuse rather than fall back
-        x = torch.zeros(1, 3, 160, 64)
-        t = torch.zeros(1, 9, 10242)
-        with pytest.raises(RuntimeError):
-            crit((x, x, x), t) if isinstance(crit, mod.P2PKLD_Loss) else crit(x, t)
+    from geniconet_b200 import losses
+    want = json.load(open(os.path.join(HERE, 'golden', 'reference_vectors.json')))['adjacency']
+    assert shim.compute_vertex_normals is mu.compute_vertex_normals and shim.compute_laplacian_batch is mu.compute_laplacian_batch
+    faces = torch.from_numpy(ig.get_ico_faces(5))
+    holder = torch.nn.Module()
+    holder.register_buffer('adj_mat', shim.compute_adjacency_matrix_sparse(int(faces.max()) + 1, faces))
+    holder.to('cpu')                                      # run.py:456 moves the criterion with .to(device)
+    adj = dict(holder.named_buffers())['adj_mat']
+    assert adj.is_sparse and list(adj.shape) == want['shape'] and adj._nnz() == want['nnz'] == 2 * 30 * 4 ** 5   # one entry per directed edge
+    assert list(faces.shape) == want['faces_shape']
+    # no CPU path: the forward must refuse rather than fall back
+    x = torch.zeros(1, 3, 160, 64)
+    t = torch.zeros(1, 9, 10242)
+    with pytest.raises(RuntimeError):
+        losses.P2P_Loss(5, 1., 0., 0.)(x, t)
+    with pytest.raises(RuntimeError):
+        losses.P2PKLD_Loss(5, 0.6, 0.2, 0.2, 1.0)((x, x, x), t)
     from oracle import mesh_ref, ico_geometry_ref as geo
     want = mesh_ref.compute_adjacency_matrix_sparse(642, torch.from_numpy(geo.get_ico_faces(3)))
     got = mu.compute_adjacency_matrix_sparse(642, torch.from_numpy(geo.get_ico_faces(3)))
@@ -183,7 +192,7 @@ def test_synthetic_data_contract():
     assert torch.equal(x, x2)
 
 
-@pytest.mark.skipif(not os.path.isdir('/root/reference'), reason='the reference checkout exists only in the build container')
+@pytest.mark.skipif(not ri.available(), reason=ri.SKIP_REASON)
 def test_golden_fixture_regenerates_from_the_reference():
     """tests/golden/make_golden.py (the reference's own models.py / losses.py imported unchanged over the oracle) still produces the
     committed fixture: every number within fp32 summation-order noise (gradients that are mathematically zero are pure noise)."""
@@ -213,19 +222,19 @@ def test_golden_fixture_regenerates_from_the_reference():
     compare(GOLD, fresh, '')
 
 
-@pytest.mark.skipif(not os.path.isdir('/root/reference'), reason='the reference checkout exists only in the build container')
 @pytest.mark.parametrize('name', ['ico2ico', 'ico2enc', 'enc2ico', 'ico2ico_vae', 'ico2enc_vae', 'enc2ico_vae'])
 def test_every_model_class_has_the_reference_state_dict(name):
-    """All six model classes of the reference's models.py (imported unchanged over the oracle layers), including the encoder-only
-    and decoder-only splits the app uses (models.py:234-252,302-340): same state-dict keys in the same order, same shapes."""
-    from oracle.install import import_reference
-    ref_models = import_reference('models')
+    """All six model classes of the original models.py, including the encoder-only and decoder-only splits the app uses
+    (models.py:234-252,302-340): same state-dict keys in the same order, same shapes (tests/golden/*.json)."""
     base = 'ico2ico_vae' if name.endswith('_vae') else 'ico2ico'
     params = gm.default_params(base)
     params['model_name'] = name
     params[name] = dict(params[base])
-    ref = getattr(ref_models, name)(params)
     ours = getattr(gm, name)(params)
-    want = [(k, tuple(v.shape)) for k, v in ref.state_dict().items()]
+    if name in GOLD:
+        want = [(k, tuple(v)) for k, v in GOLD[name]['state_dict'].items()]
+    else:
+        split = json.load(open(os.path.join(HERE, 'golden', 'reference_vectors.json')))['split_state_dicts']
+        want = [(k, tuple(v)) for k, v in split[name]]
     got = [(k, tuple(v.shape)) for k, v in ours.state_dict().items()]
     assert got == want
