@@ -69,6 +69,9 @@ _SIGS = {
     'gin_hexconv_stats_ws_bytes': (_sz, [_i]),
     'gin_hexconv_fwd_bf16_stats': (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _vp, _vp, _vp]),
     'gin_hexconv_fwd_bf16_stats2': (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _i, _vp, _i, _i, _i, _i, _vp, _vp, _vp]),
+    'gin_hexconv_affine_ring_bytes': (_sz, [_i, _i]),
+    'gin_hexconv_fwd_affine': (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _i, _vp, _i64, _i, _i, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _vp]),
+    'gin_bn_eval_consts': (_i, [_vp, _i, _i, _vp]),
     'gin_bn_stats_from_parts': (_i, [_vp, _i, _i64, _i64, _i, _vp, _vp, _f, _f, _vp, _vp, _vp, _vp, _vp]),
     'gin_bn_stats_from_parts2': (_i, [_vp, _i, _i64, _i64, _i, _i, _vp, _vp, _f, _f, _vp, _vp, _vp, _vp, _i, _vp, _vp, _f, _f, _vp, _vp, _vp, _vp, _vp]),
     'gin_hexconv_dgrad_bf16': (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _vp]),

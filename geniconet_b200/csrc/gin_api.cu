@@ -241,6 +241,13 @@ static int conv_hdr(const void* plan_host, const void* plan_dev, const GinConvPl
   return GIN_OK;
 }
 
+// the forward of this plan and size runs the second-generation patch kernel (gin_conv2.cuh)
+static bool fwd_v2_ok(const GinConvPlanHdr* h, int Cin, int Cout) {
+  return tc_mode() == 2 && gin::tc_supported(Cin, Cout) &&
+         (h->stride == 1 ? (patch_mode_enabled() && gin::tcp_supported(h->pfwd, Cin, Cout) && gin::cv2_supported(h->pfwd, Cin, Cout))
+                         : gin::cv2_supported(h->p2, Cin, Cout));
+}
+
 int gin_hexconv_fwd(const void* plan_host, const void* plan_dev, const float* x, int64_t sb, int64_t sp, int64_t sc, const void* packed,
                     const float* bias, float* y, int B, int Cin, int Cout, int impl, void* stream) {
   cudaStream_t st = (cudaStream_t)stream;
@@ -457,15 +464,66 @@ int gin_hexconv_fwd_bf16_stats2(const void* plan_host, const void* plan_dev, con
     const GinConvPlanHdr* h;
     int rc0 = conv_hdr(plan_host, plan_dev, &h);
     if (rc0) return rc0;
-    const bool v2 = tc_mode() == 2 && gin::tc_supported(Cin, Cout) &&
-                    (h->stride == 1 ? (patch_mode_enabled() && gin::tcp_supported(h->pfwd, Cin, Cout) && gin::cv2_supported(h->pfwd, Cin, Cout))
-                                    : gin::cv2_supported(h->p2, Cin, Cout));
-    if (!v2) return fail(GIN_ERR_UNSUPPORTED, "gin_hexconv_fwd_bf16_stats2: this plan / size does not run the second-generation patch kernel");
+    if (!fwd_v2_ok(h, Cin, Cout)) return fail(GIN_ERR_UNSUPPORTED, "gin_hexconv_fwd_bf16_stats2: this plan / size does not run the second-generation patch kernel");
   }
   gin::bias2_ref().p = bias1; gin::bias2_ref().split = bias1 ? split : 0; gin::bias2_ref().y_f16 = y_fp16 ? 1 : 0;
   const int rc = gin_hexconv_fwd_bf16_stats(plan_host, plan_dev, xb, packed, bias0, reinterpret_cast<float*>(y), B, Cin, Cout, stats_ws, nparts, stream);
   gin::bias2_ref() = gin::Bias2{};
   return rc;
+}
+
+size_t gin_hexconv_affine_ring_bytes(int B, int Cout) { return (B <= 0 || Cout <= 0) ? 0 : (size_t)B * 10 * Cout * 4; }
+
+int gin_hexconv_fwd_affine(const void* plan_host, const void* plan_dev, const void* xb, const void* packed, const float* scale, const float* shift,
+                           int relu_split, const void* res, int64_t ld_res, int res_fp16, int split, void* out0_b, float* out0_f, void* out1_b,
+                           float* out1_f, float* ring_ws, int B, int Cin, int Cout, void* stream) {
+  const bool two = split < Cout;
+  if (!xb || !packed || !scale || !shift || B <= 0 || Cin <= 0 || Cout <= 0 || relu_split < 0 || relu_split > Cout)
+    return fail(GIN_ERR_ARG, "gin_hexconv_fwd_affine: bad argument");
+  if (split <= 0 || split > Cout || (split & 63)) return fail(GIN_ERR_ARG, "gin_hexconv_fwd_affine: split must be a multiple of 64 in (0, Cout]");
+  if ((!out0_b && !out0_f) || (two ? (!out1_b && !out1_f) : (out1_b || out1_f)))
+    return fail(GIN_ERR_ARG, "gin_hexconv_fwd_affine: every destination needs an output (and split == Cout has no second one)");
+  if (res && (ld_res < Cout || (ld_res & 3))) return fail(GIN_ERR_ARG, "gin_hexconv_fwd_affine: ld_res must be >= Cout and a multiple of 4");
+  if ((out0_b || out1_b) && !ring_ws) return fail(GIN_ERR_ARG, "gin_hexconv_fwd_affine: an operand copy needs ring_ws");
+  const GinConvPlanHdr* h;
+  int rc = conv_hdr(plan_host, plan_dev, &h);
+  if (rc) return rc;
+  if (!fwd_v2_ok(h, Cin, Cout)) return fail(GIN_ERR_UNSUPPORTED, "gin_hexconv_fwd_affine: this plan / size does not run the second-generation patch kernel");
+  if ((long long)B * h->fwd.P_dst + 2LL * B >= 0x7fffffffLL) return fail(GIN_ERR_UNSUPPORTED, "gin_hexconv_fwd_affine: B*P too large");
+  cudaStream_t st = (cudaStream_t)stream;
+  const int f16 = (int)gin::fwd_fp16();
+  gin::cv2::Affine a{};
+  a.scale = scale; a.shift = shift; a.relu_split = relu_split; a.res = res; a.res_ld = ld_res; a.res_f16 = res_fp16 ? 1 : 0; a.split = split;
+  a.op[0] = out0_b; a.f32[0] = out0_f; a.ld[0] = split; a.ring[0] = ring_ws;
+  a.op[1] = out1_b; a.f32[1] = out1_f; a.ld[1] = Cout - split; a.ring[1] = ring_ws + (size_t)B * 10 * split;
+  a.op_f16 = f16;
+  gin::set_operand_formats(!f16, !f16);
+  const void* wb = reinterpret_cast<const char*>(packed) + packed_off_bf(Cin, Cout);
+  if (h->stride == 1)
+    rc = gin::launch_patch_conv2(plan_words(plan_dev), h->pfwd, h->group, h->fwd.P_dst, 2 << h->level_in, xb, wb, nullptr, nullptr, B, Cin, Cout, 0, st,
+                                 nullptr, nullptr, nullptr, &a);
+  else
+    rc = gin::launch_patch_conv2_s2_fwd(plan_words(plan_dev), h->p2, h->group, h->fwd.P_src, h->fwd.P_dst, 2 << h->level_out, xb, wb, nullptr, nullptr, B,
+                                        Cin, Cout, st, nullptr, nullptr, &a);
+  if (rc != GIN_OK) return fail(rc, "gin_hexconv_fwd_affine: launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+  g_launches.fetch_add(1, std::memory_order_relaxed);
+  for (int d = 0; d < 2; ++d) {
+    if (!a.op[d]) continue;
+    const long long work = 2LL * B * (a.ld[d] >> 3);
+    gin::launch_pdl(gin::bn::pole_mean_kernel, dim3(grid_for(work, 256)), dim3(256), 0, st, (const float*)a.ring[d],
+                    reinterpret_cast<__nv_bfloat16*>(a.op[d]), (long long)B * h->fwd.P_dst, B, a.ld[d], f16);
+    if ((rc = check_launch("pole_mean"))) return rc;
+  }
+  return GIN_OK;
+}
+
+int gin_bn_eval_consts(const void* table_dev, int count, int max_C, void* stream) {
+  static_assert(sizeof(gin::bn::EvalEntry) == sizeof(GinBnEvalEntry), "GinBnEvalEntry layout");
+  if (count == 0) return GIN_OK;
+  if (!table_dev || count < 0 || count > 65535 || max_C <= 0) return fail(GIN_ERR_ARG, "gin_bn_eval_consts: bad argument");
+  gin::launch_pdl(gin::bn::eval_consts_kernel, dim3((max_C + 255) / 256, count), dim3(256), 0, (cudaStream_t)stream,
+                  reinterpret_cast<const gin::bn::EvalEntry*>(table_dev));
+  return check_launch("bn_eval_consts");
 }
 
 int gin_hexconv_dgrad_bf16(const void* plan_host, const void* plan_dev, const void* dyb, const void* packed, float* dx, int B, int Cin, int Cout,

@@ -916,5 +916,57 @@ inline int grid_for_rows(long long n_threads) {
   return (int)(b < bn_ctas() ? b : bn_ctas());
 }
 
+// ------------------------------------------------------------------------------------------------ eval mode (inference)
+// One BatchNorm of a chain in eval mode (include/geniconet_b200.h: GinBnEvalEntry).
+struct EvalEntry {
+  const float* gamma;
+  const float* beta;
+  const float* running_mean;
+  const float* running_var;
+  const float* conv_bias;
+  float* scale;
+  float* shift;
+  float* stat;
+  float eps;
+  int C;
+};
+
+// grid (ceil(max_C / 256), count): the constants of every BatchNorm of a table, read from the device at run time (a captured graph
+// follows in-place updates of the parameters and running statistics)
+__global__ void __launch_bounds__(256) eval_consts_kernel(const EvalEntry* __restrict__ table) {
+  GIN_PDL_SYNC();
+  const EvalEntry t = table[blockIdx.y];
+  const int c = blockIdx.x * 256 + threadIdx.x;
+  if (c >= t.C) return;
+  const float mean = t.running_mean[c];
+  const float invstd = (float)(1.0 / sqrt((double)t.running_var[c] + (double)t.eps));
+  const float g = t.gamma ? t.gamma[c] : 1.f, b = t.beta ? t.beta[c] : 0.f;
+  const float scale = g * invstd;
+  if (t.scale) t.scale[c] = scale;
+  if (t.shift) t.shift[c] = fmaf(scale, (t.conv_bias ? t.conv_bias[c] : 0.f) - mean, b);
+  if (t.stat) { t.stat[c] = mean; t.stat[t.C + c] = invstd; t.stat[2 * t.C + c] = scale; t.stat[3 * t.C + c] = b - mean * scale; }
+}
+
+// pole-mean rows [rows + 2*sample + pole] of an operand copy from the fp32 ring values the affine conv epilogue stored
+// (cv2::Affine::ring, [B][10][C]): the same sum, in the same order, as cast_bf16_kernel over the fp32 map
+__global__ void __launch_bounds__(256) pole_mean_kernel(const float* __restrict__ ring, __nv_bfloat16* __restrict__ xb, long long rows, int B, int C,
+                                                        int f16) {
+  GIN_PDL_SYNC();
+  const int C8 = C >> 3;
+  for (long long i = blockIdx.x * 256LL + threadIdx.x; i < 2LL * B * C8; i += gridDim.x * 256LL) {
+    const int c = (int)(i % C8) * 8, sp = (int)(i / C8), sample = sp >> 1, pole = sp & 1;
+    float4 a = make_float4(0.f, 0.f, 0.f, 0.f), b = a;
+#pragma unroll
+    for (int k = 0; k < 5; ++k) {
+      const float* src = ring + ((size_t)sample * 10 + pole * 5 + k) * C + c;
+      a = fma4(0.2f, ld4(src), a);
+      b = fma4(0.2f, ld4(src + 4), b);
+    }
+    uint4 o;
+    o.x = pack2_op(a.x, a.y, f16); o.y = pack2_op(a.z, a.w, f16); o.z = pack2_op(b.x, b.y, f16); o.w = pack2_op(b.z, b.w, f16);
+    *reinterpret_cast<uint4*>(xb + (rows + sp) * C + c) = o;
+  }
+}
+
 }  // namespace bn
 }  // namespace gin

@@ -48,6 +48,28 @@ constexpr int STAGE_BYTES = EPI_WARPS * 32 * STAGE_PITCH;
 constexpr int SMEM_LIMIT = 227 * 1024;
 constexpr int MAX_PLANES = 16;
 
+// Eval-mode BatchNorm in the epilogue (forward-only inference, gin_hexconv_fwd_affine): per output column
+//   o = acc*scale[col] + shift[col]  (conv bias folded into shift);  ReLU on columns < relu_split;
+//   with res: o = relu(o + R[row][col])  (conv01 of a residual block: relu(bn01(conv01) + bn10(conv10)));
+// columns < split go to destination 0, the others to destination 1 (column col - split).  A destination is any combination of
+// the 16-bit forward operand copy [B*P + 2B][ld] and an fp32 map [B*P][ld] (ld = its width).  Where an operand copy is written,
+// the fp32 values of the ten pole-ring pixels of every sample also go to ring[d] = [B][10][ld]; pole_mean_kernel then forms the
+// pole-mean rows from them exactly as cast_bf16_kernel would from the fp32 output.
+struct Affine {
+  const float* scale;
+  const float* shift;
+  int relu_split;
+  const void* res;            // may be null; fp32, or fp16 when res_f16
+  long long res_ld;
+  int res_f16;
+  int split;                  // N when there is one destination
+  void* op[2];                // 16-bit operand copies (forward format: op_f16)
+  float* f32[2];
+  float* ring[2];
+  int ld[2];
+  int op_f16;
+};
+
 // A tile is processed as `nplanes` segments.  Each segment stages ONE image (its own source table) per 64-channel chunk and
 // applies its own short tap list to it.  Stride 1: one segment with all seven taps.  Stride-2 forward: four parity planes of
 // the fine input, 1-2 taps each, all accumulated into one output tile.  Stride-2 dgrad: the four parity classes of the fine
@@ -86,6 +108,7 @@ struct Params {
   int8_t x_tap[MAX_PLANES];
   int* stats_parts;           // host: receives the number of per-CTA statistics rows written (0: none)
   int dbg;                    // GIN_DBG bit mask (experiments only): 1 no epilogue stores, 2 no patch loads, 4 no MMAs
+  Affine aff;                 // eval-mode BatchNorm epilogue (aff.scale != null: the AFFINE instantiations; bias / Y / stats unused)
 };
 
 constexpr int kDi[7] = {0, -1, 1, 0, 0, -1, 1};
@@ -133,7 +156,17 @@ constexpr int BAR_BYTES = NBARS * 8 + 16;
 #define PROF_ADD(acc)
 #endif
 
-template <int N_TILE, bool RESIDENT, bool STATS, bool SEAM>
+// store of one 4-column group by the affine epilogue; ri = ring slot (sample*10 + pole*5 + e) of the row, or -1
+GIN_DEVINL void affine_store(const Affine& a, int d, int gd, int ri, int dcol, float4 o) {
+  const size_t off = (size_t)gd * a.ld[d] + dcol;
+  if (a.f32[d]) *reinterpret_cast<float4*>(a.f32[d] + off) = o;
+  if (a.op[d]) {
+    *reinterpret_cast<uint2*>(reinterpret_cast<__nv_bfloat16*>(a.op[d]) + off) = make_uint2(pack2_op(o.x, o.y, a.op_f16), pack2_op(o.z, o.w, a.op_f16));
+    if (ri >= 0) *reinterpret_cast<float4*>(a.ring[d] + (size_t)ri * a.ld[d] + dcol) = o;
+  }
+}
+
+template <int N_TILE, bool RESIDENT, bool STATS, bool SEAM, bool AFFINE = false>
 __global__ void __launch_bounds__(NTHREADS, 1) patch_conv_kernel(const Params p) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
@@ -443,6 +476,11 @@ __global__ void __launch_bounds__(NTHREADS, 1) patch_conv_kernel(const Params p)
         }
       }
       const int gd = extra_row ? -3 : (gdl < total_pix ? (int)gdl : -1);       // B*P < 2^31 is checked by the launcher
+      int ri = -1;                                    // AFFINE: ring slot of this row (gin_bn.cuh ring_pixel: first / last pixel of a chart)
+      if (AFFINE && gd >= 0) {
+        const int sample = gd / p.P_dst, pix = gd - sample * p.P_dst, A = p.P_dst / 5, e = pix / A, li = pix - e * A;
+        ri = li == 0 ? sample * 10 + e : li == A - 1 ? sample * 10 + 5 + e : -1;
+      }
       const uint32_t ab = wc & 1;
       { PROF_T0(); mbar_wait(&acc_full[ab], (wc >> 1) & 1u); PROF_ADD(pw[0]); }
       tc_fence_after();
@@ -463,6 +501,44 @@ __global__ void __launch_bounds__(NTHREADS, 1) patch_conv_kernel(const Params p)
           mbar_arrive(&acc_empty[ab]);
         }
         __syncwarp();
+        if (AFFINE) {
+          const int col = n0 + slab + c4;
+          const float4 sc = __ldg(reinterpret_cast<const float4*>(p.aff.scale + col)), sh = __ldg(reinterpret_cast<const float4*>(p.aff.shift + col));
+          const bool relu = col < p.aff.relu_split;
+          const int d = col >= p.aff.split ? 1 : 0, dcol = col - (d ? p.aff.split : 0);
+          // the residual rows of four stores are loaded before any of them is written: the compiler cannot move a load across a
+          // store through another pointer, and one load latency per store bounded the residual launches
+#pragma unroll
+          for (int i0 = 0; i0 < 8; i0 += 4) {
+            float4 r[4];
+#pragma unroll
+            for (int k = 0; k < 4; ++k) {
+              const int gd2 = __shfl_sync(0xffffffffu, gd, 4 * (i0 + k) + rsub);
+              r[k] = make_float4(0.f, 0.f, 0.f, 0.f);
+              if (p.aff.res && gd2 >= 0) {
+                if (p.aff.res_f16) {
+                  const uint2 u = __ldg(reinterpret_cast<const uint2*>(reinterpret_cast<const __half*>(p.aff.res) + (size_t)gd2 * p.aff.res_ld + col));
+                  const float2 lo = __half22float2(*reinterpret_cast<const __half2*>(&u.x)), hi = __half22float2(*reinterpret_cast<const __half2*>(&u.y));
+                  r[k] = make_float4(lo.x, lo.y, hi.x, hi.y);
+                } else r[k] = __ldg(reinterpret_cast<const float4*>(reinterpret_cast<const float*>(p.aff.res) + (size_t)gd2 * p.aff.res_ld + col));
+              }
+            }
+#pragma unroll
+            for (int k = 0; k < 4; ++k) {
+              const int r2 = 4 * (i0 + k) + rsub;
+              const int gd2 = __shfl_sync(0xffffffffu, gd, r2), ri2 = __shfl_sync(0xffffffffu, ri, r2);
+              const float4 a = *reinterpret_cast<const float4*>(my_stage + r2 * STAGE_PITCH + c4 * 4);
+              float4 o = make_float4(fmaf(a.x, sc.x, sh.x), fmaf(a.y, sc.y, sh.y), fmaf(a.z, sc.z, sh.z), fmaf(a.w, sc.w, sh.w));
+              if (relu) { o.x = fmaxf(o.x, 0.f); o.y = fmaxf(o.y, 0.f); o.z = fmaxf(o.z, 0.f); o.w = fmaxf(o.w, 0.f); }
+              if (p.aff.res) {
+                o.x = fmaxf(o.x + r[k].x, 0.f); o.y = fmaxf(o.y + r[k].y, 0.f); o.z = fmaxf(o.z + r[k].z, 0.f); o.w = fmaxf(o.w + r[k].w, 0.f);
+              }
+              if (gd2 >= 0) affine_store(p.aff, d, gd2, ri2, dcol, o);
+            }
+          }
+          __syncwarp();
+          continue;
+        }
         float4 bb = make_float4(0.f, 0.f, 0.f, 0.f);
         if (p.bias) {
           const int col = n0 + slab + c4;
@@ -578,15 +654,19 @@ int launch(Params p, cudaStream_t st) {
         cudaFuncSetAttribute(patch_conv_kernel<N_TILE, true, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT) != cudaSuccess ||
         cudaFuncSetAttribute(patch_conv_kernel<N_TILE, false, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT) != cudaSuccess ||
         cudaFuncSetAttribute(patch_conv_kernel<N_TILE, true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT) != cudaSuccess ||
-        cudaFuncSetAttribute(patch_conv_kernel<N_TILE, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT) != cudaSuccess) return -3;
+        cudaFuncSetAttribute(patch_conv_kernel<N_TILE, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT) != cudaSuccess ||
+        cudaFuncSetAttribute(patch_conv_kernel<N_TILE, true, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT) != cudaSuccess ||
+        cudaFuncSetAttribute(patch_conv_kernel<N_TILE, false, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT) != cudaSuccess) return -3;
     configured = true;
   }
   p.n_blocks = p.N / N_TILE;
   const bool seam = p.x_total > 0;
-  const bool stats = p.stats != nullptr && !p.flush_each && !seam;
+  const bool affine = p.aff.scale != nullptr;        // the launcher of the affine form allows no seam tiles, statistics or accumulation
+  const bool stats = p.stats != nullptr && !p.flush_each && !seam && !affine;
   const int sms = num_sms();
   void (*kern)(const Params);
-  if (seam) kern = p.resident ? patch_conv_kernel<N_TILE, true, false, true> : patch_conv_kernel<N_TILE, false, false, true>;
+  if (affine) kern = p.resident ? patch_conv_kernel<N_TILE, true, false, false, true> : patch_conv_kernel<N_TILE, false, false, false, true>;
+  else if (seam) kern = p.resident ? patch_conv_kernel<N_TILE, true, false, true> : patch_conv_kernel<N_TILE, false, false, true>;
   else if (p.resident) kern = stats ? patch_conv_kernel<N_TILE, true, true, false> : patch_conv_kernel<N_TILE, true, false, false>;
   else kern = stats ? patch_conv_kernel<N_TILE, false, true, false> : patch_conv_kernel<N_TILE, false, false, false>;
   // Streamed weights: clusters of CL CTAs share the weight stream (GIN_CLUSTER = 1 switches it off, 4 asks for clusters of four).
@@ -665,7 +745,8 @@ int cv2_launch_pair(cv2::Params& p, int nt, cudaStream_t st);
 inline bool cv2_pair_ok(const cv2::Params& p, int nt) {
   static int enabled = -1;
   if (enabled < 0) { const char* e = getenv("GIN_PAIR"); enabled = e ? atoi(e) : 1; }      // 0 off, 1 when it costs no extra round, 2 always
-  if (!enabled || p.flush_each || p.accumulate || p.dst_tab_off >= 0 || p.nplanes > 4 || p.x_total > 0) return false;
+  // the affine epilogue exists in the single-tile kernel only (DESIGN: Inference)
+  if (!enabled || p.flush_each || p.accumulate || p.dst_tab_off >= 0 || p.nplanes > 4 || p.x_total > 0 || p.aff.scale) return false;
   const int ntp = nt < 128 ? nt : 128;
   if (7 * (p.K / 64) * ntp * 128 <= 114688) return false;                   // the weights fit: the resident single-tile kernel is better
   auto rounds = [&](long long items, int n_blocks) {
@@ -716,9 +797,10 @@ inline void cv2_attach_boundary(cv2::Params& p, const GinPfSide* pf) {
 
 inline int launch_patch_conv2(const int32_t* plan_dev, const GinPSide& ps, int group, int P, int W, const void* Xb, const void* Wb,
                               const float* bias, float* Y, int B, int K, int N, int mirror, cudaStream_t st, float* stats = nullptr,
-                              int* stats_parts = nullptr, const GinPfSide* pf = nullptr) {
+                              int* stats_parts = nullptr, const GinPfSide* pf = nullptr, const cv2::Affine* aff = nullptr) {
   cv2::Params p{};
   cv2_attach_boundary(p, pf);
+  if (aff) p.aff = *aff;
   p.stats = stats; p.stats_parts = stats_parts;
   p.plan = plan_dev; p.fmt = operand_format_bits(); p.U = ps.U; p.Q = ps.Q; p.ntiles = ps.ntiles; p.group = group; p.B = B; p.K = K; p.N = N; p.P_src = P; p.P_dst = P;
   p.X = reinterpret_cast<const __nv_bfloat16*>(Xb); p.Wt = reinterpret_cast<const __nv_bfloat16*>(Wb); p.bias = bias; p.Y = Y;
@@ -743,9 +825,10 @@ constexpr int kS2B[7] = {0, 0, 0, -1, 0, 0, -1};
 // stride 2 forward: X is the FINE map (P_f pixels per sample), Y the coarse one; Wc = 2n of the coarse level
 inline int launch_patch_conv2_s2_fwd(const int32_t* plan_dev, const GinP2Side& ps, int group, int P_f, int P_c, int Wc, const void* Xb,
                                      const void* Wb, const float* bias, float* Y, int B, int K, int N, cudaStream_t st, float* stats = nullptr,
-                                     int* stats_parts = nullptr) {
+                                     int* stats_parts = nullptr, const cv2::Affine* aff = nullptr) {
   cv2::Params p{};
   p.mask_off = -1;
+  if (aff) p.aff = *aff;
   p.stats = stats; p.stats_parts = stats_parts;
   p.plan = plan_dev; p.fmt = operand_format_bits(); p.U = ps.U; p.Q = ps.Q; p.ntiles = ps.ntiles; p.group = group; p.B = B; p.K = K; p.N = N; p.P_src = P_f; p.P_dst = P_c;
   p.X = reinterpret_cast<const __nv_bfloat16*>(Xb); p.Wt = reinterpret_cast<const __nv_bfloat16*>(Wb); p.bias = bias; p.Y = Y;

@@ -17,7 +17,8 @@ from (plus the fp32 conv outputs BatchNorm needs):
     into the bf16 operand copy of the fine level.
 
 Parameters stay where models.py puts them (conv00.weight, icobn00.weight, ...), so state dicts are unchanged; BatchNorm running
-statistics are updated as torch does.  Training mode only (batch statistics); in eval mode the modules run one by one.
+statistics are updated as torch does.  With grad disabled, infer_chain runs the same chains forward-only (eval mode: BatchNorm in
+the conv epilogue, DESIGN "Inference"); eval mode with grad enabled runs the modules one by one.
 A conv bias that feeds a BatchNorm has a mathematically zero gradient; the fused path returns exactly zero for it.
 """
 import torch
@@ -272,6 +273,48 @@ def _bn_bwd(dout, mask_b, y, col0, ld, stat, B, level, C, dy_b=None, dy_b_col=0,
     return bstat, dy_f
 
 
+def _stem_conv(x, conv):
+    """The xyz convolution of a chain's stem (fp32, warp-level kernels).  Returns (plan, packed weights, xs, strides, y, parts):
+    y is fp16 with the epilogue's BatchNorm partial sums `parts` = (buffer, rows), or fp32 with parts None."""
+    import ctypes
+    dev, B = x.device, x.shape[0]
+    level, C = conv.subdivisions, conv.out_features
+    plan = get_plan(_lib.PLAN_HEXCONV, level, 1, conv.corner_mode, dev)
+    packed = _pack(conv.weight.detach().contiguous(), 3, C)
+    xs, sb, sp, sc = pixel_strides(x)
+    y = _empty((B * _P(level), C), torch.float16 if _Y16 else torch.float32, dev)
+    sparts = _empty(L.gin_hexconv_narrow_stats_ws_bytes(C) // 4, torch.float32, dev)
+    npart = ctypes.c_int(0)
+    rc = L.gin_hexconv_fwd_narrow_stats(plan.host_ptr, plan.dev_ptr, xs.data_ptr(), sb, sp, sc, packed.data_ptr(), conv.bias.data_ptr(),
+                                        y.data_ptr(), 1 if _Y16 else 0, B, 3, C, sparts.data_ptr(), ctypes.addressof(npart), _stream())
+    if rc == 0 and npart.value > 0:          # output statistics came out of the conv epilogue
+        return plan, packed, xs, (sb, sp, sc), y, (sparts, npart.value)
+    if rc != 0 and rc != _lib.ERR_UNSUPPORTED:
+        _lib.check(rc, 'gin_hexconv_fwd_narrow_stats')
+    y = _empty((B * _P(level), C), torch.float32, dev)
+    _lib.check(L.gin_hexconv_fwd(plan.host_ptr, plan.dev_ptr, xs.data_ptr(), sb, sp, sc, packed.data_ptr(), conv.bias.data_ptr(),
+                                 y.data_ptr(), B, 3, C, _lib.IMPL_AUTO, _stream()), 'gin_hexconv_fwd')
+    return plan, packed, xs, (sb, sp, sc), y, None
+
+
+def _block_stats(ycat, pcat, blk, rows, cout):
+    """Batch statistics of icobn00 / icobn10 (running statistics updated) from the sibling GEMM's output [rows][conv00 | conv10]."""
+    dev = ycat.device
+    if pcat is not None:                 # both sibling BatchNorms from the same epilogue sums: one launch
+        stat00, stat10 = _empty(4 * cout, torch.float32, dev), _empty(4 * cout, torch.float32, dev)
+        bA, bB = blk.icobn00, blk.icobn10
+        _lib.check(L.gin_bn_stats_from_parts2(pcat[0].data_ptr(), pcat[1], 2 * cout, rows, cout,
+                                              0, bA.weight.data_ptr(), bA.bias.data_ptr(), float(bA.eps), float(bA.momentum), bA.running_mean.data_ptr(),
+                                              bA.running_var.data_ptr(), bA.num_batches_tracked.data_ptr(), stat00.data_ptr(),
+                                              cout, bB.weight.data_ptr(), bB.bias.data_ptr(), float(bB.eps), float(bB.momentum), bB.running_mean.data_ptr(),
+                                              bB.running_var.data_ptr(), bB.num_batches_tracked.data_ptr(), stat10.data_ptr(), _stream()),
+                   'gin_bn_stats_from_parts2')
+    else:
+        stat00 = _bn_stats(ycat, 0, 2 * cout, rows, cout, blk.icobn00, pcat)
+        stat10 = _bn_stats(ycat, cout, 2 * cout, rows, cout, blk.icobn10, pcat)
+    return stat00, stat10
+
+
 # ------------------------------------------------------------------------------------------------ the chain
 class _Chain(torch.autograd.Function):
     @staticmethod
@@ -285,24 +328,8 @@ class _Chain(torch.autograd.Function):
         if isinstance(mods[0], IcoConvS2S):                                  # ---- stem: xyz conv (fp32, warp-level kernels) + BN + ReLU
             conv, bn = mods[0], mods[1]
             level, C = conv.subdivisions, conv.out_features
-            plan = get_plan(_lib.PLAN_HEXCONV, level, 1, conv.corner_mode, dev)
-            packed = _pack(conv.weight.detach().contiguous(), 3, C)
-            xs, sb, sp, sc = pixel_strides(x)
-            import ctypes
-            y = _empty((B * _P(level), C), torch.float16 if _Y16 else torch.float32, dev)
-            sparts = _empty(L.gin_hexconv_narrow_stats_ws_bytes(C) // 4, torch.float32, dev)
-            npart = ctypes.c_int(0)
-            rc = L.gin_hexconv_fwd_narrow_stats(plan.host_ptr, plan.dev_ptr, xs.data_ptr(), sb, sp, sc, packed.data_ptr(), conv.bias.data_ptr(),
-                                                y.data_ptr(), 1 if _Y16 else 0, B, 3, C, sparts.data_ptr(), ctypes.addressof(npart), _stream())
-            if rc == 0 and npart.value > 0:          # output statistics came out of the conv epilogue
-                stat = _bn_stats(y, 0, C, B * _P(level), C, bn, (sparts, npart.value))
-            else:
-                if rc != 0 and rc != _lib.ERR_UNSUPPORTED:
-                    _lib.check(rc, 'gin_hexconv_fwd_narrow_stats')
-                y = _empty((B * _P(level), C), torch.float32, dev)
-                _lib.check(L.gin_hexconv_fwd(plan.host_ptr, plan.dev_ptr, xs.data_ptr(), sb, sp, sc, packed.data_ptr(), conv.bias.data_ptr(),
-                                             y.data_ptr(), B, 3, C, _lib.IMPL_AUTO, _stream()), 'gin_hexconv_fwd')
-                stat = _bn_stats(y, 0, C, B * _P(level), C, bn)
+            plan, packed, xs, (sb, sp, sc), y, parts = _stem_conv(x, conv)
+            stat = _bn_stats(y, 0, C, B * _P(level), C, bn, parts)
             act_b, _, act_w = _bn_act(y, 0, C, stat, None, 0, 0, None, B, level, C)
             saved.append(dict(kind='stem', plan=plan, xs=xs, strides=(sb, sp, sc), y=y, stat=stat, out_b=act_w, C=C, level=level, packed=packed))
             i = 3
@@ -350,18 +377,7 @@ class _Chain(torch.autograd.Function):
             rows = B * _P(lvl)
             pk_cat, pk01 = packs[2 * (j - i)], packs[2 * (j - i) + 1]
             ycat, pcat = _conv_fwd(plan_a, a_b, pk_cat, blk.conv00.bias.detach(), B, cin, 2 * cout, _P(lvl), bias1=blk.conv10.bias.detach())   # [rows][conv00 | conv10]
-            if pcat is not None:                 # both sibling BatchNorms from the same epilogue sums: one launch
-                stat00, stat10 = _empty(4 * cout, torch.float32, dev), _empty(4 * cout, torch.float32, dev)
-                bA, bB = blk.icobn00, blk.icobn10
-                _lib.check(L.gin_bn_stats_from_parts2(pcat[0].data_ptr(), pcat[1], 2 * cout, rows, cout,
-                                                      0, bA.weight.data_ptr(), bA.bias.data_ptr(), float(bA.eps), float(bA.momentum), bA.running_mean.data_ptr(),
-                                                      bA.running_var.data_ptr(), bA.num_batches_tracked.data_ptr(), stat00.data_ptr(),
-                                                      cout, bB.weight.data_ptr(), bB.bias.data_ptr(), float(bB.eps), float(bB.momentum), bB.running_mean.data_ptr(),
-                                                      bB.running_var.data_ptr(), bB.num_batches_tracked.data_ptr(), stat10.data_ptr(), _stream()),
-                           'gin_bn_stats_from_parts2')
-            else:
-                stat00 = _bn_stats(ycat, 0, 2 * cout, rows, cout, blk.icobn00, pcat)
-                stat10 = _bn_stats(ycat, cout, 2 * cout, rows, cout, blk.icobn10, pcat)
+            stat00, stat10 = _block_stats(ycat, pcat, blk, rows, cout)
             h_b, _, h_w = _bn_act(ycat, 0, 2 * cout, stat00, None, 0, 0, None, B, lvl, cout)
             y01, p01 = _conv_fwd(plan_b, h_b, pk01, blk.conv01.bias.detach(), B, cout, cout, _P(lvl))
             stat01 = _bn_stats(y01, 0, cout, rows, cout, blk.icobn01, p01)
@@ -465,6 +481,199 @@ def run_chain(x, mods):
     """Forward of the module list `mods` (see chain_supported) on the fused path; x fp32 CUDA, returns the fp32 output map."""
     mods = list(mods)
     return _Chain.apply(x, mods, *chain_params(mods))
+
+
+# ------------------------------------------------------------------------------------------------ forward-only chain (inference)
+_EVAL_CACHE = {}
+
+
+def _bn_table(pairs):
+    """Device table of GinBnEvalEntry (include/geniconet_b200.h) for `pairs` = [(BatchNorm2d, conv bias or None)] and the fp32
+    buffer it fills: per entry scale [C], shift [C] (conv bias folded in), stat [4][C] (gin_bn_act_fwd layout, no bias).  Cached
+    per set of parameter storages: the table holds pointers only, so in-place load_state_dict needs no rebuild, and a captured
+    graph reads the current values at every replay."""
+    key = tuple((id(bn), bn.weight.data_ptr(), bn.bias.data_ptr(), bn.running_mean.data_ptr(), bn.running_var.data_ptr(), float(bn.eps),
+                 b.data_ptr() if b is not None else 0) for bn, b in pairs)
+    hit = _EVAL_CACHE.get(key)
+    if hit is not None:
+        return hit
+    import ctypes
+    import numpy as np
+    dev = pairs[0][0].weight.device
+    sizes = [bn.num_features for bn, _ in pairs]
+    S = sum(sizes)
+    buf = torch.empty(6 * S, dtype=torch.float32, device=dev)      # [all scales | all shifts | all stats]: consecutive entries adjacent
+    rec = np.dtype([('p', np.uint64, 8), ('eps', np.float32), ('C', np.int32)])
+    assert rec.itemsize == 72
+    tab = np.zeros(len(pairs), dtype=rec)
+    views, off = [], 0
+    for k, ((bn, b), C) in enumerate(zip(pairs, sizes)):
+        sc, sh, st = buf[off:off + C], buf[S + off:S + off + C], buf[2 * S + 4 * off:2 * S + 4 * (off + C)]
+        off += C
+        tab[k]['p'] = [bn.weight.data_ptr(), bn.bias.data_ptr(), bn.running_mean.data_ptr(), bn.running_var.data_ptr(),
+                       b.data_ptr() if b is not None else 0, sc.data_ptr(), sh.data_ptr(), st.data_ptr()]
+        tab[k]['eps'], tab[k]['C'] = bn.eps, C
+        views.append((sc, sh, st))
+    table = torch.from_numpy(tab.view(np.uint8).copy()).to(dev)
+    hit = _EVAL_CACHE[key] = (table, len(pairs), max(sizes), buf, views)
+    return hit
+
+
+def _eval_consts(pairs):
+    """[(scale, shift, stat)] per pair, computed on the device from the current parameters and running statistics (one launch)."""
+    table, n, cmax, _, views = _bn_table(pairs)
+    _lib.check(L.gin_bn_eval_consts(table.data_ptr(), n, cmax, _stream()), 'gin_bn_eval_consts')
+    return views
+
+
+def _span(t, n):
+    """n elements of t's storage from t's first element on: the constants of consecutive table entries as one vector"""
+    return t.as_strided((n,), (1,))
+
+
+def _conv_affine(plan, xb, packed, B, cin, cout, level, scale, shift, relu_split, split, want0, want1=(False, False), res=None):
+    """Convolution with eval-mode BatchNorm in the epilogue (gin_hexconv_fwd_affine).  want0 / want1 = (operand copy, fp32 map) of
+    the columns < split / >= split.  Returns [out0_b, out0_f, out1_b, out1_f] (None where not wanted), or None when the epilogue
+    does not support this plan and size."""
+    dev, rows = xb.device, B * _P(level)
+    outs = []
+    for (wb, wf), width in ((want0, split), (want1, cout - split)):
+        outs.append(_empty((rows + 2 * B, width), torch.bfloat16, dev) if wb else None)
+        outs.append(_empty((rows, width), torch.float32, dev) if wf else None)
+    ring = _empty(L.gin_hexconv_affine_ring_bytes(B, cout) // 4, torch.float32, dev) if (want0[0] or want1[0]) else None
+    ptr = lambda t: t.data_ptr() if t is not None else None
+    rc = L.gin_hexconv_fwd_affine(plan.host_ptr, plan.dev_ptr, xb.data_ptr(), packed.data_ptr(), scale.data_ptr(), shift.data_ptr(), relu_split,
+                                  ptr(res), res.shape[1] if res is not None else 0, 1 if res is not None and res.dtype == torch.float16 else 0,
+                                  split, *[ptr(t) for t in outs], ptr(ring), B, cin, cout, _stream())
+    if rc == _lib.ERR_UNSUPPORTED:
+        return None
+    _lib.check(rc, 'gin_hexconv_fwd_affine')
+    return outs
+
+
+def eval_pairs(mods):
+    """(BatchNorm2d, conv bias or None) of every BatchNorm of a chain, in the order infer_chain reads their constants; the stem's
+    BatchNorm is applied by gin_bn_act_fwd to a map that already holds the conv bias."""
+    pairs = []
+    for m in mods:
+        if isinstance(m, torch.nn.BatchNorm2d):
+            pairs.append((m, None))
+        elif _is_block(m):
+            pairs += [(m.icobn00, m.conv00.bias), (m.icobn10, m.conv10.bias), (m.icobn01, m.conv01.bias)]
+    return pairs
+
+
+def infer_chain(x, mods, want_operand=False):
+    """Forward-only execution of the chain `mods` (see chain_supported): no autograd, nothing saved, no bf16 wgrad twins.
+
+    Eval mode (every BatchNorm has training == False): the BatchNorms use their running statistics; the constants of all of them
+    come from one launch (gin_bn_eval_consts) and are applied in the epilogue of the convolution that feeds them
+    (gin_hexconv_fwd_affine), with gin_hexconv_fwd_bf16_stats2 + gin_bn_act_fwd wherever that epilogue is unsupported and for the
+    stem.  Train mode (under no_grad): the training chain's forward kernels with batch statistics; output and running statistics are
+    bit for bit those of _Chain.forward.
+
+    Returns (fp32 output map [B, C, H, W] with channels-last strides, its 16-bit forward operand copy when want_operand else None)."""
+    mods = list(mods)
+    train = mods[-1].icobn01.training
+    dev, B = x.device, x.shape[0]
+    consts = None if train else iter(_eval_consts(eval_pairs(mods)))
+    i = 0
+    if isinstance(mods[0], IcoConvS2S):
+        conv, bn = mods[0], mods[1]
+        level, C = conv.subdivisions, conv.out_features
+        _, _, _, _, y, parts = _stem_conv(x, conv)
+        stat = _bn_stats(y, 0, C, B * _P(level), C, bn, parts) if train else next(consts)[2]
+        act_b, _, _ = _bn_act(y, 0, C, stat, None, 0, 0, None, B, level, C, want_w=False)
+        act_f = None
+        i = 3
+    else:
+        blk = mods[0]
+        level, C = blk.conv00.subdivisions - (0 if blk._down else 1), blk.conv00.in_features
+        plan = get_plan(_lib.PLAN_HEXCONV, level, 1, blk.conv00.corner_mode, dev)
+        from .ico_conv import as_channels_last, cast_bf16
+        act_b = cast_bf16(as_channels_last(x), plan, 0, level)
+        act_f = as_channels_last(x).permute(0, 2, 3, 1).reshape(-1, C)
+    jobs = []
+    for blk in mods[i:]:
+        jobs.append((blk.conv00.weight.detach().contiguous(), blk.conv10.weight.detach().contiguous(), blk.conv00.in_features))
+        jobs.append((blk.conv01.weight.detach().contiguous(), None, blk.conv01.in_features))
+    packs = _pack_many(jobs)
+    last = len(mods) - 1
+    for j in range(i, len(mods)):
+        blk = mods[j]
+        cm = blk.conv00.corner_mode
+        cin, cout = blk.conv00.in_features, blk.conv00.out_features
+        if blk._down:
+            lvl = level - 1
+            plan_a = get_plan(_lib.PLAN_HEXCONV, level, 2, cm, dev)
+            a_b = act_b
+        else:
+            lvl = level + 1
+            up_plan = get_plan(_lib.PLAN_UPSAMPLE, level, 1, blk.upsample00.corner_mode, dev)
+            plan_a = get_plan(_lib.PLAN_HEXCONV, lvl, 1, cm, dev)
+            a_b = _empty((B * _P(lvl) + 2 * B, cin), torch.bfloat16, dev)
+            _lib.check(L.gin_upsample_bf16(up_plan.host_ptr, up_plan.dev_ptr, act_f.data_ptr(), 1, a_b.data_ptr(), None, B, cin, _stream()),
+                       'gin_upsample_bf16')
+        plan_b = get_plan(_lib.PLAN_HEXCONV, lvl, 1, cm, dev)
+        rows = B * _P(lvl)
+        pk_cat, pk01 = packs[2 * (j - i)], packs[2 * (j - i) + 1]
+        is_last = j == last
+        keep_f = is_last or not mods[j + 1]._down
+        want_b = not is_last or want_operand
+        if train:
+            ycat, pcat = _conv_fwd(plan_a, a_b, pk_cat, blk.conv00.bias.detach(), B, cin, 2 * cout, _P(lvl), bias1=blk.conv10.bias.detach())
+            stat00, stat10 = _block_stats(ycat, pcat, blk, rows, cout)
+            h_b, _, _ = _bn_act(ycat, 0, 2 * cout, stat00, None, 0, 0, None, B, lvl, cout, want_w=False)
+            y01, p01 = _conv_fwd(plan_b, h_b, pk01, blk.conv01.bias.detach(), B, cout, cout, _P(lvl))
+            stat01 = _bn_stats(y01, 0, cout, rows, cout, blk.icobn01, p01)
+            act_b, act_f, _ = _bn_act(y01, 0, cout, stat01, ycat, cout, 2 * cout, stat10, B, lvl, cout, want_b=want_b, want_f=keep_f, want_w=False)
+        else:
+            (sc00, sh00, st00), (_, _, st10), (sc01, sh01, st01) = next(consts), next(consts), next(consts)
+            r = _conv_affine(plan_a, a_b, pk_cat, B, cin, 2 * cout, lvl, _span(sc00, 2 * cout), _span(sh00, 2 * cout), cout, cout,
+                             (True, False), (False, True))
+            if r is not None:                                # relu(bn00(conv00)) as conv01's operand, bn10(conv10) as the skip map
+                r = _conv_affine(plan_b, r[0], pk01, B, cout, cout, lvl, sc01, sh01, 0, cout, (want_b, keep_f), res=r[3])
+            if r is not None:
+                act_b, act_f = r[0], r[1]
+            else:                                            # the composition with the same constants
+                ycat, _ = _conv_fwd(plan_a, a_b, pk_cat, blk.conv00.bias.detach(), B, cin, 2 * cout, _P(lvl), bias1=blk.conv10.bias.detach())
+                h_b, _, _ = _bn_act(ycat, 0, 2 * cout, st00, None, 0, 0, None, B, lvl, cout, want_w=False)
+                y01, _ = _conv_fwd(plan_b, h_b, pk01, blk.conv01.bias.detach(), B, cout, cout, _P(lvl))
+                act_b, act_f, _ = _bn_act(y01, 0, cout, st01, ycat, cout, 2 * cout, st10, B, lvl, cout, want_b=want_b, want_f=keep_f, want_w=False)
+        level, C = lvl, cout
+    n = 2 ** level
+    return act_f.view(B, 5 * n, 2 * n, C).permute(0, 3, 1, 2), (act_b if want_operand else None)
+
+
+def latent_supported(mu, logvar):
+    """The VAE's mu / logvar heads (IcoConvS2S stride 2 + BatchNorm2d, models.py _latent_head) in eval mode, without hooks."""
+    for head in (mu, logvar):
+        mods = list(head)
+        if len(mods) != 2 or not isinstance(mods[0], IcoConvS2S) or not isinstance(mods[1], torch.nn.BatchNorm2d):
+            return False
+        c, bn = mods
+        if (c.stride != 2 or c.bias is None or getattr(c, 'impl', 0) != 0 or bn.training or not bn.affine or not bn.track_running_stats
+                or c.in_features % 64 or c.out_features % 64):
+            return False
+        if any(m._forward_hooks or m._forward_pre_hooks for m in [head] + mods):
+            return False
+    a, b = mu[0], logvar[0]
+    return (a.in_features, a.out_features, a.subdivisions, a.corner_mode) == (b.in_features, b.out_features, b.subdivisions, b.corner_mode)
+
+
+def infer_latent(h_b, mu, logvar, B):
+    """mu and logvar heads as ONE stride-2 GEMM with two fp32 destinations; h_b = the operand copy of their common input.
+    Returns (mu, logvar) as [B, C, H, W] maps with channels-last strides, or None when the epilogue does not support the size."""
+    c0, c1 = mu[0], logvar[0]
+    cin, cout, lvl = c0.in_features, c0.out_features, c0.subdivisions - 1
+    (sa, ha, _), _ = _eval_consts([(mu[1], c0.bias), (logvar[1], c1.bias)])
+    packed = _pack_many([(c0.weight.detach().contiguous(), c1.weight.detach().contiguous(), cin)])[0]
+    plan = get_plan(_lib.PLAN_HEXCONV, c0.subdivisions, 2, c0.corner_mode, h_b.device)
+    r = _conv_affine(plan, h_b, packed, B, cin, 2 * cout, lvl, _span(sa, 2 * cout), _span(ha, 2 * cout), 0, cout, (False, True), (False, True))
+    if r is None:
+        return None
+    n = 2 ** lvl
+    return tuple(t.view(B, 5 * n, 2 * n, cout).permute(0, 3, 1, 2) for t in (r[1], r[3]))
 
 
 # ------------------------------------------------------------------ decoder head: Conv2d(64, 3, 1) -> Tanh (models.py:151-154)

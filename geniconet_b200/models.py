@@ -25,18 +25,43 @@ from .reparam import reparameterize as _reparameterize
 # set_fused(False) runs every module on its own, exactly as the unmodified reference models.py does.
 _FUSED = os.environ.get('GIN_FUSED', '1') != '0'
 _HEAD = os.environ.get('GIN_HEAD', '1') != '0'           # the decoder head through gin_head_* (A/B: GIN_HEAD=0 keeps Conv2d + Tanh)
+# Forward-only fused chains (fused.infer_chain) when grad is disabled (no_grad / inference_mode); opt-in: GIN_FUSED_INFER=1 or
+# set_fused(True, inference=True).
+_INFER = os.environ.get('GIN_FUSED_INFER', '0') == '1'
 
 
-def set_fused(flag, head=None):
-    global _FUSED, _HEAD
+def set_fused(flag, head=None, inference=None):
+    global _FUSED, _HEAD, _INFER
     _FUSED = bool(flag)
     if head is not None:
         _HEAD = bool(head)
+    if inference is not None:
+        _INFER = bool(inference)
+
+
+def _infer(mods, x, want_operand=False):
+    """fused.infer_chain over `mods` (a Sequential, whose own hooks count too, or a list of modules) when grad is disabled, every
+    BatchNorm inside is in the same mode and no module inside has a forward hook; else None (the caller runs the modules)."""
+    tops = [mods] if isinstance(mods, torch.nn.Module) else list(mods)
+    mods = list(mods)
+    if not (_FUSED and _INFER and not torch.is_grad_enabled() and x.is_cuda and x.dtype == torch.float32):
+        return None
+    inner = [m for t in tops for m in t.modules()]
+    if any(m._forward_hooks or m._forward_pre_hooks for m in inner):
+        return None
+    if len({m.training for m in inner if isinstance(m, torch.nn.BatchNorm2d)}) != 1:
+        return None
+    if any(getattr(c, 'impl', 0) != 0 for c in inner if isinstance(c, IcoConvS2S)) or not _fused.chain_supported(mods):
+        return None
+    return _fused.infer_chain(x, mods, want_operand)
 
 
 def _run(mods, x):
     """nn.Sequential semantics over the module list, through the fused chain when possible."""
     mods = list(mods)
+    r = _infer(mods, x)
+    if r is not None:
+        return r[0]
     if (_FUSED and x.is_cuda and x.dtype == torch.float32 and torch.is_grad_enabled() and all(m.training for m in mods)
             and all(getattr(c, 'impl', 0) == 0 for m in mods for c in m.modules() if isinstance(c, IcoConvS2S))
             and _fused.chain_supported(mods)):
@@ -212,7 +237,8 @@ class ico2enc(torch.nn.Module):
         self.encoder = createico2enc(params['ico']['corner_mode'], params['ico2ico']['model'], _top(params))
 
     def forward(self, x):
-        return self.encoder(x)
+        r = _infer(self.encoder, x)
+        return r[0] if r is not None else self.encoder(x)
 
 
 class enc2ico(torch.nn.Module):
@@ -222,13 +248,21 @@ class enc2ico(torch.nn.Module):
         self.decoder, self.enc2icoConv = createenc2ico(params['ico']['corner_mode'], params['ico2ico']['model'], self.subdivisions)
 
     def forward(self, x):
-        return _head(self.enc2icoConv, self.decoder(x))
+        r = _infer(self.decoder, x)
+        return _head(self.enc2icoConv, r[0] if r is not None else self.decoder(x))
 
 
 def _latent_head(params, level):
     return torch.nn.Sequential(IcoConvS2S(in_features=256, out_features=512, stride=2, bias=True, subdivisions=level,
                                           corner_mode=params['ico']['corner_mode']),
                                BatchNorm2d(512))
+
+
+def _latent(r, mu, logvar, x):
+    """(mu, logvar) from the encoder output r = (map, operand copy) of _infer as one GEMM (fused.infer_latent), or None."""
+    if not _fused.latent_supported(mu, logvar):
+        return None
+    return _fused.infer_latent(r[1], mu, logvar, x.shape[0])
 
 
 class ico2ico_vae(VAE):
@@ -252,7 +286,14 @@ class ico2ico_vae(VAE):
         return _latent_head(self.params, _top(self.params) - 2)
 
     def encode(self, input):
-        h = _run(self.encoder, input)
+        r = _infer(list(self.encoder), input, want_operand=True)
+        if r is None:
+            h = _run(self.encoder, input)
+        else:
+            lat = _latent(r, self.mu, self.logvar, input)
+            if lat is not None:
+                return self.mu_hook(lat[0]), self.logvar_hook(lat[1])
+            h = r[0]
         return self.mu_hook(self.mu(h)), self.logvar_hook(self.logvar(h))
 
     def decode(self, z):
@@ -269,7 +310,14 @@ class ico2enc_vae(VAE):
         self.logvar = _latent_head(params, _top(params) - 2)
 
     def encode(self, input):
-        h = self.encoder(input)
+        r = _infer(self.encoder, input, want_operand=True)
+        if r is None:
+            h = self.encoder(input)
+        else:
+            lat = _latent(r, self.mu, self.logvar, input)
+            if lat is not None:
+                return lat
+            h = r[0]
         return self.mu(h), self.logvar(h)
 
     def forward(self, x):
@@ -289,7 +337,8 @@ class enc2ico_vae(VAE):
         return torch.add(trn_mean, trn_logvar * torch.randn(trn_logvar.shape))
 
     def decode(self, z):
-        return _head(self.final_layer, self.decoder(z))
+        r = _infer(self.decoder, z)
+        return _head(self.final_layer, r[0] if r is not None else self.decoder(z))
 
     def forward(self, x):
         return self.decode(x), torch.tensor([]), torch.tensor([])

@@ -285,6 +285,37 @@ int gin_adam_chunk(void);
 int gin_adam_step(const void* table_dev, const int32_t* chunk_first_dev, int count, int total_chunks, float lr, const float* lr_dev, float beta1,
                   float beta2, float eps, float weight_decay, void* ticket_dev, void* stream);
 
+/* ------------------------------------------------------------------ device: eval-mode (inference) forward ---- */
+/* Forward-only convolution with an eval-mode BatchNorm applied in the epilogue (second-generation patch kernel, stride 1 or 2).
+ * Per output column: o = acc*scale[col] + shift[col] (the conv bias folded into shift: gin_bn_eval_consts); ReLU on columns
+ * < relu_split; with res != NULL (fp32, or fp16 when res_fp16; row stride ld_res elements) o = relu(o + res[row][col]).
+ * Columns < split go to destination 0, the others (split < Cout) to destination 1: out*_b = the 16-bit forward operand copy
+ * [B*P + 2B][width] (pixels, then the pole means, bit for bit what gin_cast_bf16(which = 0) makes of the fp32 values), out*_f =
+ * fp32 [B*P][width]; each may be NULL, not both.  split is a multiple of 64 in (0, Cout]; split == Cout: one destination.
+ * ring_ws: gin_hexconv_affine_ring_bytes(B, Cout) bytes, needed when an operand copy is written.
+ * GIN_ERR_UNSUPPORTED where gin_hexconv_fwd_bf16_stats2 would return it (compose it with gin_bn_act_fwd there). */
+size_t gin_hexconv_affine_ring_bytes(int B, int Cout);
+int gin_hexconv_fwd_affine(const void* plan_host, const void* plan_dev, const void* xb, const void* packed, const float* scale,
+                           const float* shift, int relu_split, const void* res, int64_t ld_res, int res_fp16, int split, void* out0_b,
+                           float* out0_f, void* out1_b, float* out1_f, float* ring_ws, int B, int Cin, int Cout, void* stream);
+/* The eval constants of `count` BatchNorms in one launch, read from the device at run time (a captured graph follows later in-place
+ * updates of the parameters and running statistics).  table_dev: GinBnEvalEntry[count] in device memory; max_C >= every C.
+ *   scale = gamma*invstd, invstd = 1/sqrt(running_var + eps);  shift = beta + scale*(conv_bias - running_mean);
+ *   stat (torch's gin_bn_stats layout, for gin_bn_act_fwd): running_mean, invstd, scale, beta - running_mean*scale. */
+typedef struct {
+  const float* gamma;          /* may be NULL: 1 */
+  const float* beta;           /* may be NULL: 0 */
+  const float* running_mean;
+  const float* running_var;
+  const float* conv_bias;      /* may be NULL: 0 */
+  float* scale;                /* [C], may be NULL */
+  float* shift;                /* [C], may be NULL */
+  float* stat;                 /* [4][C], may be NULL */
+  float eps;
+  int C;
+} GinBnEvalEntry;
+int gin_bn_eval_consts(const void* table_dev, int count, int max_C, void* stream);
+
 /* number of kernel launches issued through this library since load (bench.py's gpu_launches) */
 int64_t gin_launch_count(void);
 
