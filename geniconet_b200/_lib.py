@@ -82,7 +82,10 @@ _SIGS = {
     'gin_bn_act_bwd': (_i, [_vp, _i64, _vp, _vp, _i64, _i, _vp, _vp, _vp, _i64, _vp, _i64, _vp, _i, _i, _i, _i, _vp]),
     'gin_bn_pair_ws_bytes': (_sz, [_i]),
     'gin_bn_act_bwd_pair': (_i, [_vp, _i64, _vp, _vp, _i64, _vp, _vp, _vp, _i64, _vp, _i64, _vp, _vp, _vp, _i64, _i, _vp, _i, _i, _i, _i, _vp]),
-    'gin_upsample_bf16': (_i, [_vp, _vp, _vp, _i, _vp, _vp, _i, _i, _vp]),
+    'gin_bn_eval_bwd_ws_bytes': (_sz, [_i]),
+    'gin_bn_eval_bwd': (_i, [_vp, _i64, _vp, _vp, _i64, _i, _vp, _vp, _vp, _i64, _vp, _i64, _vp, _i, _i, _i, _i, _vp]),
+    'gin_bn_eval_bwd_pair': (_i, [_vp, _i64, _vp, _vp, _i64, _vp, _vp, _vp, _i64, _vp, _i64, _vp, _vp, _vp, _i64, _i, _vp, _i, _i, _i, _i, _vp]),
+    'gin_upsample_bf16':(_i, [_vp, _vp, _vp, _i, _vp, _vp, _i, _i, _vp]),
     'gin_upsample_fwd': (_i, [_vp, _vp, _vp, _vp, _i, _i, _vp]),
     'gin_upsample_bwd': (_i, [_vp, _vp, _vp, _vp, _i, _i, _vp]),
     'gin_reparam_fwd': (_i, [_vp, _vp, _vp, _vp, _i64, _u64, _u64, _vp]),

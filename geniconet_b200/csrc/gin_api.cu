@@ -798,6 +798,64 @@ int gin_bn_act_bwd_pair(const float* dout, int64_t ldg, const void* mask_b, cons
   return check_launch("bn_bwd_apply2");
 }
 
+// ------------------------------------------------------------------ eval-mode BatchNorm backward (frozen statistics)
+size_t gin_bn_eval_bwd_ws_bytes(int C) { return C <= 0 ? 0 : (size_t)gin::bn::MAX_CTAS * 3 * C * 4; }
+
+static bool eval_bwd_shape_ok(int C) { return bn_shape_ok(C) && C <= gin::bn::CST_MAX_C; }
+
+int gin_bn_eval_bwd(const float* dout, int64_t ldg, const void* mask_b, const void* y, int64_t ld, int y_fp16, const float* stat, float* bsum,
+                    void* dy_b, int64_t ldo, float* dy_f, int64_t ldf, void* ws, int B, int level, int C, int relu_from_y, void* stream) {
+  cudaStream_t st = (cudaStream_t)stream;
+  if (!dout || !y || !stat || (!dy_b && !dy_f) || (bsum && !ws) || B <= 0 || level < 0 || level > 9 || !eval_bwd_shape_ok(C))
+    return fail(GIN_ERR_ARG, "gin_bn_eval_bwd: bad argument (C/8 must divide 256, C <= %d)", gin::bn::CST_MAX_C);
+  if (ldg < C || ld < C || (dy_b && ldo < C) || (dy_f && ldf < C) || ((ldg | ld | (dy_b ? ldo : 0) | (dy_f ? ldf : 0)) & 7))
+    return fail(GIN_ERR_ARG, "gin_bn_eval_bwd: bad row stride (each must be >= C and a multiple of 8)");
+  const int n = 1 << level, P = 10 << (2 * level);
+  const long long rows = (long long)B * P;
+  const gin::bn::Src sy{reinterpret_cast<const float*>(y), (long long)ld, y_fp16 ? 1 : 0};
+  const __nv_bfloat16* mask = relu_from_y ? nullptr : reinterpret_cast<const __nv_bfloat16*>(mask_b);
+  const int from_y = relu_from_y ? 1 : 0;
+  const int ctas = gin::bn::grid_for_rows((rows + (dy_b ? 2LL * B : 0)) * (C >> 3));
+  float* part = reinterpret_cast<float*>(ws);
+  __nv_bfloat16* dyb = reinterpret_cast<__nv_bfloat16*>(dy_b);
+  auto k = bsum ? (y_fp16 ? gin::bn::eval_bwd_kernel<true, true> : gin::bn::eval_bwd_kernel<false, true>)
+                : (y_fp16 ? gin::bn::eval_bwd_kernel<true, false> : gin::bn::eval_bwd_kernel<false, false>);
+  gin::launch_pdl(k, dim3(ctas), dim3(256), 0, st, dout, (long long)ldg, mask, sy, stat, dyb, (long long)ldo, dy_f, (long long)ldf, part, n, B, P, C, from_y);
+  int rc = check_launch("bn_eval_bwd");
+  if (rc || !bsum) return rc;
+  gin::launch_pdl(gin::bn::eval_bwd_final_kernel, dim3(C / 8), dim3(256), 0, st, (const float*)part, ctas, 2, C, stat, bsum, (const float*)nullptr,
+                  (float*)nullptr);
+  return check_launch("bn_eval_bwd_final");
+}
+
+int gin_bn_eval_bwd_pair(const float* dout, int64_t ldg, const void* mask_b, const void* yA, int64_t ldA, const float* statA, float* bsumA,
+                         void* dyA_b, int64_t ldoA, const void* yB, int64_t ldB, const float* statB, float* bsumB, void* dyB_b, int64_t ldoB,
+                         int y_fp16, void* ws, int B, int level, int C, int relu_from_y, void* stream) {
+  cudaStream_t st = (cudaStream_t)stream;
+  if (!dout || !yA || !yB || !statA || !statB || !dyA_b || !dyB_b || ((bsumA || bsumB) && !ws) || B <= 0 || level < 0 || level > 9 ||
+      !eval_bwd_shape_ok(C))
+    return fail(GIN_ERR_ARG, "gin_bn_eval_bwd_pair: bad argument (C/8 must divide 256, C <= %d)", gin::bn::CST_MAX_C);
+  if (ldg < C || ldA < C || ldB < C || ldoA < C || ldoB < C || ((ldg | ldA | ldB | ldoA | ldoB) & 7))
+    return fail(GIN_ERR_ARG, "gin_bn_eval_bwd_pair: bad row stride (each must be >= C and a multiple of 8)");
+  const int n = 1 << level, P = 10 << (2 * level);
+  const long long rows = (long long)B * P;
+  const gin::bn::Src sA{reinterpret_cast<const float*>(yA), (long long)ldA, y_fp16 ? 1 : 0}, sB{reinterpret_cast<const float*>(yB), (long long)ldB, y_fp16 ? 1 : 0};
+  const __nv_bfloat16* mask = relu_from_y ? nullptr : reinterpret_cast<const __nv_bfloat16*>(mask_b);
+  const int from_y = relu_from_y ? 1 : 0;
+  const bool red = bsumA || bsumB;
+  const int ctas = gin::bn::grid_for_rows((rows + 2LL * B) * (C >> 3));
+  float* part = reinterpret_cast<float*>(ws);
+  __nv_bfloat16 *da = reinterpret_cast<__nv_bfloat16*>(dyA_b), *db = reinterpret_cast<__nv_bfloat16*>(dyB_b);
+  auto k = red ? (y_fp16 ? gin::bn::eval_bwd2_kernel<true, true> : gin::bn::eval_bwd2_kernel<false, true>)
+               : (y_fp16 ? gin::bn::eval_bwd2_kernel<true, false> : gin::bn::eval_bwd2_kernel<false, false>);
+  gin::launch_pdl(k, dim3(ctas), dim3(256), 0, st, dout, (long long)ldg, mask, sA, statA, sB, statB, da, (long long)ldoA, db, (long long)ldoB, part, n, B,
+                  P, C, from_y);
+  int rc = check_launch("bn_eval_bwd2");
+  if (rc || !red) return rc;
+  gin::launch_pdl(gin::bn::eval_bwd_final_kernel, dim3(C / 8), dim3(256), 0, st, (const float*)part, ctas, 3, C, statA, bsumA, statB, bsumB);
+  return check_launch("bn_eval_bwd_final");
+}
+
 // ------------------------------------------------------------------ optimizer step (run.py:446, 250)
 int gin_adam_chunk(void) { return gin::adam::CHUNK; }
 

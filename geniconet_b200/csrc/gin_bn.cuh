@@ -968,5 +968,220 @@ __global__ void __launch_bounds__(256) pole_mean_kernel(const float* __restrict_
   }
 }
 
+// ------------------------------------------------------------------------------------------------ eval mode backward (frozen BatchNorm)
+// out = relu(bn(y) [+ bn'(y')]) with the running statistics: dy = scale * g does not depend on any reduction, so the gradient
+// copies and the sums come out of ONE streaming pass (the training backward needs a reduction pass first).  Same thread layout,
+// register budget (4 CTAs of 256 threads per SM) and shared-memory constants as bwd_apply_kernel / bwd_reduce2_kernel.  The
+// ReLU mask is read (mask != null, from_y == 0) or re-evaluated with relu_from_y / relu_from_y2, bit for bit act_fwd_kernel.
+// RED: partial[blk][NS][C] = sum g | sum g*yhatA [| sum g*yhatB]  (main rows only; eval_bwd_final_kernel adds them up).
+// dy = __fmul_rn(scale, g), and the pole-mean rows are fmaf(0.2, dy, .) over the five ring pixels from 0: the same sum, in the
+// same order, as cast_bf16_kernel over the fp32 dy.
+
+// constants of eval_bwd_kernel: 0 scale, 1 shift, 2 mean
+template <bool F16, bool RED>
+__global__ void __launch_bounds__(256, 4)
+eval_bwd_kernel(const float* __restrict__ dout, long long ldg, const __nv_bfloat16* __restrict__ mask, Src y, const float* __restrict__ stat,
+                __nv_bfloat16* __restrict__ dy_b, long long ldo, float* __restrict__ dy_f, long long ldf, float* __restrict__ partial, int nlat,
+                int B, int P, int C, int from_y) {
+  GIN_PDL_SYNC();
+  __shared__ __align__(16) float cst[3][2][32][4];
+  for (int ch = threadIdx.x; ch < C; ch += 256) { cst_put(cst, 0, ch, stat[2 * C + ch]); cst_put(cst, 1, ch, stat[3 * C + ch]); cst_put(cst, 2, ch, stat[ch]); }
+  __syncthreads();
+  const int C8 = C >> 3, sh = log2_pow2(C8), c8 = threadIdx.x & (C8 - 1), c = c8 * 8;
+  const uint32_t cb = (uint32_t)__cvta_generic_to_shared(&cst[0][0][c8][0]);
+  const long long rows = (long long)B * P, n_main = rows << sh, n_all = n_main + (dy_b ? (2LL * B) << sh : 0);
+  float s0[8], s1[8];
+#pragma unroll
+  for (int k = 0; k < 8; ++k) s0[k] = s1[k] = 0.f;
+  for (long long i = blockIdx.x * 256LL + threadIdx.x; i < n_all; i += gridDim.x * 256LL) {
+    const long long row = i >> sh;
+    float o[8], g[8], k8[8];
+    if (i < n_main) {
+      masked_grad(dout, ldg, mask, from_y, row, c, C, g);
+      if (RED || from_y) ld8_y<F16>(y, row, c, o);
+      if (from_y) relu_from_y<0, 1>(cb, o, g);
+      if (RED) {
+        lds8<2>(cb, k8);
+#pragma unroll
+        for (int k = 0; k < 8; ++k) { s0[k] += g[k]; s1[k] = fmaf(g[k], o[k] - k8[k], s1[k]); }
+      }
+      lds8<0>(cb, k8);
+#pragma unroll
+      for (int k = 0; k < 8; ++k) o[k] = __fmul_rn(k8[k], g[k]);
+      if (dy_f) st8(dy_f + row * ldf + c, o);
+    } else {
+      const int j = (int)(row - rows), sample = j >> 1, pole = j & 1;
+#pragma unroll
+      for (int k = 0; k < 8; ++k) o[k] = 0.f;
+      for (int e = 0; e < 5; ++e) {
+        const long long r = (long long)sample * P + ring_pixel(nlat, pole, e);
+        masked_grad(dout, ldg, mask, from_y, r, c, C, g);
+        if (from_y) {
+          float t[8];
+          ld8_y<F16>(y, r, c, t);
+          relu_from_y<0, 1>(cb, t, g);
+        }
+        lds8<0>(cb, k8);
+#pragma unroll
+        for (int k = 0; k < 8; ++k) o[k] = fmaf(0.2f, __fmul_rn(k8[k], g[k]), o[k]);
+      }
+    }
+    if (dy_b) st8_bf16(dy_b + row * ldo + c, o);
+  }
+  if constexpr (RED) {
+    float inv[8];
+    ld8(stat + C + c, inv);
+#pragma unroll
+    for (int k = 0; k < 8; ++k) s1[k] *= inv[k];
+    block_partials(s0, s1, C, partial);
+  }
+}
+
+// Sums of three per-thread vectors over a CTA in two steps, so that the vectors can die in between: stash_partials3 puts this
+// thread's values into shared memory, finish_partials3 (once every thread stashed) writes partial[blockIdx][3][C].
+GIN_DEVINL float (*part3_smem())[256][9] {
+  __shared__ float part[3][256][9];
+  return part;
+}
+GIN_DEVINL void stash_partials3(const float s0[8], const float s1[8], const float s2[8]) {
+  float (*part)[256][9] = part3_smem();
+#pragma unroll
+  for (int k = 0; k < 8; ++k) { part[0][threadIdx.x][k] = s0[k]; part[1][threadIdx.x][k] = s1[k]; part[2][threadIdx.x][k] = s2[k]; }
+}
+GIN_DEVINL void finish_partials3(int C, float* __restrict__ partial) {
+  float (*part)[256][9] = part3_smem();
+  __syncthreads();
+  const int C8 = C >> 3;
+  float* mine = partial + (size_t)blockIdx.x * 3 * C;
+  for (int i = threadIdx.x; i < 3 * C; i += 256) {
+    const int w = i / C, cc = i - w * C, g8 = cc >> 3, k = cc & 7;
+    float acc = 0.f;
+    for (int t = g8; t < 256; t += C8) acc += part[w][t][k];
+    mine[i] = acc;
+  }
+}
+
+// out = relu(bnA(yA) + bnB(yB)); constants: 0 scaleA, 1 scaleB, 2 shiftA + shiftB, 3 meanA, 4 meanB
+template <bool F16, bool RED>
+__global__ void __launch_bounds__(256, 4)
+eval_bwd2_kernel(const float* __restrict__ dout, long long ldg, const __nv_bfloat16* __restrict__ mask, Src yA, const float* __restrict__ statA,
+                 Src yB, const float* __restrict__ statB, __nv_bfloat16* __restrict__ dyA, long long ldoA, __nv_bfloat16* __restrict__ dyB,
+                 long long ldoB, float* __restrict__ partial, int nlat, int B, int P, int C, int from_y) {
+  GIN_PDL_SYNC();
+  __shared__ __align__(16) float cst[5][2][32][4];
+  for (int ch = threadIdx.x; ch < C; ch += 256) {
+    cst_put(cst, 0, ch, statA[2 * C + ch]); cst_put(cst, 1, ch, statB[2 * C + ch]); cst_put(cst, 2, ch, statA[3 * C + ch] + statB[3 * C + ch]);
+    cst_put(cst, 3, ch, statA[ch]); cst_put(cst, 4, ch, statB[ch]);
+  }
+  __syncthreads();
+  const int C8 = C >> 3, sh = log2_pow2(C8), c8 = threadIdx.x & (C8 - 1), c = c8 * 8;
+  const uint32_t cb = (uint32_t)__cvta_generic_to_shared(&cst[0][0][c8][0]);
+  const long long rows = (long long)B * P, n_main = rows << sh, n_all = n_main + ((2LL * B) << sh);
+  long long i = blockIdx.x * 256LL + threadIdx.x;
+  {
+    // the pixel rows (every one of them comes before the pole rows in the grid-stride order): the sums are live only here
+    float s0[8], s1[8], s2[8];
+#pragma unroll
+    for (int k = 0; k < 8; ++k) s0[k] = s1[k] = s2[k] = 0.f;
+    for (; i < n_main; i += gridDim.x * 256LL) {
+      const long long row = i >> sh;
+      float g[8], oA[8], oB[8], k8[8];
+      masked_grad(dout, ldg, mask, from_y, row, c, C, g);
+      if (RED || from_y) { ld8_y<F16>(yA, row, c, oA); ld8_y<F16>(yB, row, c, oB); }
+      if (from_y) relu_from_y2<0, 1, 2>(cb, oA, oB, g);
+      if (RED) {
+        lds8<3>(cb, k8);
+#pragma unroll
+        for (int k = 0; k < 8; ++k) { s0[k] += g[k]; s1[k] = fmaf(g[k], oA[k] - k8[k], s1[k]); }
+        lds8<4>(cb, k8);
+#pragma unroll
+        for (int k = 0; k < 8; ++k) s2[k] = fmaf(g[k], oB[k] - k8[k], s2[k]);
+      }
+      lds8<0>(cb, k8);
+#pragma unroll
+      for (int k = 0; k < 8; ++k) oA[k] = __fmul_rn(k8[k], g[k]);
+      st8_bf16(dyA + row * ldoA + c, oA);
+      lds8<1>(cb, k8);
+#pragma unroll
+      for (int k = 0; k < 8; ++k) oB[k] = __fmul_rn(k8[k], g[k]);
+      st8_bf16(dyB + row * ldoB + c, oB);
+    }
+    if constexpr (RED) {
+      float iA[8], iB[8];
+      ld8(statA + C + c, iA); ld8(statB + C + c, iB);
+#pragma unroll
+      for (int k = 0; k < 8; ++k) { s1[k] *= iA[k]; s2[k] *= iB[k]; }
+      stash_partials3(s0, s1, s2);
+    }
+  }
+  for (; i < n_all; i += gridDim.x * 256LL) {
+    // pole-mean rows (2B of them): one BatchNorm after the other keeps the register count of the pixel rows
+    const long long row = i >> sh;
+    const int j = (int)(row - rows), sample = j >> 1, pole = j & 1;
+    float o[8], g[8], k8[8];
+#pragma unroll
+    for (int k = 0; k < 8; ++k) o[k] = 0.f;
+    for (int e = 0; e < 10; ++e) {
+      const long long r = (long long)sample * P + ring_pixel(nlat, pole, e % 5);
+      masked_grad(dout, ldg, mask, from_y, r, c, C, g);
+      if (from_y) {
+        float t[8], u[8];
+        ld8_y<F16>(yA, r, c, t);
+        ld8_y<F16>(yB, r, c, u);
+        relu_from_y2<0, 1, 2>(cb, t, u, g);
+      }
+      if (e < 5) lds8<0>(cb, k8);
+      else lds8<1>(cb, k8);
+#pragma unroll
+      for (int k = 0; k < 8; ++k) o[k] = fmaf(0.2f, __fmul_rn(k8[k], g[k]), o[k]);
+      if (e == 4) {
+        st8_bf16(dyA + row * ldoA + c, o);
+#pragma unroll
+        for (int k = 0; k < 8; ++k) o[k] = 0.f;
+      }
+    }
+    st8_bf16(dyB + row * ldoB + c, o);
+  }
+  if constexpr (RED) finish_partials3(C, partial);
+}
+
+// bsum[3][C] = dbeta = sum g, dgamma = sum g*yhat, conv-bias gradient = scale * sum g, from partial[nblocks][ns][C] (ns = 2: one
+// BatchNorm, rows g | g*yhatA; ns = 3: a pair, rows g | g*yhatA | g*yhatB); bsumA / bsumB may be NULL.  Fixed-order fp64 sums.
+// grid = C/8, block = 256 (8 row groups x 32 (sum, channel) lanes).
+__global__ void __launch_bounds__(256)
+eval_bwd_final_kernel(const float* __restrict__ partial, int nblocks, int ns, int C, const float* __restrict__ statA, float* __restrict__ bsumA,
+                      const float* __restrict__ statB, float* __restrict__ bsumB) {
+  GIN_PDL_SYNC();
+  __shared__ double red[8][33];
+  const int j = threadIdx.x & 31, rg = threadIdx.x >> 5;
+  const int k = j >> 3, c = blockIdx.x * 8 + (j & 7);
+  double acc = 0.0;
+  if (k < ns && c < C) {
+    float v[(MAX_CTAS + 7) / 8];
+#pragma unroll
+    for (int i = 0; i < (MAX_CTAS + 7) / 8; ++i) {
+      const int b = rg + 8 * i;
+      v[i] = b < nblocks ? __ldg(partial + ((size_t)b * ns + k) * C + c) : 0.f;
+    }
+#pragma unroll
+    for (int i = 0; i < (MAX_CTAS + 7) / 8; ++i) acc += (double)v[i];
+  }
+  red[rg][j] = acc;
+  __syncthreads();
+  if (threadIdx.x < 32 && k < ns && c < C) {
+    double t = 0.0;
+#pragma unroll
+    for (int r = 0; r < 8; ++r) t += red[r][threadIdx.x];
+    if (k == 0) {                 // sum g: shared by both BatchNorms of a pair
+      if (bsumA) { bsumA[c] = (float)t; bsumA[2 * C + c] = (float)((double)statA[2 * C + c] * t); }
+      if (bsumB) { bsumB[c] = (float)t; bsumB[2 * C + c] = (float)((double)statB[2 * C + c] * t); }
+    } else if (k == 1) {
+      if (bsumA) bsumA[C + c] = (float)t;
+    } else if (bsumB) {
+      bsumB[C + c] = (float)t;
+    }
+  }
+}
+
 }  // namespace bn
 }  // namespace gin

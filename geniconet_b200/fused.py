@@ -18,8 +18,11 @@ from (plus the fp32 conv outputs BatchNorm needs):
 
 Parameters stay where models.py puts them (conv00.weight, icobn00.weight, ...), so state dicts are unchanged; BatchNorm running
 statistics are updated as torch does.  With grad disabled, infer_chain runs the same chains forward-only (eval mode: BatchNorm in
-the conv epilogue, DESIGN "Inference"); eval mode with grad enabled runs the modules one by one.
-A conv bias that feeds a BatchNorm has a mathematically zero gradient; the fused path returns exactly zero for it.
+the conv epilogue, DESIGN "Inference").  Eval mode with grad enabled runs run_frozen_chain (opt-in, DESIGN "Frozen BatchNorm"):
+the training chain's forward kernels with the running statistics, nothing updated, and a backward of one streaming pass per
+BatchNorm (gin_bn_eval_bwd / _pair) that computes weight gradients only for weights that need them.
+In train mode a conv bias that feeds a BatchNorm has a mathematically zero gradient and the training chain returns exactly zero
+for it; in eval mode its gradient is scale * sum(g), which the frozen chain returns.
 """
 import torch
 
@@ -643,6 +646,205 @@ def infer_chain(x, mods, want_operand=False):
         level, C = lvl, cout
     n = 2 ** level
     return act_f.view(B, 5 * n, 2 * n, C).permute(0, 3, 1, 2), (act_b if want_operand else None)
+
+
+# ------------------------------------------------------------------------------------------------ frozen BatchNorm (eval mode with grad)
+def frozen_supported(mods):
+    """chain_supported, and every BatchNorm at most 256 wide (gin_bn_eval_bwd keeps its constants in shared memory)."""
+    return chain_supported(mods) and all(bn.num_features <= 256 for bn, _ in eval_pairs(mods))
+
+
+def _own_consts(pairs):
+    """The eval constants of `pairs` (see _eval_consts) in a buffer of this call's own: _bn_table's buffer is shared by every call
+    on the same parameters and rewritten by each, while a backward must see the constants of its own forward."""
+    _, _, _, buf, views = _bn_table(pairs)
+    _eval_consts(pairs)
+    own = buf.clone()
+    return [tuple(own[v.storage_offset():v.storage_offset() + v.numel()] for v in vs) for vs in views]
+
+
+def _eval_bwd(dout, y, col0, ld, stat, B, level, C, bsum, dy_b=None, dy_b_col=0, ldo=0, want_f=False):
+    """gin_bn_eval_bwd with the ReLU mask re-evaluated from y.  Returns dy_f (or None); writes bsum [3C] when given and the bf16
+    gradient copy into dy_b[:, dy_b_col:dy_b_col+C]."""
+    dev = dout.device
+    dy_f = _empty((B * _P(level), C), torch.float32, dev) if want_f else None
+    ws = _empty(L.gin_bn_eval_bwd_ws_bytes(C), torch.uint8, dev) if bsum is not None else None
+    ptr = lambda t: t.data_ptr() if t is not None else None
+    _lib.check(L.gin_bn_eval_bwd(dout.data_ptr(), C, None, y.data_ptr() + y.element_size() * col0, ld, 1 if y.dtype == torch.float16 else 0,
+                                 stat.data_ptr(), ptr(bsum), (dy_b.data_ptr() + 2 * dy_b_col) if dy_b is not None else None, ldo, ptr(dy_f), C,
+                                 ptr(ws), B, level, C, 1, _stream()), 'gin_bn_eval_bwd')
+    return dy_f
+
+
+def _take_sums(grads, need, k, bs, C):
+    """conv bias, gamma, beta (parameters k + 1 .. k + 3 of chain_params) from bsum = [dbeta | dgamma | conv-bias gradient]"""
+    for kk, g in ((k + 1, bs[2 * C:]), (k + 2, bs[C:2 * C]), (k + 3, bs[:C])):
+        grads[kk] = g if need[kk] else None
+
+
+class _FrozenChain(torch.autograd.Function):
+    """The chain with every BatchNorm in eval mode and grad enabled: the training chain's forward kernels with the running-statistic
+    constants (nothing is updated), and a backward through gin_bn_eval_bwd(_pair).  Weight gradients are computed only for weights
+    that need them; BatchNorm sums only where gamma, beta or the conv bias needs a gradient."""
+
+    @staticmethod
+    def forward(ctx, x, mods, *params):
+        dev, B = x.device, x.shape[0]
+        need = [p.requires_grad for p in params]
+        consts = iter(_own_consts(eval_pairs(mods)))
+        saved, i, k = [], 0, 0                 # k: index of the stage's first parameter in `params`
+        if isinstance(mods[0], IcoConvS2S):
+            conv = mods[0]
+            level, C = conv.subdivisions, conv.out_features
+            plan, packed, xs, strides, y, _ = _stem_conv(x, conv)
+            stat = next(consts)[2]
+            # the stem's output is the first block's input: its bf16 twin is that block's wgrad operand
+            blk = mods[3]
+            want_w = blk.conv00.weight.requires_grad or blk.conv10.weight.requires_grad
+            act_b, _, act_w = _bn_act(y, 0, C, stat, None, 0, 0, None, B, level, C, want_w=want_w)
+            saved.append(dict(kind='stem', plan=plan, xs=xs, strides=strides, y=y, stat=stat, C=C, level=level, packed=packed, k=0))
+            act_f, i, k = None, 3, 4
+        else:
+            blk = mods[0]
+            level, C = blk.conv00.subdivisions - (0 if blk._down else 1), blk.conv00.in_features
+            from .ico_conv import as_channels_last, cast_bf16
+            xl = as_channels_last(x)
+            act_f = xl.permute(0, 2, 3, 1).reshape(-1, C)
+            if blk._down:
+                plan = get_plan(_lib.PLAN_HEXCONV, level, 1, blk.conv00.corner_mode, dev)
+                act_b = cast_bf16(xl, plan, 0, level)
+                act_w = (cast_bf16(xl, plan, 2, level) if _DUAL else act_b) if (blk.conv00.weight.requires_grad or blk.conv10.weight.requires_grad) else None
+            saved.append(dict(kind='input', level=level, C=C))
+        jobs = []
+        for blk in mods[i:]:
+            jobs.append((blk.conv00.weight.detach().contiguous(), blk.conv10.weight.detach().contiguous(), blk.conv00.in_features))
+            jobs.append((blk.conv01.weight.detach().contiguous(), None, blk.conv01.in_features))
+        packs = _pack_many(jobs)
+        last = len(mods) - 1
+        for j in range(i, len(mods)):
+            blk = mods[j]
+            cm = blk.conv00.corner_mode
+            cin, cout = blk.conv00.in_features, blk.conv00.out_features
+            w_cat = blk.conv00.weight.requires_grad or blk.conv10.weight.requires_grad
+            st = dict(kind='down' if blk._down else 'up', cin=cin, cout=cout, in_level=level, k=k)
+            if blk._down:
+                lvl = level - 1
+                plan_a = get_plan(_lib.PLAN_HEXCONV, level, 2, cm, dev)
+                a_b, a_w = act_b, act_w
+            else:
+                lvl = level + 1
+                up_plan = get_plan(_lib.PLAN_UPSAMPLE, level, 1, blk.upsample00.corner_mode, dev)
+                plan_a = get_plan(_lib.PLAN_HEXCONV, lvl, 1, cm, dev)
+                a_b = _empty((B * _P(lvl) + 2 * B, cin), torch.bfloat16, dev)
+                a_w = (_empty((B * _P(lvl) + 2 * B, cin), torch.bfloat16, dev) if _DUAL else a_b) if w_cat else None
+                _lib.check(L.gin_upsample_bf16(up_plan.host_ptr, up_plan.dev_ptr, act_f.data_ptr(), 1, a_b.data_ptr(),
+                                               a_w.data_ptr() if (_DUAL and a_w is not None) else None, B, cin, _stream()), 'gin_upsample_bf16')
+                st['up_plan'] = up_plan
+            plan_b = get_plan(_lib.PLAN_HEXCONV, lvl, 1, cm, dev)
+            pk_cat, pk01 = packs[2 * (j - i)], packs[2 * (j - i) + 1]
+            (_, _, stat00), (_, _, stat10), (_, _, stat01) = next(consts), next(consts), next(consts)
+            ycat, _ = _conv_fwd(plan_a, a_b, pk_cat, blk.conv00.bias.detach(), B, cin, 2 * cout, _P(lvl), bias1=blk.conv10.bias.detach())
+            h_b, _, h_w = _bn_act(ycat, 0, 2 * cout, stat00, None, 0, 0, None, B, lvl, cout, want_w=blk.conv01.weight.requires_grad)
+            y01, _ = _conv_fwd(plan_b, h_b, pk01, blk.conv01.bias.detach(), B, cout, cout, _P(lvl))
+            is_last = j == last
+            keep_f = is_last or not mods[j + 1]._down
+            nxt_w = not is_last and mods[j + 1]._down and (mods[j + 1].conv00.weight.requires_grad or mods[j + 1].conv10.weight.requires_grad)
+            # an Up block upsamples from the fp32 map: the operand copy is made only for a Down block
+            out_b, out_f, out_w = _bn_act(y01, 0, cout, stat01, ycat, cout, 2 * cout, stat10, B, lvl, cout, want_b=not keep_f, want_f=keep_f,
+                                          want_w=nxt_w)
+            st.update(plan_a=plan_a, plan_b=plan_b, a_w=a_w if w_cat else None, h_w=h_w if blk.conv01.weight.requires_grad else None,
+                      pk_cat=pk_cat, pk01=pk01, ycat=ycat, y01=y01, stat00=stat00, stat01=stat01, stat10=stat10, level=lvl)
+            saved.append(st)
+            act_b, act_w, act_f, level, C = out_b, out_w, out_f, lvl, cout
+            k += 12
+        ctx.saved, ctx.B, ctx.need, ctx.x_needs_grad = saved, B, need, x.requires_grad
+        n = 2 ** level
+        return act_f.view(B, 5 * n, 2 * n, C).permute(0, 3, 1, 2)
+
+    @staticmethod
+    def backward(ctx, d_out):
+        B, saved, need = ctx.B, ctx.saved, ctx.need
+        from .ico_conv import as_channels_last
+        d = as_channels_last(d_out).permute(0, 2, 3, 1).reshape(-1, d_out.shape[1])
+        if not d.is_contiguous():
+            d = d.contiguous()
+        grads = [None] * len(need)
+        dx = None
+        # upstream[s]: something before stage s (an earlier stage's parameter, or x) needs a gradient
+        upstream, acc = [], ctx.x_needs_grad
+        for st in saved:
+            upstream.append(acc)
+            if st['kind'] != 'input':
+                acc = acc or any(need[st['k']:st['k'] + (4 if st['kind'] == 'stem' else 12)])
+        dev = d.device
+        sums = lambda k, C: _empty(3 * C, torch.float32, dev) if any(need[k + 1:k + 4]) else None
+        for s in range(len(saved) - 1, -1, -1):
+            st = saved[s]
+            if st['kind'] in ('down', 'up'):
+                cin, cout, lvl, k = st['cin'], st['cout'], st['level'], st['k']
+                # parameter order of chain_params: conv00 (w, b, gamma, beta) at k, conv01 at k + 4, conv10 at k + 8
+                bs00, bs01, bs10 = sums(k, cout), sums(k + 4, cout), sums(k + 8, cout)
+                dycat_b = torch.empty((B * _P(lvl) + 2 * B, 2 * cout), dtype=torch.bfloat16, device=dev)
+                dy01_b = torch.empty((B * _P(lvl) + 2 * B, cout), dtype=torch.bfloat16, device=dev)
+                ws = _empty(L.gin_bn_eval_bwd_ws_bytes(cout), torch.uint8, dev) if (bs01 is not None or bs10 is not None) else None
+                ycat = st['ycat']
+                ptr = lambda t: t.data_ptr() if t is not None else None
+                _lib.check(L.gin_bn_eval_bwd_pair(d.data_ptr(), cout, None, st['y01'].data_ptr(), cout, st['stat01'].data_ptr(), ptr(bs01),
+                                                  dy01_b.data_ptr(), cout, ycat.data_ptr() + ycat.element_size() * cout, 2 * cout,
+                                                  st['stat10'].data_ptr(), ptr(bs10), dycat_b.data_ptr() + 2 * cout, 2 * cout,
+                                                  1 if ycat.dtype == torch.float16 else 0, ptr(ws), B, lvl, cout, 1, _stream()), 'gin_bn_eval_bwd_pair')
+                if need[k + 4]:
+                    grads[k + 4] = _conv_wgrad(st['plan_b'], st['h_w'], dy01_b, B, cout, cout)
+                d_h = _conv_dgrad(st['plan_b'], dy01_b, st['pk01'], B, cout, cout, _P(lvl))
+                _eval_bwd(d_h, ycat, 0, 2 * cout, st['stat00'], B, lvl, cout, bs00, dycat_b, 0, 2 * cout)
+                if need[k] or need[k + 8]:
+                    dWcat = _conv_wgrad(st['plan_a'], st['a_w'], dycat_b, B, cin, 2 * cout)
+                    grads[k], grads[k + 8] = (dWcat[:cout] if need[k] else None), (dWcat[cout:] if need[k + 8] else None)
+                for kk, bs in ((k, bs00), (k + 4, bs01), (k + 8, bs10)):
+                    if bs is not None:
+                        _take_sums(grads, need, kk, bs, cout)
+                if not upstream[s]:
+                    break
+                p_in = _P(lvl + 1) if st['kind'] == 'down' else _P(lvl)
+                d = _conv_dgrad(st['plan_a'], dycat_b, st['pk_cat'], B, cin, 2 * cout, p_in)
+                if st['kind'] == 'up':
+                    upp = st['up_plan']
+                    d_prev = torch.empty((B * _P(st['in_level']), cin), dtype=torch.float32, device=dev)
+                    _lib.check(L.gin_upsample_bwd(upp.host_ptr, upp.dev_ptr, d.data_ptr(), d_prev.data_ptr(), B, cin, _stream()), 'gin_upsample_bwd')
+                    d = d_prev
+            elif st['kind'] == 'stem':
+                C, lvl = st['C'], st['level']
+                bs = sums(0, C)
+                if not (need[0] or bs is not None or ctx.x_needs_grad):
+                    break
+                dy_f = _eval_bwd(d, st['y'], 0, C, st['stat'], B, lvl, C, bs, want_f=True)
+                plan = st['plan']
+                sb, sp, sc = st['strides']
+                if need[0]:
+                    dW = torch.empty((C, 3, 7), dtype=torch.float32, device=dev)
+                    ws = torch.empty(L.gin_hexconv_wgrad_ws_bytes(3, C), dtype=torch.uint8, device=dev)
+                    _lib.check(L.gin_hexconv_wgrad(plan.host_ptr, plan.dev_ptr, st['xs'].data_ptr(), sb, sp, sc, dy_f.data_ptr(), dW.data_ptr(), None,
+                                                   ws.data_ptr(), B, 3, C, _lib.IMPL_AUTO, _stream()), 'gin_hexconv_wgrad')
+                    grads[0] = dW
+                if bs is not None:
+                    _take_sums(grads, need, 0, bs, C)
+                if ctx.x_needs_grad:
+                    n = 2 ** lvl
+                    dxs = torch.empty((B * _P(lvl), 3), dtype=torch.float32, device=dev)
+                    _lib.check(L.gin_hexconv_dgrad(plan.host_ptr, plan.dev_ptr, dy_f.data_ptr(), st['packed'].data_ptr(), dxs.data_ptr(), B, 3, C,
+                                                   _lib.IMPL_SIMT, _stream()), 'gin_hexconv_dgrad')
+                    dx = dxs.view(B, 5 * n, 2 * n, 3).permute(0, 3, 1, 2)
+            else:
+                n = 2 ** st['level']
+                dx = d.view(B, 5 * n, 2 * n, st['C']).permute(0, 3, 1, 2)
+        return (dx, None) + tuple(grads)
+
+
+def run_frozen_chain(x, mods):
+    """Forward of the module list `mods` (see frozen_supported) with every BatchNorm in eval mode, differentiable: the running
+    statistics are used and left untouched, gradients flow to x and to every parameter that requires one."""
+    mods = list(mods)
+    return _FrozenChain.apply(x, mods, *chain_params(mods))
 
 
 def latent_supported(mu, logvar):

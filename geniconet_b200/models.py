@@ -28,15 +28,25 @@ _HEAD = os.environ.get('GIN_HEAD', '1') != '0'           # the decoder head thro
 # Forward-only fused chains (fused.infer_chain) when grad is disabled (no_grad / inference_mode); opt-in: GIN_FUSED_INFER=1 or
 # set_fused(True, inference=True).
 _INFER = os.environ.get('GIN_FUSED_INFER', '0') == '1'
+# Fused chains with every BatchNorm in eval mode and grad enabled (fused.run_frozen_chain: frozen-statistics fine-tuning, latent
+# fitting, input gradients); opt-in: GIN_FUSED_FROZEN=1 or set_fused(True, frozen=True).
+_FROZEN = os.environ.get('GIN_FUSED_FROZEN', '0') == '1'
 
 
-def set_fused(flag, head=None, inference=None):
-    global _FUSED, _HEAD, _INFER
+def set_fused(flag, head=None, inference=None, frozen=None):
+    global _FUSED, _HEAD, _INFER, _FROZEN
     _FUSED = bool(flag)
     if head is not None:
         _HEAD = bool(head)
     if inference is not None:
         _INFER = bool(inference)
+    if frozen is not None:
+        _FROZEN = bool(frozen)
+
+
+def _bn_modes(tops):
+    """The set of `training` flags of every BatchNorm2d inside the modules `tops`."""
+    return {m.training for t in tops for m in t.modules() if isinstance(m, torch.nn.BatchNorm2d)}
 
 
 def _infer(mods, x, want_operand=False):
@@ -56,19 +66,49 @@ def _infer(mods, x, want_operand=False):
     return _fused.infer_chain(x, mods, want_operand)
 
 
+def _frozen(mods, x):
+    """fused.run_frozen_chain over `mods` (a Sequential, whose own hooks count too, or a list of modules) when the switch is on, grad
+    is enabled, every BatchNorm inside is in eval mode and no module inside has a forward hook; else None (the caller runs the
+    modules)."""
+    tops = [mods] if isinstance(mods, torch.nn.Module) else list(mods)
+    mods = list(mods)
+    if not (_FUSED and _FROZEN and torch.is_grad_enabled() and x.is_cuda and x.dtype == torch.float32):
+        return None
+    inner = [m for t in tops for m in t.modules()]
+    if any(m._forward_hooks or m._forward_pre_hooks for m in inner) or _bn_modes(tops) != {False}:
+        return None
+    if any(getattr(c, 'impl', 0) != 0 for c in inner if isinstance(c, IcoConvS2S)) or not _fused.frozen_supported(mods):
+        return None
+    return _fused.run_frozen_chain(x, mods)
+
+
 def _run(mods, x):
-    """nn.Sequential semantics over the module list, through the fused chain when possible."""
+    """nn.Sequential semantics over the module list, through a fused chain when possible.  With grad enabled the BatchNorms inside
+    decide: all in train mode -> the training chain, all in eval mode -> the frozen chain (when switched on), mixed -> the modules."""
     mods = list(mods)
     r = _infer(mods, x)
     if r is not None:
         return r[0]
-    if (_FUSED and x.is_cuda and x.dtype == torch.float32 and torch.is_grad_enabled() and all(m.training for m in mods)
+    if (_FUSED and x.is_cuda and x.dtype == torch.float32 and torch.is_grad_enabled() and _bn_modes(mods) == {True}
             and all(getattr(c, 'impl', 0) == 0 for m in mods for c in m.modules() if isinstance(c, IcoConvS2S))
             and _fused.chain_supported(mods)):
         return _fused.run_chain(x, mods)
+    r = _frozen(mods, x)
+    if r is not None:
+        return r
     for m in mods:
         x = m(x)
     return x
+
+
+def _body(seq, x):
+    """A split model's body `seq` (a Sequential) on x: through the forward-only or the frozen chain where one applies, else module by
+    module (the split models never take the training chain)."""
+    r = _infer(seq, x)
+    if r is not None:
+        return r[0]
+    r = _frozen(seq, x)
+    return r if r is not None else seq(x)
 
 BatchNorm2d = torch.nn.BatchNorm2d
 
@@ -226,8 +266,11 @@ class ico2ico(torch.nn.Module):
         self.decoder, self.enc2icoConv = createenc2ico(params['ico']['corner_mode'], params['ico2ico']['model'], self.subdivisions)
 
     def forward(self, x):
-        if isinstance(self.enc, torch.nn.Identity) and not self.enc._forward_hooks:
-            return _head(self.enc2icoConv, _run(list(self.encoder) + list(self.decoder), x))       # one fused chain through both halves
+        whole = list(self.encoder) + list(self.decoder)
+        # one fused chain through both halves, unless grad is enabled and the halves differ in BatchNorm mode (e.g. a frozen encoder
+        # under a trained decoder): then each half is a chain of its own
+        if isinstance(self.enc, torch.nn.Identity) and not self.enc._forward_hooks and (not torch.is_grad_enabled() or len(_bn_modes(whole)) < 2):
+            return _head(self.enc2icoConv, _run(whole, x))
         return _head(self.enc2icoConv, _run(self.decoder, self.enc(_run(self.encoder, x))))
 
 
@@ -237,8 +280,7 @@ class ico2enc(torch.nn.Module):
         self.encoder = createico2enc(params['ico']['corner_mode'], params['ico2ico']['model'], _top(params))
 
     def forward(self, x):
-        r = _infer(self.encoder, x)
-        return r[0] if r is not None else self.encoder(x)
+        return _body(self.encoder, x)
 
 
 class enc2ico(torch.nn.Module):
@@ -248,8 +290,7 @@ class enc2ico(torch.nn.Module):
         self.decoder, self.enc2icoConv = createenc2ico(params['ico']['corner_mode'], params['ico2ico']['model'], self.subdivisions)
 
     def forward(self, x):
-        r = _infer(self.decoder, x)
-        return _head(self.enc2icoConv, r[0] if r is not None else self.decoder(x))
+        return _head(self.enc2icoConv, _body(self.decoder, x))
 
 
 def _latent_head(params, level):
@@ -312,7 +353,9 @@ class ico2enc_vae(VAE):
     def encode(self, input):
         r = _infer(self.encoder, input, want_operand=True)
         if r is None:
-            h = self.encoder(input)
+            h = _frozen(self.encoder, input)
+            if h is None:
+                h = self.encoder(input)
         else:
             lat = _latent(r, self.mu, self.logvar, input)
             if lat is not None:
@@ -337,8 +380,7 @@ class enc2ico_vae(VAE):
         return torch.add(trn_mean, trn_logvar * torch.randn(trn_logvar.shape))
 
     def decode(self, z):
-        r = _infer(self.decoder, z)
-        return _head(self.final_layer, r[0] if r is not None else self.decoder(z))
+        return _head(self.final_layer, _body(self.decoder, z))
 
     def forward(self, x):
         return self.decode(x), torch.tensor([]), torch.tensor([])

@@ -166,4 +166,8 @@ class Adam(torch.optim.Optimizer):
             _lib.check(_lib.lib.gin_adam_step(t['dev'].data_ptr(), t['dev'].data_ptr() + tb['rows_bytes'], t['count'], t['chunks'], float(lr), lr_dev,
                                               float(b1), float(b2), float(group['eps']), float(group['weight_decay']), tb['ticket'].data_ptr(), _stream()),
                        'gin_adam_step')
+            # the kernel writes through raw pointers: bump the version counters as an in-place torch update would, so that caches
+            # keyed on (data_ptr, _version) -- IcoConvS2S's packed weights -- see the new values
+            for p in live:
+                torch.autograd.graph.increment_version(p)
         return loss

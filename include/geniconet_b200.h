@@ -316,6 +316,26 @@ typedef struct {
 } GinBnEvalEntry;
 int gin_bn_eval_consts(const void* table_dev, int count, int max_C, void* stream);
 
+/* ------------------------------------------------------------------ device: eval-mode BatchNorm backward ---- */
+/* Backward of out = relu(bn(y)) with bn in eval mode (running statistics; stat[4][C] as gin_bn_eval_consts writes it: running_mean,
+ * invstd, scale = gamma*invstd, shift): g = dout * (out > 0), dy = scale*g -- ONE streaming pass, no reduction ahead of it.
+ * The mask is re-evaluated from y and stat when relu_from_y != 0 (bit-identical to gin_bn_act_fwd(y, stat, relu = 1); mask_b is
+ * then ignored), else read from mask_b (a 16-bit copy of out, either format; NULL: no ReLU).
+ * dy is written as the bf16 copy dy_b [B*P + 2B][.] with row stride ldo (the pole-mean rows included, bit for bit what
+ * gin_cast_bf16(which = 1) makes of the fp32 dy) and / or as fp32 dy_f with row stride ldf.
+ * bsum (may be NULL: no reduction at all) = [3][C]: dbeta = sum g, dgamma = sum g*yhat (yhat = (y - running_mean)*invstd) and the
+ * gradient of the conv bias that feeds the BatchNorm, scale * sum g (not zero in eval mode).  Two-stage, fixed-order fp64 sums.
+ * C/8 divides 256 and C <= 256; every row stride >= C and a multiple of 8.  ws: gin_bn_eval_bwd_ws_bytes(C) when a sum is taken. */
+size_t gin_bn_eval_bwd_ws_bytes(int C);
+int gin_bn_eval_bwd(const float* dout, int64_t ldg, const void* mask_b, const void* y, int64_t ld, int y_fp16, const float* stat, float* bsum,
+                    void* dy_b, int64_t ldo, float* dy_f, int64_t ldf, void* ws, int B, int level, int C, int relu_from_y, void* stream);
+/* The residual output out = relu(bnA(yA) + bnB(yB)), both in eval mode: dout is read once, dyA_b / dyB_b are bf16 copies (pole
+ * rows included) with row strides ldoA / ldoB.  bsumA / bsumB [3][C] as above, each may be NULL; relu_from_y: the mask is
+ * re-evaluated exactly as gin_bn_act_fwd(yA, statA, yB, statB, relu = 1) computed out. */
+int gin_bn_eval_bwd_pair(const float* dout, int64_t ldg, const void* mask_b, const void* yA, int64_t ldA, const float* statA, float* bsumA,
+                         void* dyA_b, int64_t ldoA, const void* yB, int64_t ldB, const float* statB, float* bsumB, void* dyB_b, int64_t ldoB,
+                         int y_fp16, void* ws, int B, int level, int C, int relu_from_y, void* stream);
+
 /* number of kernel launches issued through this library since load (bench.py's gpu_launches) */
 int64_t gin_launch_count(void);
 
