@@ -27,7 +27,7 @@ for it; in eval mode its gradient is scale * sum(g), which the frozen chain retu
 import torch
 
 from . import _lib
-from .ico_conv import IcoConvS2S, IcoUpsampleS2S, get_plan, _stream, pixel_strides
+from .ico_conv import IcoConvS2S, get_plan, _stream, pixel_strides, as_channels_last, cast_bf16
 
 L = _lib.lib
 
@@ -88,15 +88,6 @@ def _pack(w, cin, cout):
     return packed
 
 
-def _pack_bf16(w0, w1, cin):
-    """bf16 tile images of [w0; w1] (concatenated output channels) without materialising the concatenation."""
-    c0, c1 = w0.shape[0], (w1.shape[0] if w1 is not None else 0)
-    packed = _empty(L.gin_hexconv_packed_bytes(cin, c0 + c1), torch.uint8, w0.device)
-    _lib.check(L.gin_hexconv_pack_weights_bf16(w0.data_ptr(), c0, w1.data_ptr() if w1 is not None else None, c1, packed.data_ptr(), cin, _stream()),
-               'gin_hexconv_pack_weights_bf16')
-    return packed
-
-
 def _pack_many(jobs):
     """jobs: list of (w0, w1 or None, cin) -> list of packed blobs (16-bit tile images only), ONE launch for all of them."""
     import ctypes
@@ -150,31 +141,17 @@ def _conv_dgrad(plan, dyb, packed, B, cin, cout, p_in):
     return dx
 
 
-def _conv_wgrad(plan, xb, dyb, B, cin, cout, side=None, out=None):
-    """dW [cout][cin][7] (written into `out` when given: a data-parallel bucket slot).  With `side` (a CUDA stream) the wgrad is
-    issued there: nothing on the rest of the backward pass depends on it, so the tensor-bound wgrad overlaps the memory-bound
-    BatchNorm backward kernels of the main stream."""
-    if side is None:
-        dW = out if out is not None else _empty((cout, cin, 7), torch.float32, xb.device)
-        ws = _empty(L.gin_hexconv_wgrad_ws_bytes(cin, cout), torch.uint8, xb.device)
-        _lib.check(L.gin_hexconv_wgrad_bf16(plan.host_ptr, plan.dev_ptr, xb.data_ptr(), dyb.data_ptr(), None, dW.data_ptr(), None, ws.data_ptr(),
-                                            B, cin, cout, _stream()), 'gin_hexconv_wgrad_bf16')
-        return dW
-    main = torch.cuda.current_stream()
-    side.wait_stream(main)                               # dyb (and xb) are complete on the main stream
-    with torch.cuda.stream(side):
-        dW = _empty((cout, cin, 7), torch.float32, xb.device)
-        ws = _empty(L.gin_hexconv_wgrad_ws_bytes(cin, cout), torch.uint8, xb.device)
-        _lib.check(L.gin_hexconv_wgrad_bf16(plan.host_ptr, plan.dev_ptr, xb.data_ptr(), dyb.data_ptr(), None, dW.data_ptr(), None, ws.data_ptr(),
-                                            B, cin, cout, side.cuda_stream), 'gin_hexconv_wgrad_bf16')
-    xb.record_stream(side)                               # their memory must not be recycled on the main stream while the side stream reads it
-    dyb.record_stream(side)
+def _conv_wgrad(plan, xb, dyb, B, cin, cout, out=None):
+    """dW [cout][cin][7] (written into `out` when given: a data-parallel bucket slot)."""
+    dW = out if out is not None else _empty((cout, cin, 7), torch.float32, xb.device)
+    ws = _empty(L.gin_hexconv_wgrad_ws_bytes(cin, cout), torch.uint8, xb.device)
+    _lib.check(L.gin_hexconv_wgrad_bf16(plan.host_ptr, plan.dev_ptr, xb.data_ptr(), dyb.data_ptr(), None, dW.data_ptr(), None, ws.data_ptr(),
+                                        B, cin, cout, _stream()), 'gin_hexconv_wgrad_bf16')
     return dW
 
 
 import os as _os
 _Y16 = _os.environ.get('GIN_Y_FP16', '1') != '0'
-_side_streams = {}
 _grad_sink = None
 _grad_dest = None
 
@@ -205,18 +182,6 @@ def _dest(params, shape):
         return None
     t = _grad_dest(params)
     return t.view(shape) if t is not None and t.numel() == int(torch.Size(shape).numel()) else None
-
-
-def _wgrad_stream(dev):
-    import os
-    # measured at I5 / B=36: no gain (4.30 vs 4.26 ms per step) -- the persistent conv kernels leave no room for co-resident CTAs --
-    # so the side stream is opt-in (GIN_WGRAD_STREAM=1)
-    if os.environ.get('GIN_WGRAD_STREAM', '0') != '1':
-        return None
-    key = (dev.type, dev.index)
-    if key not in _side_streams:
-        _side_streams[key] = torch.cuda.Stream(device=dev)
-    return _side_streams[key]
 
 
 def _bn_stats(y, col0, ld, rows, C, bn, parts=None):
@@ -256,15 +221,11 @@ def _bn_act(y1, col1, ld1, stat1, y2, col2, ld2, stat2, B, level, C, want_b=True
     return out_b, out_f, out_w
 
 
-# The BatchNorm backward kernels re-evaluate the ReLU mask from y and the BatchNorm constants instead of reading it from the
-# activation copy (include/geniconet_b200.h: relu_from_y): 2 B / element less in each pass, step 3.40 -> 3.27 ms on the same box
-# (profiles/r02_ab_mask_*.json).  GIN_BN_MASK_FROM_Y=0 reads the mask.
-_MASK_FROM_Y = 0 if _os.environ.get('GIN_BN_MASK_FROM_Y', '1') == '0' else 1
-
-
-def _bn_bwd(dout, mask_b, y, col0, ld, stat, B, level, C, dy_b=None, dy_b_col=0, ldo=0, want_f=False, mask_from_y=None):
+def _bn_bwd(dout, mask_b, y, col0, ld, stat, B, level, C, dy_b=None, dy_b_col=0, ldo=0, want_f=False, mask_from_y=True):
     """Returns (bstat [4C]: dbeta, dgamma, ..., dy_f or None); writes the bf16 gradient copy into dy_b[:, dy_b_col:dy_b_col+C].
-    mask_b must be the activation copy _bn_act produced from (y, stat) with ReLU (it may then be re-evaluated instead of read)."""
+    mask_b must be the activation copy _bn_act produced from (y, stat) with ReLU.  With mask_from_y the kernel re-evaluates the
+    mask from y and the BatchNorm constants instead of reading it (include/geniconet_b200.h: relu_from_y): 2 B / element less in
+    each pass, step 3.40 -> 3.27 ms on the same box (profiles/r02_ab_mask_*.json)."""
     dev = dout.device
     bstat = _empty(4 * C, torch.float32, dev)
     ws = _empty(L.gin_bn_ws_bytes(C), torch.uint8, dev)
@@ -272,7 +233,7 @@ def _bn_bwd(dout, mask_b, y, col0, ld, stat, B, level, C, dy_b=None, dy_b_col=0,
     _lib.check(L.gin_bn_act_bwd(dout.data_ptr(), C, mask_b.data_ptr() if mask_b is not None else None, y.data_ptr() + y.element_size() * col0, ld,
                                 1 if y.dtype == torch.float16 else 0, stat.data_ptr(), bstat.data_ptr(), (dy_b.data_ptr() + 2 * dy_b_col) if dy_b is not None else None, ldo,
                                 dy_f.data_ptr() if want_f else None, C, ws.data_ptr(), B, level, C,
-                                _MASK_FROM_Y if mask_from_y is None else int(mask_from_y), _stream()), 'gin_bn_act_bwd')
+                                int(mask_from_y), _stream()), 'gin_bn_act_bwd')
     return bstat, dy_f
 
 
@@ -318,165 +279,220 @@ def _block_stats(ycat, pcat, blk, rows, cout):
     return stat00, stat10
 
 
+def _nchw(rows, B, level, C):
+    """[B, C, H, W] view, with channels-last strides, of a row-major map [B * P(level)][C]."""
+    n = 2 ** level
+    return rows.view(B, 5 * n, 2 * n, C).permute(0, 3, 1, 2)
+
+
+def _rows(t):
+    """fp32 [B * P][C] rows of a [B, C, H, W] map; no copy when it has channels-last strides."""
+    d = as_channels_last(t).permute(0, 2, 3, 1).reshape(-1, t.shape[1])
+    return d if d.is_contiguous() else d.contiguous()
+
+
+def _cat(blk):
+    """The weights of a block's sibling GEMM conv00 | conv10: their wgrad reads the block's input."""
+    return (blk.conv00.weight, blk.conv10.weight)
+
+
 # ------------------------------------------------------------------------------------------------ the chain
+def _block(blk, plan_a, plan_b, a_b, pk_cat, pk01, B, lvl, consts, want_h_w, want_b, want_f, want_w):
+    """A residual block from the forward operand copy a_b of its input: the sibling GEMM conv00 | conv10, BatchNorm 00 / 10,
+    relu(bn00) as conv01's operand, conv01, BatchNorm 01, relu(bn01 + bn10).  Batch statistics (running statistics updated) when
+    consts is None, else the eval constants consts[bn].  Returns (out_b, out_f, what a backward needs: fp32 / fp16 conv outputs,
+    BatchNorm constants and the bf16 twins h_w of conv01's operand and out_w of the output, None where not wanted)."""
+    cin, cout, rows = blk.conv00.in_features, blk.conv00.out_features, B * _P(lvl)
+    ycat, pcat = _conv_fwd(plan_a, a_b, pk_cat, blk.conv00.bias.detach(), B, cin, 2 * cout, _P(lvl), bias1=blk.conv10.bias.detach())   # [rows][conv00 | conv10]
+    if consts is None:
+        stat00, stat10 = _block_stats(ycat, pcat, blk, rows, cout)
+    else:
+        stat00, stat10 = consts[blk.icobn00][2], consts[blk.icobn10][2]
+    h_b, _, h_w = _bn_act(ycat, 0, 2 * cout, stat00, None, 0, 0, None, B, lvl, cout, want_w=want_h_w)
+    y01, p01 = _conv_fwd(plan_b, h_b, pk01, blk.conv01.bias.detach(), B, cout, cout, _P(lvl))
+    stat01 = _bn_stats(y01, 0, cout, rows, cout, blk.icobn01, p01) if consts is None else consts[blk.icobn01][2]
+    out_b, out_f, out_w = _bn_act(y01, 0, cout, stat01, ycat, cout, 2 * cout, stat10, B, lvl, cout, want_b=want_b, want_f=want_f, want_w=want_w)
+    return out_b, out_f, dict(ycat=ycat, y01=y01, h_w=h_w, out_w=out_w, stat00=stat00, stat01=stat01, stat10=stat10)
+
+
+def _block_affine(blk, plan_a, plan_b, a_b, pk_cat, pk01, B, lvl, consts, want_b, want_f):
+    """The block in eval mode with each BatchNorm in the epilogue of the convolution that feeds it: relu(bn00(conv00)) as conv01's
+    operand, bn10(conv10) as the skip map, then relu(bn01(conv01) + skip).  (out_b, out_f), or None where the epilogue is
+    unsupported."""
+    cin, cout = blk.conv00.in_features, blk.conv00.out_features
+    (sc00, sh00, _), (sc01, sh01, _) = consts[blk.icobn00], consts[blk.icobn01]
+    r = _conv_affine(plan_a, a_b, pk_cat, B, cin, 2 * cout, lvl, _span(sc00, 2 * cout), _span(sh00, 2 * cout), cout, cout, (True, False), (False, True))
+    if r is not None:
+        r = _conv_affine(plan_b, r[0], pk01, B, cout, cout, lvl, sc01, sh01, 0, cout, (want_b, want_f), res=r[3])
+    return (r[0], r[1]) if r is not None else None
+
+
+def _walk(x, mods, consts, twin, copy, record):
+    """The forward of the chain `mods` (see chain_supported) on x, for the training, forward-only and frozen chains.
+
+    consts: None for batch statistics that update the running statistics, else the eval constants of eval_pairs(mods) in that
+    order (with record False the blocks then try the affine epilogue first).  twin(weights): whether to make the bf16 twin of an
+    activation copy whose wgrad readers are `weights` (none for a block output that no Down block reads).  copy(nxt): whether to
+    make the forward operand copy of the activation that the module nxt reads (None: the chain's output).  record: keep, per
+    stage, what a backward needs.  Returns (fp32 output map [B, C, H, W] with channels-last strides, its forward operand copy or
+    None, the stages)."""
+    dev, B = x.device, x.shape[0]
+    if consts is not None:
+        consts = {bn: c for (bn, _), c in zip(eval_pairs(mods), consts)}
+    stages = []
+    if isinstance(mods[0], IcoConvS2S):                                  # ---- stem: xyz conv (fp32, warp-level kernels) + BN + ReLU
+        conv, bn = mods[0], mods[1]
+        level, C = conv.subdivisions, conv.out_features
+        plan, packed, xs, strides, y, parts = _stem_conv(x, conv)
+        stat = _bn_stats(y, 0, C, B * _P(level), C, bn, parts) if consts is None else consts[bn][2]
+        act_b, _, act_w = _bn_act(y, 0, C, stat, None, 0, 0, None, B, level, C, want_b=copy(mods[3]), want_w=twin(_cat(mods[3])))
+        if record:
+            stages.append(dict(kind='stem', plan=plan, xs=xs, strides=strides, y=y, stat=stat, out_w=act_w, C=C, level=level, packed=packed, k=0))
+        act_f, i, k = None, 3, 4
+    else:                                                                # ---- chain starts on an fp32 map
+        blk = mods[0]
+        level, C = blk.conv00.subdivisions - (0 if blk._down else 1), blk.conv00.in_features
+        xl = as_channels_last(x)
+        act_f, act_b, act_w = xl.permute(0, 2, 3, 1).reshape(-1, C), None, None
+        if copy(blk):
+            plan = get_plan(_lib.PLAN_HEXCONV, level, 1, blk.conv00.corner_mode, dev)
+            act_b = cast_bf16(xl, plan, 0, level)
+            if twin(_cat(blk)):
+                act_w = cast_bf16(xl, plan, 2, level) if _DUAL else act_b
+        if record:
+            stages.append(dict(kind='input', level=level, C=C, k=0))
+        i, k = 0, 0
+    # every weight of the chain's tensor-core convolutions is packed by ONE launch
+    jobs = []
+    for blk in mods[i:]:
+        jobs.append((blk.conv00.weight.detach().contiguous(), blk.conv10.weight.detach().contiguous(), blk.conv00.in_features))
+        jobs.append((blk.conv01.weight.detach().contiguous(), None, blk.conv01.in_features))
+    packs = _pack_many(jobs)
+    for j in range(i, len(mods)):
+        blk = mods[j]
+        nxt = mods[j + 1] if j + 1 < len(mods) else None
+        cm = blk.conv00.corner_mode
+        cin, cout = blk.conv00.in_features, blk.conv00.out_features
+        st = dict(kind='down' if blk._down else 'up', cin=cin, cout=cout, in_level=level, blk=blk, k=k)
+        if blk._down:
+            lvl = level - 1
+            plan_a = get_plan(_lib.PLAN_HEXCONV, level, 2, cm, dev)
+            a_b, a_w = act_b, act_w
+        else:
+            lvl = level + 1
+            up_plan = st['up_plan'] = get_plan(_lib.PLAN_UPSAMPLE, level, 1, blk.upsample00.corner_mode, dev)
+            plan_a = get_plan(_lib.PLAN_HEXCONV, lvl, 1, cm, dev)
+            # upsample straight into the operand copy of the fine level, from the fp32 coarse map (one rounding)
+            a_b = _empty((B * _P(lvl) + 2 * B, cin), torch.bfloat16, dev)
+            a_w = None
+            if twin(_cat(blk)):
+                a_w = _empty((B * _P(lvl) + 2 * B, cin), torch.bfloat16, dev) if _DUAL else a_b
+            _lib.check(L.gin_upsample_bf16(up_plan.host_ptr, up_plan.dev_ptr, act_f.data_ptr(), 1, a_b.data_ptr(),
+                                           a_w.data_ptr() if (_DUAL and a_w is not None) else None, B, cin, _stream()), 'gin_upsample_bf16')
+        plan_b = get_plan(_lib.PLAN_HEXCONV, lvl, 1, cm, dev)
+        pk_cat, pk01 = packs[2 * (j - i)], packs[2 * (j - i) + 1]
+        want_b = copy(nxt)
+        want_f = nxt is None or not nxt._down          # an Up block upsamples from the fp32 map (one rounding instead of two)
+        r = _block_affine(blk, plan_a, plan_b, a_b, pk_cat, pk01, B, lvl, consts, want_b, want_f) if consts is not None and not record else None
+        if r is None:
+            out_b, out_f, saved = _block(blk, plan_a, plan_b, a_b, pk_cat, pk01, B, lvl, consts, twin((blk.conv01.weight,)), want_b, want_f,
+                                         twin(_cat(nxt) if nxt is not None and nxt._down else ()))
+            act_w = saved['out_w']
+        else:
+            (out_b, out_f), act_w = r, None
+        if record:
+            # the bf16 twins are kept (wgrad operands, ReLU masks); the forward-format copies die with the forward pass
+            st.update(saved, plan_a=plan_a, plan_b=plan_b, a_w=a_w, pk_cat=pk_cat, pk01=pk01, level=lvl)
+            stages.append(st)
+        act_b, act_f, level, C, k = out_b, out_f, lvl, cout, k + 12
+    return _nchw(act_f, B, level, C), act_b, stages
+
+
+def _block_input_grad(st, dycat_b, B):
+    """fp32 gradient of a block's input from the bf16 gradient copy of its sibling GEMM's output: ONE dgrad of conv00 | conv10
+    (concatenated along K, which adds the two input gradients), then the upsample's backward for an Up block."""
+    cin, cout, lvl = st['cin'], st['cout'], st['level']
+    d = _conv_dgrad(st['plan_a'], dycat_b, st['pk_cat'], B, cin, 2 * cout, _P(lvl + 1) if st['kind'] == 'down' else _P(lvl))
+    if st['kind'] == 'up':
+        upp = st['up_plan']
+        d_prev = _empty((B * _P(st['in_level']), cin), torch.float32, d.device)
+        _lib.check(L.gin_upsample_bwd(upp.host_ptr, upp.dev_ptr, d.data_ptr(), d_prev.data_ptr(), B, cin, _stream()), 'gin_upsample_bwd')
+        d = d_prev
+    return d
+
+
+def _stem_bwd(st, dy_f, B, want_dW, want_db, want_dx):
+    """From the fp32 gradient dy_f of the stem convolution's output: (weight gradient, conv-bias gradient, gradient of the xyz
+    input), each None where not wanted.  The bias gradient comes out of the weight-gradient kernel."""
+    plan, (sb, sp, sc), C, lvl, dev = st['plan'], st['strides'], st['C'], st['level'], dy_f.device
+    dW = db = dx = None
+    if want_dW:
+        dW = _empty((C, 3, 7), torch.float32, dev)
+        db = _empty((C,), torch.float32, dev) if want_db else None
+        ws = _empty(L.gin_hexconv_wgrad_ws_bytes(3, C), torch.uint8, dev)
+        _lib.check(L.gin_hexconv_wgrad(plan.host_ptr, plan.dev_ptr, st['xs'].data_ptr(), sb, sp, sc, dy_f.data_ptr(), dW.data_ptr(),
+                                       db.data_ptr() if db is not None else None, ws.data_ptr(), B, 3, C, _lib.IMPL_AUTO, _stream()), 'gin_hexconv_wgrad')
+    if want_dx:                     # exact fp32 gather-GEMM: 3 output channels
+        dxs = _empty((B * _P(lvl), 3), torch.float32, dev)
+        _lib.check(L.gin_hexconv_dgrad(plan.host_ptr, plan.dev_ptr, dy_f.data_ptr(), st['packed'].data_ptr(), dxs.data_ptr(), B, 3, C,
+                                       _lib.IMPL_SIMT, _stream()), 'gin_hexconv_dgrad')
+        dx = _nchw(dxs, B, lvl, 3)
+    return dW, db, dx
+
+
 class _Chain(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, mods, *params):
-        dev = x.device
-        B = x.shape[0]
-        saved = []                # per stage: dict of what backward needs
-        i = 0
-        act_b, level, C = None, None, None
-        ctx.x_needs_grad = x.requires_grad
-        if isinstance(mods[0], IcoConvS2S):                                  # ---- stem: xyz conv (fp32, warp-level kernels) + BN + ReLU
-            conv, bn = mods[0], mods[1]
-            level, C = conv.subdivisions, conv.out_features
-            plan, packed, xs, (sb, sp, sc), y, parts = _stem_conv(x, conv)
-            stat = _bn_stats(y, 0, C, B * _P(level), C, bn, parts)
-            act_b, _, act_w = _bn_act(y, 0, C, stat, None, 0, 0, None, B, level, C)
-            saved.append(dict(kind='stem', plan=plan, xs=xs, strides=(sb, sp, sc), y=y, stat=stat, out_b=act_w, C=C, level=level, packed=packed))
-            i = 3
-        else:                                                                # ---- chain starts on an fp32 map: make the operand copy
-            blk = mods[0]
-            level, C = blk.conv00.subdivisions - (0 if blk._down else 1), blk.conv00.in_features
-            plan = get_plan(_lib.PLAN_HEXCONV, level, 1, blk.conv00.corner_mode, dev)
-            from .ico_conv import as_channels_last, cast_bf16
-            act_b = cast_bf16(as_channels_last(x), plan, 0, level)
-            act_w = cast_bf16(as_channels_last(x), plan, 2, level) if _DUAL else act_b
-            saved.append(dict(kind='input', level=level, C=C))
-        ctx.in_shape = tuple(x.shape)
-        act_f = None
-        if saved[0]['kind'] == 'input':
-            from .ico_conv import as_channels_last as _acl
-            act_f = _acl(x).permute(0, 2, 3, 1).reshape(-1, C)
-        last = len(mods) - 1
-        out_f = None
-        # every weight of the chain's tensor-core convolutions is packed by ONE launch
-        jobs = []
-        for blk in mods[i:]:
-            jobs.append((blk.conv00.weight.detach().contiguous(), blk.conv10.weight.detach().contiguous(), blk.conv00.in_features))
-            jobs.append((blk.conv01.weight.detach().contiguous(), None, blk.conv01.in_features))
-        packs = _pack_many(jobs)
-        for j in range(i, len(mods)):
-            blk = mods[j]
-            cm = blk.conv00.corner_mode
-            cin, cout = blk.conv00.in_features, blk.conv00.out_features
-            st = dict(kind='down' if blk._down else 'up', cin=cin, cout=cout, in_level=level, blk=blk)
-            if blk._down:
-                lvl = level - 1
-                plan_a = get_plan(_lib.PLAN_HEXCONV, level, 2, cm, dev)
-                a_b, a_w = act_b, act_w
-            else:
-                lvl = level + 1
-                up_plan = get_plan(_lib.PLAN_UPSAMPLE, level, 1, blk.upsample00.corner_mode, dev)
-                plan_a = get_plan(_lib.PLAN_HEXCONV, lvl, 1, cm, dev)
-                # upsample straight into the operand copy of the fine level, from the fp32 coarse map (one rounding)
-                a_b = _empty((B * _P(lvl) + 2 * B, cin), torch.bfloat16, dev)
-                a_w = _empty((B * _P(lvl) + 2 * B, cin), torch.bfloat16, dev) if _DUAL else a_b
-                _lib.check(L.gin_upsample_bf16(up_plan.host_ptr, up_plan.dev_ptr, act_f.data_ptr(), 1, a_b.data_ptr(), a_w.data_ptr() if _DUAL else None,
-                                               B, cin, _stream()), 'gin_upsample_bf16')
-                st['up_plan'] = up_plan
-            plan_b = get_plan(_lib.PLAN_HEXCONV, lvl, 1, cm, dev)
-            rows = B * _P(lvl)
-            pk_cat, pk01 = packs[2 * (j - i)], packs[2 * (j - i) + 1]
-            ycat, pcat = _conv_fwd(plan_a, a_b, pk_cat, blk.conv00.bias.detach(), B, cin, 2 * cout, _P(lvl), bias1=blk.conv10.bias.detach())   # [rows][conv00 | conv10]
-            stat00, stat10 = _block_stats(ycat, pcat, blk, rows, cout)
-            h_b, _, h_w = _bn_act(ycat, 0, 2 * cout, stat00, None, 0, 0, None, B, lvl, cout)
-            y01, p01 = _conv_fwd(plan_b, h_b, pk01, blk.conv01.bias.detach(), B, cout, cout, _P(lvl))
-            stat01 = _bn_stats(y01, 0, cout, rows, cout, blk.icobn01, p01)
-            is_last = j == last
-            keep_f = is_last or not mods[j + 1]._down         # an Up block upsamples from the fp32 map (one rounding instead of two)
-            # the bf16 copy of the block output is the ReLU mask of the backward, so it is always produced
-            # the forward copy of the last block's output has no consumer; its bf16 twin is still the ReLU mask of the backward
-            out_b, out_f, out_w = _bn_act(y01, 0, cout, stat01, ycat, cout, 2 * cout, stat10, B, lvl, cout, want_b=not is_last or not _DUAL, want_f=keep_f)
-            act_f = out_f
-            # saved for backward: the bf16 twins (wgrad operands / ReLU masks); the forward-format copies die with the forward pass
-            st.update(plan_a=plan_a, plan_b=plan_b, a_b=a_w, pk_cat=pk_cat, pk01=pk01, ycat=ycat, y01=y01, h_b=h_w, out_b=out_w,
-                      stat00=stat00, stat01=stat01, stat10=stat10, level=lvl)
-            saved.append(st)
-            act_b, act_w, level, C = out_b, out_w, lvl, cout
-        ctx.saved, ctx.B, ctx.nparams = saved, B, len(params)
-        ctx.mods = mods
-        n = 2 ** level
-        return out_f.view(B, 5 * n, 2 * n, C).permute(0, 3, 1, 2)
+        # every twin (the block outputs' are the ReLU masks of backward); the forward copy of every activation but the output, which
+        # with bf16 forward operands is its own twin
+        out, _, ctx.stages = _walk(x, mods, None, lambda ws: True, lambda nxt: nxt is not None or not _DUAL, True)
+        ctx.mods, ctx.B, ctx.x_needs_grad = mods, x.shape[0], x.requires_grad
+        return out
 
     @staticmethod
     def backward(ctx, d_out):
-        B = ctx.B
-        saved = ctx.saved
-        from .ico_conv import as_channels_last
-        d = as_channels_last(d_out).permute(0, 2, 3, 1).reshape(-1, d_out.shape[1])          # fp32 [rows][C], no copy when channels-last
-        if not d.is_contiguous():
-            d = d.contiguous()
-        grads = []                # filled back to front, reversed at the end
-        dx = None
-        side = _wgrad_stream(d.device)
+        B, d, dx = ctx.B, _rows(d_out), None
         plist = chain_params(ctx.mods)          # the Parameter objects, in the order of the gradients this function returns
-        zmax = max([st['cout'] for st in saved if st['kind'] in ('down', 'up')] + [1])
+        grads = [None] * len(plist)
+        zmax = max([st['cout'] for st in ctx.stages if st['kind'] in ('down', 'up')] + [1])
         zeros = torch.zeros(zmax, dtype=torch.float32, device=d.device)     # the (exactly zero) gradients of conv biases that feed a BatchNorm
-        for st in reversed(saved):
-            n_before = len(grads)
+        for st in reversed(ctx.stages):
+            k = st['k']
             if st['kind'] in ('down', 'up'):
-                cin, cout, lvl = st['cin'], st['cout'], st['level']
+                cin, cout, lvl, blk = st['cin'], st['cout'], st['level'], st['blk']
                 dev = d.device
-                dycat_b = torch.empty((B * _P(lvl) + 2 * B, 2 * cout), dtype=torch.bfloat16, device=dev)
-                dy01_b = torch.empty((B * _P(lvl) + 2 * B, cout), dtype=torch.bfloat16, device=dev)
+                dycat_b = _empty((B * _P(lvl) + 2 * B, 2 * cout), torch.bfloat16, dev)
+                dy01_b = _empty((B * _P(lvl) + 2 * B, cout), torch.bfloat16, dev)
                 # bn01 and bn10 see the same g = d * (out > 0): one pass pair for both
-                bs01 = torch.empty(4 * cout, dtype=torch.float32, device=dev)
-                bs10 = torch.empty(4 * cout, dtype=torch.float32, device=dev)
-                ws = torch.empty(L.gin_bn_pair_ws_bytes(cout), dtype=torch.uint8, device=dev)
-                assert st['y01'].dtype == st['ycat'].dtype
-                _lib.check(L.gin_bn_act_bwd_pair(d.data_ptr(), cout, st['out_b'].data_ptr(), st['y01'].data_ptr(), cout, st['stat01'].data_ptr(),
-                                                 bs01.data_ptr(), dy01_b.data_ptr(), cout, st['ycat'].data_ptr() + st['ycat'].element_size() * cout, 2 * cout,
+                bs01 = _empty(4 * cout, torch.float32, dev)
+                bs10 = _empty(4 * cout, torch.float32, dev)
+                ws = _empty(L.gin_bn_pair_ws_bytes(cout), torch.uint8, dev)
+                ycat = st['ycat']
+                assert st['y01'].dtype == ycat.dtype
+                _lib.check(L.gin_bn_act_bwd_pair(d.data_ptr(), cout, st['out_w'].data_ptr(), st['y01'].data_ptr(), cout, st['stat01'].data_ptr(),
+                                                 bs01.data_ptr(), dy01_b.data_ptr(), cout, ycat.data_ptr() + ycat.element_size() * cout, 2 * cout,
                                                  st['stat10'].data_ptr(), bs10.data_ptr(), dycat_b.data_ptr() + 2 * cout, 2 * cout,
-                                                 1 if st['ycat'].dtype == torch.float16 else 0, ws.data_ptr(), B, lvl, cout, _MASK_FROM_Y, _stream()), 'gin_bn_act_bwd_pair')
-                blk = st['blk']
-                dW01 = _conv_wgrad(st['plan_b'], st['h_b'], dy01_b, B, cout, cout, side,
-                                   out=_dest((blk.conv01.weight,), (cout, cout, 7)) if side is None else None)
+                                                 1 if ycat.dtype == torch.float16 else 0, ws.data_ptr(), B, lvl, cout, 1, _stream()), 'gin_bn_act_bwd_pair')
+                dW01 = _conv_wgrad(st['plan_b'], st['h_w'], dy01_b, B, cout, cout, out=_dest((blk.conv01.weight,), (cout, cout, 7)))
                 d_h = _conv_dgrad(st['plan_b'], dy01_b, st['pk01'], B, cout, cout, _P(lvl))
-                bs00, _ = _bn_bwd(d_h, st['h_b'], st['ycat'], 0, 2 * cout, st['stat00'], B, lvl, cout, dycat_b, 0, 2 * cout)
-                dWcat = _conv_wgrad(st['plan_a'], st['a_b'], dycat_b, B, cin, 2 * cout, side,
-                                    out=_dest((blk.conv00.weight, blk.conv10.weight), (2 * cout, cin, 7)) if side is None else None)
-                p_in = _P(lvl + 1) if st['kind'] == 'down' else _P(lvl)
-                d_in = _conv_dgrad(st['plan_a'], dycat_b, st['pk_cat'], B, cin, 2 * cout, p_in)
-                if st['kind'] == 'up':
-                    upp = st['up_plan']
-                    d_prev = torch.empty((B * _P(st['in_level']), cin), dtype=torch.float32, device=dev)
-                    _lib.check(L.gin_upsample_bwd(upp.host_ptr, upp.dev_ptr, d_in.data_ptr(), d_prev.data_ptr(), B, cin, _stream()), 'gin_upsample_bwd')
-                    d_in = d_prev
+                bs00, _ = _bn_bwd(d_h, st['h_w'], ycat, 0, 2 * cout, st['stat00'], B, lvl, cout, dycat_b, 0, 2 * cout)
+                dWcat = _conv_wgrad(st['plan_a'], st['a_w'], dycat_b, B, cin, 2 * cout, out=_dest(_cat(blk), (2 * cout, cin, 7)))
+                d = _block_input_grad(st, dycat_b, B)
                 zero_b = zeros[:cout]
-                # parameter order of chain_params: conv00 (w, b, gamma, beta), conv01 (...), conv10 (...); appended reversed
-                grads += [bs10[:cout], bs10[cout:2 * cout], zero_b, dWcat[cout:],
-                          bs01[:cout], bs01[cout:2 * cout], zero_b, dW01,
-                          bs00[:cout], bs00[cout:2 * cout], zero_b, dWcat[:cout]]
-                d = d_in
+                # parameter order of chain_params: conv00 (w, b, gamma, beta) at k, conv01 at k + 4, conv10 at k + 8
+                grads[k:k + 12] = [dWcat[:cout], zero_b, bs00[cout:2 * cout], bs00[:cout], dW01, zero_b, bs01[cout:2 * cout], bs01[:cout],
+                                   dWcat[cout:], zero_b, bs10[cout:2 * cout], bs10[:cout]]
+                n = 12
             elif st['kind'] == 'stem':
-                C, lvl = st['C'], st['level']
-                bs, dy_f = _bn_bwd(d, st['out_b'], st['y'], 0, C, st['stat'], B, lvl, C, want_f=True)
-                plan = st['plan']
-                dW = torch.empty((C, 3, 7), dtype=torch.float32, device=d.device)
-                db = torch.empty((C,), dtype=torch.float32, device=d.device)
-                ws = torch.empty(L.gin_hexconv_wgrad_ws_bytes(3, C), dtype=torch.uint8, device=d.device)
-                sb, sp, sc = st['strides']
-                _lib.check(L.gin_hexconv_wgrad(plan.host_ptr, plan.dev_ptr, st['xs'].data_ptr(), sb, sp, sc, dy_f.data_ptr(), dW.data_ptr(), db.data_ptr(),
-                                               ws.data_ptr(), B, 3, C, _lib.IMPL_AUTO, _stream()), 'gin_hexconv_wgrad')
-                grads += [bs[:C], bs[C:2 * C], db, dW]
-                if ctx.x_needs_grad:                     # gradient of the xyz input (exact fp32 gather-GEMM: 3 output channels)
-                    n = 2 ** lvl
-                    dxs = torch.empty((B * _P(lvl), 3), dtype=torch.float32, device=d.device)
-                    _lib.check(L.gin_hexconv_dgrad(plan.host_ptr, plan.dev_ptr, dy_f.data_ptr(), st['packed'].data_ptr(), dxs.data_ptr(), B, 3, C,
-                                                   _lib.IMPL_SIMT, _stream()), 'gin_hexconv_dgrad')
-                    dx = dxs.view(B, 5 * n, 2 * n, 3).permute(0, 3, 1, 2)
+                C = st['C']
+                bs, dy_f = _bn_bwd(d, st['out_w'], st['y'], 0, C, st['stat'], B, st['level'], C, want_f=True)
+                dW, db, dx = _stem_bwd(st, dy_f, B, True, True, ctx.x_needs_grad)
+                grads[0:4] = [dW, db, bs[C:2 * C], bs[:C]]
+                n = 4
             else:   # 'input': gradient of the fp32 map the chain started from
-                n = 2 ** st['level']
-                dx = d.view(B, 5 * n, 2 * n, st['C']).permute(0, 3, 1, 2)
-            if _grad_sink is not None and side is None and len(grads) > n_before:
-                # grads[k] (appended back to front) belongs to plist[nparams - 1 - k]
-                _grad_sink([(plist[ctx.nparams - 1 - k], grads[k]) for k in range(n_before, len(grads))])
-        if side is not None:
-            torch.cuda.current_stream().wait_stream(side)      # the weight gradients are consumed (optimizer, all-reduce) on the main stream
-        grads.reverse()
-        assert len(grads) == ctx.nparams
+                dx, n = _nchw(d, B, st['level'], st['C']), 0
+            if _grad_sink is not None and n:
+                _grad_sink([(plist[q], grads[q]) for q in reversed(range(k, k + n))])     # last parameter first
         return (dx, None) + tuple(grads)
 
 
@@ -577,75 +593,9 @@ def infer_chain(x, mods, want_operand=False):
 
     Returns (fp32 output map [B, C, H, W] with channels-last strides, its 16-bit forward operand copy when want_operand else None)."""
     mods = list(mods)
-    train = mods[-1].icobn01.training
-    dev, B = x.device, x.shape[0]
-    consts = None if train else iter(_eval_consts(eval_pairs(mods)))
-    i = 0
-    if isinstance(mods[0], IcoConvS2S):
-        conv, bn = mods[0], mods[1]
-        level, C = conv.subdivisions, conv.out_features
-        _, _, _, _, y, parts = _stem_conv(x, conv)
-        stat = _bn_stats(y, 0, C, B * _P(level), C, bn, parts) if train else next(consts)[2]
-        act_b, _, _ = _bn_act(y, 0, C, stat, None, 0, 0, None, B, level, C, want_w=False)
-        act_f = None
-        i = 3
-    else:
-        blk = mods[0]
-        level, C = blk.conv00.subdivisions - (0 if blk._down else 1), blk.conv00.in_features
-        plan = get_plan(_lib.PLAN_HEXCONV, level, 1, blk.conv00.corner_mode, dev)
-        from .ico_conv import as_channels_last, cast_bf16
-        act_b = cast_bf16(as_channels_last(x), plan, 0, level)
-        act_f = as_channels_last(x).permute(0, 2, 3, 1).reshape(-1, C)
-    jobs = []
-    for blk in mods[i:]:
-        jobs.append((blk.conv00.weight.detach().contiguous(), blk.conv10.weight.detach().contiguous(), blk.conv00.in_features))
-        jobs.append((blk.conv01.weight.detach().contiguous(), None, blk.conv01.in_features))
-    packs = _pack_many(jobs)
-    last = len(mods) - 1
-    for j in range(i, len(mods)):
-        blk = mods[j]
-        cm = blk.conv00.corner_mode
-        cin, cout = blk.conv00.in_features, blk.conv00.out_features
-        if blk._down:
-            lvl = level - 1
-            plan_a = get_plan(_lib.PLAN_HEXCONV, level, 2, cm, dev)
-            a_b = act_b
-        else:
-            lvl = level + 1
-            up_plan = get_plan(_lib.PLAN_UPSAMPLE, level, 1, blk.upsample00.corner_mode, dev)
-            plan_a = get_plan(_lib.PLAN_HEXCONV, lvl, 1, cm, dev)
-            a_b = _empty((B * _P(lvl) + 2 * B, cin), torch.bfloat16, dev)
-            _lib.check(L.gin_upsample_bf16(up_plan.host_ptr, up_plan.dev_ptr, act_f.data_ptr(), 1, a_b.data_ptr(), None, B, cin, _stream()),
-                       'gin_upsample_bf16')
-        plan_b = get_plan(_lib.PLAN_HEXCONV, lvl, 1, cm, dev)
-        rows = B * _P(lvl)
-        pk_cat, pk01 = packs[2 * (j - i)], packs[2 * (j - i) + 1]
-        is_last = j == last
-        keep_f = is_last or not mods[j + 1]._down
-        want_b = not is_last or want_operand
-        if train:
-            ycat, pcat = _conv_fwd(plan_a, a_b, pk_cat, blk.conv00.bias.detach(), B, cin, 2 * cout, _P(lvl), bias1=blk.conv10.bias.detach())
-            stat00, stat10 = _block_stats(ycat, pcat, blk, rows, cout)
-            h_b, _, _ = _bn_act(ycat, 0, 2 * cout, stat00, None, 0, 0, None, B, lvl, cout, want_w=False)
-            y01, p01 = _conv_fwd(plan_b, h_b, pk01, blk.conv01.bias.detach(), B, cout, cout, _P(lvl))
-            stat01 = _bn_stats(y01, 0, cout, rows, cout, blk.icobn01, p01)
-            act_b, act_f, _ = _bn_act(y01, 0, cout, stat01, ycat, cout, 2 * cout, stat10, B, lvl, cout, want_b=want_b, want_f=keep_f, want_w=False)
-        else:
-            (sc00, sh00, st00), (_, _, st10), (sc01, sh01, st01) = next(consts), next(consts), next(consts)
-            r = _conv_affine(plan_a, a_b, pk_cat, B, cin, 2 * cout, lvl, _span(sc00, 2 * cout), _span(sh00, 2 * cout), cout, cout,
-                             (True, False), (False, True))
-            if r is not None:                                # relu(bn00(conv00)) as conv01's operand, bn10(conv10) as the skip map
-                r = _conv_affine(plan_b, r[0], pk01, B, cout, cout, lvl, sc01, sh01, 0, cout, (want_b, keep_f), res=r[3])
-            if r is not None:
-                act_b, act_f = r[0], r[1]
-            else:                                            # the composition with the same constants
-                ycat, _ = _conv_fwd(plan_a, a_b, pk_cat, blk.conv00.bias.detach(), B, cin, 2 * cout, _P(lvl), bias1=blk.conv10.bias.detach())
-                h_b, _, _ = _bn_act(ycat, 0, 2 * cout, st00, None, 0, 0, None, B, lvl, cout, want_w=False)
-                y01, _ = _conv_fwd(plan_b, h_b, pk01, blk.conv01.bias.detach(), B, cout, cout, _P(lvl))
-                act_b, act_f, _ = _bn_act(y01, 0, cout, st01, ycat, cout, 2 * cout, st10, B, lvl, cout, want_b=want_b, want_f=keep_f, want_w=False)
-        level, C = lvl, cout
-    n = 2 ** level
-    return act_f.view(B, 5 * n, 2 * n, C).permute(0, 3, 1, 2), (act_b if want_operand else None)
+    consts = None if mods[-1].icobn01.training else _eval_consts(eval_pairs(mods))
+    out, act_b, _ = _walk(x, mods, consts, lambda ws: False, lambda nxt: nxt is not None or want_operand, False)
+    return out, act_b
 
 
 # ------------------------------------------------------------------------------------------------ frozen BatchNorm (eval mode with grad)
@@ -689,106 +639,35 @@ class _FrozenChain(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, x, mods, *params):
-        dev, B = x.device, x.shape[0]
-        need = [p.requires_grad for p in params]
-        consts = iter(_own_consts(eval_pairs(mods)))
-        saved, i, k = [], 0, 0                 # k: index of the stage's first parameter in `params`
-        if isinstance(mods[0], IcoConvS2S):
-            conv = mods[0]
-            level, C = conv.subdivisions, conv.out_features
-            plan, packed, xs, strides, y, _ = _stem_conv(x, conv)
-            stat = next(consts)[2]
-            # the stem's output is the first block's input: its bf16 twin is that block's wgrad operand
-            blk = mods[3]
-            want_w = blk.conv00.weight.requires_grad or blk.conv10.weight.requires_grad
-            act_b, _, act_w = _bn_act(y, 0, C, stat, None, 0, 0, None, B, level, C, want_w=want_w)
-            saved.append(dict(kind='stem', plan=plan, xs=xs, strides=strides, y=y, stat=stat, C=C, level=level, packed=packed, k=0))
-            act_f, i, k = None, 3, 4
-        else:
-            blk = mods[0]
-            level, C = blk.conv00.subdivisions - (0 if blk._down else 1), blk.conv00.in_features
-            from .ico_conv import as_channels_last, cast_bf16
-            xl = as_channels_last(x)
-            act_f = xl.permute(0, 2, 3, 1).reshape(-1, C)
-            if blk._down:
-                plan = get_plan(_lib.PLAN_HEXCONV, level, 1, blk.conv00.corner_mode, dev)
-                act_b = cast_bf16(xl, plan, 0, level)
-                act_w = (cast_bf16(xl, plan, 2, level) if _DUAL else act_b) if (blk.conv00.weight.requires_grad or blk.conv10.weight.requires_grad) else None
-            saved.append(dict(kind='input', level=level, C=C))
-        jobs = []
-        for blk in mods[i:]:
-            jobs.append((blk.conv00.weight.detach().contiguous(), blk.conv10.weight.detach().contiguous(), blk.conv00.in_features))
-            jobs.append((blk.conv01.weight.detach().contiguous(), None, blk.conv01.in_features))
-        packs = _pack_many(jobs)
-        last = len(mods) - 1
-        for j in range(i, len(mods)):
-            blk = mods[j]
-            cm = blk.conv00.corner_mode
-            cin, cout = blk.conv00.in_features, blk.conv00.out_features
-            w_cat = blk.conv00.weight.requires_grad or blk.conv10.weight.requires_grad
-            st = dict(kind='down' if blk._down else 'up', cin=cin, cout=cout, in_level=level, k=k)
-            if blk._down:
-                lvl = level - 1
-                plan_a = get_plan(_lib.PLAN_HEXCONV, level, 2, cm, dev)
-                a_b, a_w = act_b, act_w
-            else:
-                lvl = level + 1
-                up_plan = get_plan(_lib.PLAN_UPSAMPLE, level, 1, blk.upsample00.corner_mode, dev)
-                plan_a = get_plan(_lib.PLAN_HEXCONV, lvl, 1, cm, dev)
-                a_b = _empty((B * _P(lvl) + 2 * B, cin), torch.bfloat16, dev)
-                a_w = (_empty((B * _P(lvl) + 2 * B, cin), torch.bfloat16, dev) if _DUAL else a_b) if w_cat else None
-                _lib.check(L.gin_upsample_bf16(up_plan.host_ptr, up_plan.dev_ptr, act_f.data_ptr(), 1, a_b.data_ptr(),
-                                               a_w.data_ptr() if (_DUAL and a_w is not None) else None, B, cin, _stream()), 'gin_upsample_bf16')
-                st['up_plan'] = up_plan
-            plan_b = get_plan(_lib.PLAN_HEXCONV, lvl, 1, cm, dev)
-            pk_cat, pk01 = packs[2 * (j - i)], packs[2 * (j - i) + 1]
-            (_, _, stat00), (_, _, stat10), (_, _, stat01) = next(consts), next(consts), next(consts)
-            ycat, _ = _conv_fwd(plan_a, a_b, pk_cat, blk.conv00.bias.detach(), B, cin, 2 * cout, _P(lvl), bias1=blk.conv10.bias.detach())
-            h_b, _, h_w = _bn_act(ycat, 0, 2 * cout, stat00, None, 0, 0, None, B, lvl, cout, want_w=blk.conv01.weight.requires_grad)
-            y01, _ = _conv_fwd(plan_b, h_b, pk01, blk.conv01.bias.detach(), B, cout, cout, _P(lvl))
-            is_last = j == last
-            keep_f = is_last or not mods[j + 1]._down
-            nxt_w = not is_last and mods[j + 1]._down and (mods[j + 1].conv00.weight.requires_grad or mods[j + 1].conv10.weight.requires_grad)
-            # an Up block upsamples from the fp32 map: the operand copy is made only for a Down block
-            out_b, out_f, out_w = _bn_act(y01, 0, cout, stat01, ycat, cout, 2 * cout, stat10, B, lvl, cout, want_b=not keep_f, want_f=keep_f,
-                                          want_w=nxt_w)
-            st.update(plan_a=plan_a, plan_b=plan_b, a_w=a_w if w_cat else None, h_w=h_w if blk.conv01.weight.requires_grad else None,
-                      pk_cat=pk_cat, pk01=pk01, ycat=ycat, y01=y01, stat00=stat00, stat01=stat01, stat10=stat10, level=lvl)
-            saved.append(st)
-            act_b, act_w, act_f, level, C = out_b, out_w, out_f, lvl, cout
-            k += 12
-        ctx.saved, ctx.B, ctx.need, ctx.x_needs_grad = saved, B, need, x.requires_grad
-        n = 2 ** level
-        return act_f.view(B, 5 * n, 2 * n, C).permute(0, 3, 1, 2)
+        # twins only for weights that need a gradient, forward copies only where a Down block reads them
+        out, _, ctx.stages = _walk(x, mods, _own_consts(eval_pairs(mods)), lambda ws: any(w.requires_grad for w in ws),
+                                   lambda nxt: nxt is not None and nxt._down, True)
+        ctx.B, ctx.need, ctx.x_needs_grad = x.shape[0], [p.requires_grad for p in params], x.requires_grad
+        return out
 
     @staticmethod
     def backward(ctx, d_out):
-        B, saved, need = ctx.B, ctx.saved, ctx.need
-        from .ico_conv import as_channels_last
-        d = as_channels_last(d_out).permute(0, 2, 3, 1).reshape(-1, d_out.shape[1])
-        if not d.is_contiguous():
-            d = d.contiguous()
+        B, stages, need, d, dx = ctx.B, ctx.stages, ctx.need, _rows(d_out), None
         grads = [None] * len(need)
-        dx = None
         # upstream[s]: something before stage s (an earlier stage's parameter, or x) needs a gradient
         upstream, acc = [], ctx.x_needs_grad
-        for st in saved:
+        for st in stages:
             upstream.append(acc)
             if st['kind'] != 'input':
                 acc = acc or any(need[st['k']:st['k'] + (4 if st['kind'] == 'stem' else 12)])
         dev = d.device
         sums = lambda k, C: _empty(3 * C, torch.float32, dev) if any(need[k + 1:k + 4]) else None
-        for s in range(len(saved) - 1, -1, -1):
-            st = saved[s]
+        ptr = lambda t: t.data_ptr() if t is not None else None
+        for s in range(len(stages) - 1, -1, -1):
+            st = stages[s]
             if st['kind'] in ('down', 'up'):
                 cin, cout, lvl, k = st['cin'], st['cout'], st['level'], st['k']
                 # parameter order of chain_params: conv00 (w, b, gamma, beta) at k, conv01 at k + 4, conv10 at k + 8
                 bs00, bs01, bs10 = sums(k, cout), sums(k + 4, cout), sums(k + 8, cout)
-                dycat_b = torch.empty((B * _P(lvl) + 2 * B, 2 * cout), dtype=torch.bfloat16, device=dev)
-                dy01_b = torch.empty((B * _P(lvl) + 2 * B, cout), dtype=torch.bfloat16, device=dev)
+                dycat_b = _empty((B * _P(lvl) + 2 * B, 2 * cout), torch.bfloat16, dev)
+                dy01_b = _empty((B * _P(lvl) + 2 * B, cout), torch.bfloat16, dev)
                 ws = _empty(L.gin_bn_eval_bwd_ws_bytes(cout), torch.uint8, dev) if (bs01 is not None or bs10 is not None) else None
                 ycat = st['ycat']
-                ptr = lambda t: t.data_ptr() if t is not None else None
                 _lib.check(L.gin_bn_eval_bwd_pair(d.data_ptr(), cout, None, st['y01'].data_ptr(), cout, st['stat01'].data_ptr(), ptr(bs01),
                                                   dy01_b.data_ptr(), cout, ycat.data_ptr() + ycat.element_size() * cout, 2 * cout,
                                                   st['stat10'].data_ptr(), ptr(bs10), dycat_b.data_ptr() + 2 * cout, 2 * cout,
@@ -805,38 +684,18 @@ class _FrozenChain(torch.autograd.Function):
                         _take_sums(grads, need, kk, bs, cout)
                 if not upstream[s]:
                     break
-                p_in = _P(lvl + 1) if st['kind'] == 'down' else _P(lvl)
-                d = _conv_dgrad(st['plan_a'], dycat_b, st['pk_cat'], B, cin, 2 * cout, p_in)
-                if st['kind'] == 'up':
-                    upp = st['up_plan']
-                    d_prev = torch.empty((B * _P(st['in_level']), cin), dtype=torch.float32, device=dev)
-                    _lib.check(L.gin_upsample_bwd(upp.host_ptr, upp.dev_ptr, d.data_ptr(), d_prev.data_ptr(), B, cin, _stream()), 'gin_upsample_bwd')
-                    d = d_prev
+                d = _block_input_grad(st, dycat_b, B)
             elif st['kind'] == 'stem':
-                C, lvl = st['C'], st['level']
+                C = st['C']
                 bs = sums(0, C)
                 if not (need[0] or bs is not None or ctx.x_needs_grad):
                     break
-                dy_f = _eval_bwd(d, st['y'], 0, C, st['stat'], B, lvl, C, bs, want_f=True)
-                plan = st['plan']
-                sb, sp, sc = st['strides']
-                if need[0]:
-                    dW = torch.empty((C, 3, 7), dtype=torch.float32, device=dev)
-                    ws = torch.empty(L.gin_hexconv_wgrad_ws_bytes(3, C), dtype=torch.uint8, device=dev)
-                    _lib.check(L.gin_hexconv_wgrad(plan.host_ptr, plan.dev_ptr, st['xs'].data_ptr(), sb, sp, sc, dy_f.data_ptr(), dW.data_ptr(), None,
-                                                   ws.data_ptr(), B, 3, C, _lib.IMPL_AUTO, _stream()), 'gin_hexconv_wgrad')
-                    grads[0] = dW
+                dy_f = _eval_bwd(d, st['y'], 0, C, st['stat'], B, st['level'], C, bs, want_f=True)
+                grads[0], _, dx = _stem_bwd(st, dy_f, B, need[0], False, ctx.x_needs_grad)
                 if bs is not None:
                     _take_sums(grads, need, 0, bs, C)
-                if ctx.x_needs_grad:
-                    n = 2 ** lvl
-                    dxs = torch.empty((B * _P(lvl), 3), dtype=torch.float32, device=dev)
-                    _lib.check(L.gin_hexconv_dgrad(plan.host_ptr, plan.dev_ptr, dy_f.data_ptr(), st['packed'].data_ptr(), dxs.data_ptr(), B, 3, C,
-                                                   _lib.IMPL_SIMT, _stream()), 'gin_hexconv_dgrad')
-                    dx = dxs.view(B, 5 * n, 2 * n, 3).permute(0, 3, 1, 2)
             else:
-                n = 2 ** st['level']
-                dx = d.view(B, 5 * n, 2 * n, st['C']).permute(0, 3, 1, 2)
+                dx = _nchw(d, B, st['level'], st['C'])
         return (dx, None) + tuple(grads)
 
 
@@ -874,8 +733,7 @@ def infer_latent(h_b, mu, logvar, B):
     r = _conv_affine(plan, h_b, packed, B, cin, 2 * cout, lvl, _span(sa, 2 * cout), _span(ha, 2 * cout), 0, cout, (False, True), (False, True))
     if r is None:
         return None
-    n = 2 ** lvl
-    return tuple(t.view(B, 5 * n, 2 * n, cout).permute(0, 3, 1, 2) for t in (r[1], r[3]))
+    return _nchw(r[1], B, lvl, cout), _nchw(r[3], B, lvl, cout)
 
 
 # ------------------------------------------------------------------ decoder head: Conv2d(64, 3, 1) -> Tanh (models.py:151-154)
@@ -896,7 +754,6 @@ def head_supported(head, x):
 class _Head(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, weight, bias):
-        from .ico_conv import as_channels_last
         B, C, H, W = x.shape
         xs = as_channels_last(x)                              # [B*P][64] in memory; no copy after a fused chain
         w = weight.reshape(3, C).contiguous()

@@ -49,66 +49,60 @@ def _bn_modes(tops):
     return {m.training for t in tops for m in t.modules() if isinstance(m, torch.nn.BatchNorm2d)}
 
 
-def _infer(mods, x, want_operand=False):
-    """fused.infer_chain over `mods` (a Sequential, whose own hooks count too, or a list of modules) when grad is disabled, every
-    BatchNorm inside is in the same mode and no module inside has a forward hook; else None (the caller runs the modules)."""
+def _route(mods, x, train_chain=True):
+    """Which fused chain runs `mods` (a Sequential, whose own hooks count too, or a list of modules) on x: 'infer' (fused.infer_chain),
+    'train' (fused.run_chain), 'frozen' (fused.run_frozen_chain), or None (the caller runs the modules).  A chain needs a CUDA fp32 x,
+    no forward (pre-)hook and no `impl` override inside, a supported module list, and every BatchNorm inside in the same mode.  With
+    grad disabled that is the forward-only chain (when switched on); with grad enabled the BatchNorms decide: train mode -> the
+    training chain (unless train_chain is False: the split models never take it), eval mode -> the frozen chain (when switched on)."""
     tops = [mods] if isinstance(mods, torch.nn.Module) else list(mods)
     mods = list(mods)
-    if not (_FUSED and _INFER and not torch.is_grad_enabled() and x.is_cuda and x.dtype == torch.float32):
+    if not (_FUSED and x.is_cuda and x.dtype == torch.float32):
         return None
     inner = [m for t in tops for m in t.modules()]
-    if any(m._forward_hooks or m._forward_pre_hooks for m in inner):
+    if any(m._forward_hooks or m._forward_pre_hooks or (isinstance(m, IcoConvS2S) and getattr(m, 'impl', 0) != 0) for m in inner):
         return None
-    if len({m.training for m in inner if isinstance(m, torch.nn.BatchNorm2d)}) != 1:
-        return None
-    if any(getattr(c, 'impl', 0) != 0 for c in inner if isinstance(c, IcoConvS2S)) or not _fused.chain_supported(mods):
-        return None
-    return _fused.infer_chain(x, mods, want_operand)
+    modes = _bn_modes(tops)
+    if not torch.is_grad_enabled():
+        return 'infer' if _INFER and len(modes) == 1 and _fused.chain_supported(mods) else None
+    if modes == {True}:
+        return 'train' if train_chain and _fused.chain_supported(mods) else None
+    return 'frozen' if _FROZEN and modes == {False} and _fused.frozen_supported(mods) else None
 
 
-def _frozen(mods, x):
-    """fused.run_frozen_chain over `mods` (a Sequential, whose own hooks count too, or a list of modules) when the switch is on, grad
-    is enabled, every BatchNorm inside is in eval mode and no module inside has a forward hook; else None (the caller runs the
-    modules)."""
-    tops = [mods] if isinstance(mods, torch.nn.Module) else list(mods)
+def _apply(route, mods, x):
+    """`mods` on x through the fused chain `route` (see _route), or for None through the modules themselves: a Sequential is
+    called, a list runs in order."""
+    if route is None:
+        if isinstance(mods, torch.nn.Module):
+            return mods(x)
+        for m in mods:
+            x = m(x)
+        return x
     mods = list(mods)
-    if not (_FUSED and _FROZEN and torch.is_grad_enabled() and x.is_cuda and x.dtype == torch.float32):
-        return None
-    inner = [m for t in tops for m in t.modules()]
-    if any(m._forward_hooks or m._forward_pre_hooks for m in inner) or _bn_modes(tops) != {False}:
-        return None
-    if any(getattr(c, 'impl', 0) != 0 for c in inner if isinstance(c, IcoConvS2S)) or not _fused.frozen_supported(mods):
-        return None
-    return _fused.run_frozen_chain(x, mods)
+    if route == 'infer':
+        return _fused.infer_chain(x, mods)[0]
+    return (_fused.run_chain if route == 'train' else _fused.run_frozen_chain)(x, mods)
 
 
 def _run(mods, x):
-    """nn.Sequential semantics over the module list, through a fused chain when possible.  With grad enabled the BatchNorms inside
-    decide: all in train mode -> the training chain, all in eval mode -> the frozen chain (when switched on), mixed -> the modules."""
+    """nn.Sequential semantics over the module list, through a fused chain when one applies (_route)."""
     mods = list(mods)
-    r = _infer(mods, x)
-    if r is not None:
-        return r[0]
-    if (_FUSED and x.is_cuda and x.dtype == torch.float32 and torch.is_grad_enabled() and _bn_modes(mods) == {True}
-            and all(getattr(c, 'impl', 0) == 0 for m in mods for c in m.modules() if isinstance(c, IcoConvS2S))
-            and _fused.chain_supported(mods)):
-        return _fused.run_chain(x, mods)
-    r = _frozen(mods, x)
-    if r is not None:
-        return r
-    for m in mods:
-        x = m(x)
-    return x
+    return _apply(_route(mods, x), mods, x)
 
 
 def _body(seq, x):
     """A split model's body `seq` (a Sequential) on x: through the forward-only or the frozen chain where one applies, else module by
     module (the split models never take the training chain)."""
-    r = _infer(seq, x)
-    if r is not None:
-        return r[0]
-    r = _frozen(seq, x)
-    return r if r is not None else seq(x)
+    return _apply(_route(seq, x, train_chain=False), seq, x)
+
+
+def _infer_encode(encoder, mu, logvar, x):
+    """A VAE encoder body on the forward-only chain: (its output map, (mu, logvar) or None).  The mu and logvar heads run as ONE GEMM
+    on the body's operand copy (fused.infer_latent) where that is supported; None: the caller runs them."""
+    h, h_b = _fused.infer_chain(x, list(encoder), want_operand=True)
+    return h, (_fused.infer_latent(h_b, mu, logvar, x.shape[0]) if _fused.latent_supported(mu, logvar) else None)
+
 
 BatchNorm2d = torch.nn.BatchNorm2d
 
@@ -299,13 +293,6 @@ def _latent_head(params, level):
                                BatchNorm2d(512))
 
 
-def _latent(r, mu, logvar, x):
-    """(mu, logvar) from the encoder output r = (map, operand copy) of _infer as one GEMM (fused.infer_latent), or None."""
-    if not _fused.latent_supported(mu, logvar):
-        return None
-    return _fused.infer_latent(r[1], mu, logvar, x.shape[0])
-
-
 class ico2ico_vae(VAE):
     def __init__(self, params):
         super().__init__()
@@ -327,14 +314,14 @@ class ico2ico_vae(VAE):
         return _latent_head(self.params, _top(self.params) - 2)
 
     def encode(self, input):
-        r = _infer(list(self.encoder), input, want_operand=True)
-        if r is None:
-            h = _run(self.encoder, input)
-        else:
-            lat = _latent(r, self.mu, self.logvar, input)
+        mods = list(self.encoder)
+        route = _route(mods, input)
+        if route == 'infer':
+            h, lat = _infer_encode(mods, self.mu, self.logvar, input)
             if lat is not None:
                 return self.mu_hook(lat[0]), self.logvar_hook(lat[1])
-            h = r[0]
+        else:
+            h = _apply(route, mods, input)
         return self.mu_hook(self.mu(h)), self.logvar_hook(self.logvar(h))
 
     def decode(self, z):
@@ -351,16 +338,13 @@ class ico2enc_vae(VAE):
         self.logvar = _latent_head(params, _top(params) - 2)
 
     def encode(self, input):
-        r = _infer(self.encoder, input, want_operand=True)
-        if r is None:
-            h = _frozen(self.encoder, input)
-            if h is None:
-                h = self.encoder(input)
-        else:
-            lat = _latent(r, self.mu, self.logvar, input)
+        route = _route(self.encoder, input, train_chain=False)
+        if route == 'infer':
+            h, lat = _infer_encode(self.encoder, self.mu, self.logvar, input)
             if lat is not None:
                 return lat
-            h = r[0]
+        else:
+            h = _apply(route, self.encoder, input)
         return self.mu(h), self.logvar(h)
 
     def forward(self, x):

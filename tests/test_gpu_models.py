@@ -287,6 +287,30 @@ def test_bench_configurations_run_and_agree(name, level, B):
     assert abs(vals[True] - vals[False]) <= 5e-3 * abs(vals[False]), vals
 
 
+def test_hook_inside_a_training_chain_runs_the_modules():
+    """A forward or forward-pre hook on a module inside a chain sends the chain to the modules in train mode with grad too: both
+    hooks fire and the output is bit for bit that of set_fused(False)."""
+    import copy
+    from geniconet_b200 import models as gm, data
+    level, B = 5, 3
+    a = om.fill_params_deterministic(gm.ico2ico(gm.default_params('ico2ico', level))).cuda().train()
+    b = copy.deepcopy(a)
+    x, _ = data.synthetic_batch(level, 0, B)
+    x = x.cuda()
+    fired = []
+    a.encoder[3].conv01.register_forward_hook(lambda m, i, o: fired.append('conv01'))
+    a.decoder[0].icobn01.register_forward_pre_hook(lambda m, i: fired.append('icobn01'))
+    try:
+        gm.set_fused(True, head=False)                       # the module head on both sides
+        y_a = a(x)
+        gm.set_fused(False)
+        y_b = b(x)
+    finally:
+        gm.set_fused(True, True)
+    assert fired == ['conv01', 'icobn01']
+    assert torch.equal(y_a, y_b)
+
+
 def test_fused_chain_returns_the_xyz_input_gradient():
     """d loss / d input through the fused chain (the xyz stem's dgrad) against the module-wise fp32 path."""
     from geniconet_b200 import models as gm, losses, data
