@@ -110,7 +110,8 @@ int run_gather_gemm_simt(const int32_t* plan_dev, const GinSide& side, int group
 
 // tcgen05 path on the bf16 activation copy: patch mode for stride 1, gather mode otherwise
 int run_gemm_tc(const int32_t* plan_dev, const GinConvPlanHdr* h, const void* Xb, const char* packed, int B, bool dgrad,
-                const float* bias, float* Y, cudaStream_t st, int Cin, int Cout, float* stats = nullptr, int* stats_parts = nullptr) {
+                const float* bias, float* Y, cudaStream_t st, int Cin, int Cout, float* stats = nullptr, int* stats_parts = nullptr,
+                const gin::Bias2& bias2 = {}) {
   if (stats_parts) *stats_parts = 0;
   const GinSide& side = dgrad ? h->dg : h->fwd;
   const int K = dgrad ? Cout : Cin, N = dgrad ? Cin : Cout;
@@ -120,51 +121,42 @@ int run_gemm_tc(const int32_t* plan_dev, const GinConvPlanHdr* h, const void* Xb
   const GinPSide& ps = dgrad ? h->pdg : h->pfwd;
   int rc;
   // forward: activation copy x forward weight tiles (both the forward format); dgrad: dy copy x dgrad weight tiles (both bf16)
-  gin::set_operand_formats(dgrad || !gin::fwd_fp16(), dgrad || !gin::fwd_fp16());
+  const bool bf16 = dgrad || !gin::fwd_fp16();
+  bool fold;                                          // dgrad: the boundary pixels are part of the in-chart launch
   if (h->stride == 1 && patch_mode_enabled() && gin::tcp_supported(ps, K, N)) {
-    const bool fold = dgrad && tc_mode() == 2 && gin::cv2_supported(ps, K, N) && seam_fold_ok(h->pf);
+    fold = dgrad && tc_mode() == 2 && gin::cv2_supported(ps, K, N) && seam_fold_ok(h->pf);
     if (tc_mode() == 2 && gin::cv2_supported(ps, K, N))
-      rc = gin::launch_patch_conv2(plan_dev, ps, h->group, side.P_dst, 2 << h->level_in, Xb, wb, bias, Y, B, K, N, dgrad ? 1 : 0, st, dgrad ? nullptr : stats,
-                                   dgrad ? nullptr : stats_parts, fold ? &h->pf : nullptr);
-    else rc = gin::launch_patch_gemm_tc(plan_dev, ps, h->group, side.P_dst, Xb, wb, bias, Y, B, K, N, dgrad ? 1 : 0, st);
+      rc = gin::launch_patch_conv2(plan_dev, ps, h->group, side.P_dst, 2 << h->level_in, Xb, wb, bias, bias2, Y, B, K, N, dgrad ? 1 : 0, bf16, st,
+                                   dgrad ? nullptr : stats, dgrad ? nullptr : stats_parts, fold ? &h->pf : nullptr);
+    else rc = gin::launch_patch_gemm_tc(plan_dev, ps, h->group, side.P_dst, Xb, wb, bias, Y, B, K, N, dgrad ? 1 : 0, bf16, st);
     if (rc != GIN_OK) return fail(rc, "tcgen05 patch-GEMM launch failed: %s", cudaGetErrorString(cudaGetLastError()));
-    g_launches.fetch_add(1, std::memory_order_relaxed);
-    if (fold) return GIN_OK;                          // boundary pixels were part of the same launch
-    if (dgrad && tc_mode() == 2 && seam_v2_enabled() && gin::cv2_seam_supported(h->px, K, N)) {   // cross-seam and pole entries, added on top
-      rc = gin::launch_patch_conv2_seam(plan_dev, h->px, h->group, side.P_src, side.P_dst, Xb, wb, Y, B, K, N, st);
-      if (rc != GIN_OK) return fail(rc, "tcgen05 seam pass (v2) launch failed: %s", cudaGetErrorString(cudaGetLastError()));
-      g_launches.fetch_add(1, std::memory_order_relaxed);
-    } else if (dgrad && h->dgx.ntiles > 0) {
-      rc = gin::launch_gather_gemm_tc(plan_dev, h->dgx, h->group, Xb, wb, nullptr, Y, B, K, N, groups * h->dgx.ntiles, st, 1);
-      if (rc != GIN_OK) return fail(rc, "tcgen05 seam pass launch failed: %s", cudaGetErrorString(cudaGetLastError()));
-      g_launches.fetch_add(1, std::memory_order_relaxed);
-    }
-    return GIN_OK;
-  }
-  if (h->stride == 2 && tc_mode() == 2 && gin::cv2_supported(h->p2, K, N)) {
+  } else if (h->stride == 2 && tc_mode() == 2 && gin::cv2_supported(h->p2, K, N)) {
     // stride 2 in patch mode on the coarse lattice: four parity planes (gin_plan.h: GinP2Side)
     const int Pf = h->fwd.P_src, Pc = h->fwd.P_dst;
-    rc = GIN_OK;
-    if (!dgrad) rc = gin::launch_patch_conv2_s2_fwd(plan_dev, h->p2, h->group, Pf, Pc, 2 << h->level_out, Xb, wb, bias, Y, B, K, N, st, stats, stats_parts);
-    const bool fold = dgrad && seam_fold_ok(h->pf);
-    if (dgrad) rc = gin::launch_patch_conv2_s2_dgrad(plan_dev, h->p2, h->group, Pf, Pc, 2 << h->level_in, Xb, wb, Y, B, K, N, st, fold ? &h->pf : nullptr);
+    fold = dgrad && seam_fold_ok(h->pf);
+    if (!dgrad)
+      rc = gin::launch_patch_conv2_s2_fwd(plan_dev, h->p2, h->group, Pf, Pc, 2 << h->level_out, Xb, wb, bias, bias2, Y, B, K, N, bf16, st, stats,
+                                          stats_parts);
+    else rc = gin::launch_patch_conv2_s2_dgrad(plan_dev, h->p2, h->group, Pf, Pc, 2 << h->level_in, Xb, wb, Y, B, K, N, bf16, st, fold ? &h->pf : nullptr);
     if (rc != GIN_OK) return fail(rc, "tcgen05 stride-2 patch launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+  } else {                                            // gather mode: the one launch covers the seams too
+    rc = gin::launch_gather_gemm_tc(plan_dev, side, h->group, Xb, wb, bias, Y, B, K, N, groups * side.ntiles, bf16, st);
+    if (rc != GIN_OK) return fail(rc, "tcgen05 gather-GEMM launch failed: %s", cudaGetErrorString(cudaGetLastError()));
     g_launches.fetch_add(1, std::memory_order_relaxed);
-    if (fold) return GIN_OK;
-    if (dgrad && seam_v2_enabled() && gin::cv2_seam_supported(h->px, K, N)) {
-      rc = gin::launch_patch_conv2_seam(plan_dev, h->px, h->group, Pc, Pf, Xb, wb, Y, B, K, N, st);
-      if (rc != GIN_OK) return fail(rc, "tcgen05 seam pass (v2) launch failed: %s", cudaGetErrorString(cudaGetLastError()));
-      g_launches.fetch_add(1, std::memory_order_relaxed);
-    } else if (dgrad && h->dgx.ntiles > 0) {
-      rc = gin::launch_gather_gemm_tc(plan_dev, h->dgx, h->group, Xb, wb, nullptr, Y, B, K, N, groups * h->dgx.ntiles, st, 1);
-      if (rc != GIN_OK) return fail(rc, "tcgen05 seam pass launch failed: %s", cudaGetErrorString(cudaGetLastError()));
-      g_launches.fetch_add(1, std::memory_order_relaxed);
-    }
     return GIN_OK;
   }
-  rc = gin::launch_gather_gemm_tc(plan_dev, side, h->group, Xb, wb, bias, Y, B, K, N, groups * side.ntiles, st);
-  if (rc != GIN_OK) return fail(rc, "tcgen05 gather-GEMM launch failed: %s", cudaGetErrorString(cudaGetLastError()));
   g_launches.fetch_add(1, std::memory_order_relaxed);
+  if (!dgrad || fold) return GIN_OK;
+  // the cross-seam and pole entries of dgrad, added on top of the in-chart pass (side = h->dg: coarse dy -> fine dx at stride 2)
+  if (tc_mode() == 2 && seam_v2_enabled() && gin::cv2_seam_supported(h->px, K, N)) {
+    rc = gin::launch_patch_conv2_seam(plan_dev, h->px, h->group, side.P_src, side.P_dst, Xb, wb, Y, B, K, N, bf16, st);
+    if (rc != GIN_OK) return fail(rc, "tcgen05 seam pass (v2) launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+    g_launches.fetch_add(1, std::memory_order_relaxed);
+  } else if (h->dgx.ntiles > 0) {
+    rc = gin::launch_gather_gemm_tc(plan_dev, h->dgx, h->group, Xb, wb, nullptr, Y, B, K, N, groups * h->dgx.ntiles, bf16, st, 1);
+    if (rc != GIN_OK) return fail(rc, "tcgen05 seam pass launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+    g_launches.fetch_add(1, std::memory_order_relaxed);
+  }
   return GIN_OK;
 }
 
@@ -315,13 +307,13 @@ static int wgrad_common(const GinConvPlanHdr* h, const void* plan_dev, const flo
                         int impl = GIN_IMPL_SIMT) {
   float* dWp = reinterpret_cast<float*>(ws);
   int rc;
-  gin::set_operand_formats(true, true);                    // wgrad: A = the bf16 twin of the forward activation copy, B = the bf16 dy copy
+  const bool bf16 = true;                                  // A = the bf16 twin of the forward activation copy, B = the bf16 dy copy
   const bool wg2_s1 = h->stride == 1 && gin::wg2_supported(h->pfwd, Cin, Cout), wg2_s2 = h->stride == 2 && gin::wg2_supported(h->p2, Cin, Cout);
   if (xb && B > 0 && tc_mode() == 2 && (wg2_s1 || wg2_s2)) {
     // second-generation patch wgrad: split-K partials in the workspace, reduced (and laid out as dW[Cout][Cin][7]) by a second kernel
     float* partial = dWp + (size_t)7 * Cin * Cout;
-    if (wg2_s1) rc = gin::launch_wgrad_patch2(plan_words(plan_dev), h->pfwd, h->group, h->fwd.P_dst, xb, dyb, partial, dW, B, Cin, Cout, st);
-    else rc = gin::launch_wgrad_patch2_s2(plan_words(plan_dev), h->p2, h->group, h->fwd.P_src, h->fwd.P_dst, xb, dyb, partial, dW, B, Cin, Cout, st);
+    if (wg2_s1) rc = gin::launch_wgrad_patch2(plan_words(plan_dev), h->pfwd, h->group, h->fwd.P_dst, xb, dyb, partial, dW, B, Cin, Cout, bf16, st);
+    else rc = gin::launch_wgrad_patch2_s2(plan_words(plan_dev), h->p2, h->group, h->fwd.P_src, h->fwd.P_dst, xb, dyb, partial, dW, B, Cin, Cout, bf16, st);
     if (rc != GIN_OK) return fail(rc, "tcgen05 patch wgrad (v2) launch failed: %s", cudaGetErrorString(cudaGetLastError()));
     g_launches.fetch_add(2, std::memory_order_relaxed);
     if (db) {
@@ -343,10 +335,10 @@ static int wgrad_common(const GinConvPlanHdr* h, const void* plan_dev, const flo
     if (xb) {
       if (!gin::tc_wgrad_supported(Cin, Cout)) return fail(GIN_ERR_UNSUPPORTED, "tcgen05 wgrad needs Cin %% 64 == 0 and Cout %% 64 == 0");
       if (h->stride == 1 && patch_mode_enabled() && gin::tcwp_supported(h->pfwd, Cin, Cout)) {
-        rc = gin::launch_wgrad_patch_tc(plan_words(plan_dev), h->pfwd, h->group, side.P_dst, xb, dyb, dWp, B, Cin, Cout, st);
+        rc = gin::launch_wgrad_patch_tc(plan_words(plan_dev), h->pfwd, h->group, side.P_dst, xb, dyb, dWp, B, Cin, Cout, bf16, st);
         if (rc != GIN_OK) return fail(rc, "tcgen05 patch wgrad launch failed: %s", cudaGetErrorString(cudaGetLastError()));
       } else {
-        rc = gin::launch_wgrad_tc(plan_words(plan_dev), side, h->group, xb, dyb, dWp, B, Cin, Cout, total_tiles, st);
+        rc = gin::launch_wgrad_tc(plan_words(plan_dev), side, h->group, xb, dyb, dWp, B, Cin, Cout, total_tiles, bf16, st);
         if (rc != GIN_OK) return fail(rc, "tcgen05 wgrad launch failed: %s", cudaGetErrorString(cudaGetLastError()));
       }
       g_launches.fetch_add(1, std::memory_order_relaxed);
@@ -460,16 +452,14 @@ int gin_hexconv_fwd_bf16_stats2(const void* plan_host, const void* plan_dev, con
                                 const float* bias1, int split, void* y, int y_fp16, int B, int Cin, int Cout, float* stats_ws, int* nparts,
                                 void* stream) {
   if (!bias0 || (bias1 && (split <= 0 || split >= Cout || (split & 63)))) return fail(GIN_ERR_ARG, "gin_hexconv_fwd_bf16_stats2: bad bias split");
-  {
-    const GinConvPlanHdr* h;
-    int rc0 = conv_hdr(plan_host, plan_dev, &h);
-    if (rc0) return rc0;
-    if (!fwd_v2_ok(h, Cin, Cout)) return fail(GIN_ERR_UNSUPPORTED, "gin_hexconv_fwd_bf16_stats2: this plan / size does not run the second-generation patch kernel");
-  }
-  gin::bias2_ref().p = bias1; gin::bias2_ref().split = bias1 ? split : 0; gin::bias2_ref().y_f16 = y_fp16 ? 1 : 0;
-  const int rc = gin_hexconv_fwd_bf16_stats(plan_host, plan_dev, xb, packed, bias0, reinterpret_cast<float*>(y), B, Cin, Cout, stats_ws, nparts, stream);
-  gin::bias2_ref() = gin::Bias2{};
-  return rc;
+  const GinConvPlanHdr* h;
+  int rc = conv_hdr(plan_host, plan_dev, &h);
+  if (rc) return rc;
+  if (!fwd_v2_ok(h, Cin, Cout)) return fail(GIN_ERR_UNSUPPORTED, "gin_hexconv_fwd_bf16_stats2: this plan / size does not run the second-generation patch kernel");
+  if (!xb || !packed || !y || !stats_ws || !nparts || B <= 0 || Cin <= 0 || Cout <= 0) return fail(GIN_ERR_ARG, "gin_hexconv_fwd_bf16_stats2: bad argument");
+  const gin::Bias2 bias2{bias1, bias1 ? split : 0, y_fp16 ? 1 : 0};
+  return run_gemm_tc(plan_words(plan_dev), h, xb, reinterpret_cast<const char*>(packed), B, false, bias0, reinterpret_cast<float*>(y), (cudaStream_t)stream,
+                     Cin, Cout, stats_ws, nparts, bias2);
 }
 
 size_t gin_hexconv_affine_ring_bytes(int B, int Cout) { return (B <= 0 || Cout <= 0) ? 0 : (size_t)B * 10 * Cout * 4; }
@@ -497,14 +487,13 @@ int gin_hexconv_fwd_affine(const void* plan_host, const void* plan_dev, const vo
   a.op[0] = out0_b; a.f32[0] = out0_f; a.ld[0] = split; a.ring[0] = ring_ws;
   a.op[1] = out1_b; a.f32[1] = out1_f; a.ld[1] = Cout - split; a.ring[1] = ring_ws + (size_t)B * 10 * split;
   a.op_f16 = f16;
-  gin::set_operand_formats(!f16, !f16);
   const void* wb = reinterpret_cast<const char*>(packed) + packed_off_bf(Cin, Cout);
   if (h->stride == 1)
-    rc = gin::launch_patch_conv2(plan_words(plan_dev), h->pfwd, h->group, h->fwd.P_dst, 2 << h->level_in, xb, wb, nullptr, nullptr, B, Cin, Cout, 0, st,
-                                 nullptr, nullptr, nullptr, &a);
+    rc = gin::launch_patch_conv2(plan_words(plan_dev), h->pfwd, h->group, h->fwd.P_dst, 2 << h->level_in, xb, wb, nullptr, {}, nullptr, B, Cin, Cout, 0,
+                                 !f16, st, nullptr, nullptr, nullptr, &a);
   else
-    rc = gin::launch_patch_conv2_s2_fwd(plan_words(plan_dev), h->p2, h->group, h->fwd.P_src, h->fwd.P_dst, 2 << h->level_out, xb, wb, nullptr, nullptr, B,
-                                        Cin, Cout, st, nullptr, nullptr, &a);
+    rc = gin::launch_patch_conv2_s2_fwd(plan_words(plan_dev), h->p2, h->group, h->fwd.P_src, h->fwd.P_dst, 2 << h->level_out, xb, wb, nullptr, {},
+                                        nullptr, B, Cin, Cout, !f16, st, nullptr, nullptr, &a);
   if (rc != GIN_OK) return fail(rc, "gin_hexconv_fwd_affine: launch failed: %s", cudaGetErrorString(cudaGetLastError()));
   g_launches.fetch_add(1, std::memory_order_relaxed);
   for (int d = 0; d < 2; ++d) {

@@ -59,10 +59,8 @@ inline bool fwd_fp16() {
   if (v < 0) { const char* e = getenv("GIN_FWD_FP16"); v = (e && e[0] == '0') ? 0 : 1; }
   return v == 1;
 }
-inline uint32_t& fmt_bits_ref() { static thread_local uint32_t bits = (1u << 7) | (1u << 10); return bits; }
-// set by the C-ABI entry points right before a tcgen05 launch: are the A / B operands of this launch bf16 (else fp16)?
-inline void set_operand_formats(bool a_bf16, bool b_bf16) { fmt_bits_ref() = ((uint32_t)a_bf16 << 7) | ((uint32_t)b_bf16 << 10); }
-inline uint32_t operand_format_bits() { return fmt_bits_ref(); }
+// operand-format bits of a tcgen05 launch's instruction descriptor: both operands bf16, or both fp16 (the two must agree)
+inline uint32_t idesc_fmt_bits(bool bf16) { return bf16 ? (1u << 7) | (1u << 10) : 0u; }
 
 inline bool pdl_enabled() {
   static int v = -1;

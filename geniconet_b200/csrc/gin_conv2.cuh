@@ -76,7 +76,7 @@ struct Affine {
 // output, each its own output tile (flush_each) gathered from the same coarse dy image.  (gin_plan.h: GinPSide / GinP2Side.)
 struct Params {
   const int32_t* plan;
-  uint32_t fmt;               // operand-format bits of the instruction descriptor (gin_common.cuh: operand_format_bits)
+  uint32_t fmt;               // operand-format bits of the instruction descriptor (gin_common.cuh: idesc_fmt_bits)
   int U, Q, ntiles;           // patch rows per image, octets per patch row, tiles per sample group
   int group, B, K, N;
   int P_src, P_dst;           // pixels per sample of the gathered / written map
@@ -781,10 +781,9 @@ inline int cv2_dispatch(cv2::Params& p, int max_ntile, cudaStream_t st) {
   }
 }
 
-// stride 1: forward (mirror 0) / in-chart dgrad (mirror 1: tap (di,dj) reads cell (-di,-dj)); W = 2n pixels per chart row
-// second bias of a concatenated forward (set by the C-ABI entry point around the launch; null otherwise)
+// forward epilogue options: a second bias when two sibling convolutions run as one GEMM (columns >= split take p[col - split];
+// none when p is null), and y_f16: write Y as fp16 instead of fp32
 struct Bias2 { const float* p = nullptr; int split = 0; int y_f16 = 0; };
-inline Bias2& bias2_ref() { static thread_local Bias2 b; return b; }
 
 // `pf` (dgrad only): fold the boundary tiles of the plan into the same launch
 inline void cv2_attach_boundary(cv2::Params& p, const GinPfSide* pf) {
@@ -795,16 +794,17 @@ inline void cv2_attach_boundary(cv2::Params& p, const GinPfSide* pf) {
   p.x_all = pf->all;
 }
 
+// stride 1: forward (mirror 0) / in-chart dgrad (mirror 1: tap (di,dj) reads cell (-di,-dj)); W = 2n pixels per chart row
 inline int launch_patch_conv2(const int32_t* plan_dev, const GinPSide& ps, int group, int P, int W, const void* Xb, const void* Wb,
-                              const float* bias, float* Y, int B, int K, int N, int mirror, cudaStream_t st, float* stats = nullptr,
-                              int* stats_parts = nullptr, const GinPfSide* pf = nullptr, const cv2::Affine* aff = nullptr) {
+                              const float* bias, const Bias2& bias2, float* Y, int B, int K, int N, int mirror, bool bf16, cudaStream_t st,
+                              float* stats = nullptr, int* stats_parts = nullptr, const GinPfSide* pf = nullptr, const cv2::Affine* aff = nullptr) {
   cv2::Params p{};
   cv2_attach_boundary(p, pf);
   if (aff) p.aff = *aff;
   p.stats = stats; p.stats_parts = stats_parts;
-  p.plan = plan_dev; p.fmt = operand_format_bits(); p.U = ps.U; p.Q = ps.Q; p.ntiles = ps.ntiles; p.group = group; p.B = B; p.K = K; p.N = N; p.P_src = P; p.P_dst = P;
+  p.plan = plan_dev; p.fmt = idesc_fmt_bits(bf16); p.U = ps.U; p.Q = ps.Q; p.ntiles = ps.ntiles; p.group = group; p.B = B; p.K = K; p.N = N; p.P_src = P; p.P_dst = P;
   p.X = reinterpret_cast<const __nv_bfloat16*>(Xb); p.Wt = reinterpret_cast<const __nv_bfloat16*>(Wb); p.bias = bias; p.Y = Y;
-  if (bias) { p.bias1 = bias2_ref().p; p.bias_split = bias2_ref().split; p.y_f16 = bias2_ref().y_f16; }
+  p.bias1 = bias2.p; p.bias_split = bias2.split; p.y_f16 = bias2.y_f16;
   p.nplanes = 1; p.flush_each = 0; p.ntaps[0] = 7; p.group_bytes = 1280; p.dst_tab_off = -1;
   for (int t = 0; t < 7; ++t) {
     const int di = mirror ? -cv2::kDi[t] : cv2::kDi[t], dj = mirror ? -cv2::kDj[t] : cv2::kDj[t];
@@ -824,15 +824,15 @@ constexpr int kS2B[7] = {0, 0, 0, -1, 0, 0, -1};
 
 // stride 2 forward: X is the FINE map (P_f pixels per sample), Y the coarse one; Wc = 2n of the coarse level
 inline int launch_patch_conv2_s2_fwd(const int32_t* plan_dev, const GinP2Side& ps, int group, int P_f, int P_c, int Wc, const void* Xb,
-                                     const void* Wb, const float* bias, float* Y, int B, int K, int N, cudaStream_t st, float* stats = nullptr,
-                                     int* stats_parts = nullptr, const cv2::Affine* aff = nullptr) {
+                                     const void* Wb, const float* bias, const Bias2& bias2, float* Y, int B, int K, int N, bool bf16,
+                                     cudaStream_t st, float* stats = nullptr, int* stats_parts = nullptr, const cv2::Affine* aff = nullptr) {
   cv2::Params p{};
   p.mask_off = -1;
   if (aff) p.aff = *aff;
   p.stats = stats; p.stats_parts = stats_parts;
-  p.plan = plan_dev; p.fmt = operand_format_bits(); p.U = ps.U; p.Q = ps.Q; p.ntiles = ps.ntiles; p.group = group; p.B = B; p.K = K; p.N = N; p.P_src = P_f; p.P_dst = P_c;
+  p.plan = plan_dev; p.fmt = idesc_fmt_bits(bf16); p.U = ps.U; p.Q = ps.Q; p.ntiles = ps.ntiles; p.group = group; p.B = B; p.K = K; p.N = N; p.P_src = P_f; p.P_dst = P_c;
   p.X = reinterpret_cast<const __nv_bfloat16*>(Xb); p.Wt = reinterpret_cast<const __nv_bfloat16*>(Wb); p.bias = bias; p.Y = Y;
-  if (bias) { p.bias1 = bias2_ref().p; p.bias_split = bias2_ref().split; p.y_f16 = bias2_ref().y_f16; }
+  p.bias1 = bias2.p; p.bias_split = bias2.split; p.y_f16 = bias2.y_f16;
   p.nplanes = 4; p.flush_each = 0; p.group_bytes = 1280; p.dst_tab_off = -1;
   for (int t = 0; t < 7; ++t) {
     const int pl = kS2Plane[t], j = p.ntaps[pl]++;
@@ -847,10 +847,10 @@ inline int launch_patch_conv2_s2_fwd(const int32_t* plan_dev, const GinP2Side& p
 
 // stride 2 dgrad, in-chart part: X is the coarse dy (K = Cout channels), Y the fine dx; Wf = 2n of the fine level
 inline int launch_patch_conv2_s2_dgrad(const int32_t* plan_dev, const GinP2Side& ps, int group, int P_f, int P_c, int Wf, const void* dYb,
-                                       const void* Wb, float* dX, int B, int K, int N, cudaStream_t st, const GinPfSide* pf = nullptr) {
+                                       const void* Wb, float* dX, int B, int K, int N, bool bf16, cudaStream_t st, const GinPfSide* pf = nullptr) {
   cv2::Params p{};
   cv2_attach_boundary(p, pf);
-  p.plan = plan_dev; p.fmt = operand_format_bits(); p.U = ps.U; p.Q = ps.Q; p.ntiles = ps.ntiles; p.group = group; p.B = B; p.K = K; p.N = N; p.P_src = P_c; p.P_dst = P_f;
+  p.plan = plan_dev; p.fmt = idesc_fmt_bits(bf16); p.U = ps.U; p.Q = ps.Q; p.ntiles = ps.ntiles; p.group = group; p.B = B; p.K = K; p.N = N; p.P_src = P_c; p.P_dst = P_f;
   p.X = reinterpret_cast<const __nv_bfloat16*>(dYb); p.Wt = reinterpret_cast<const __nv_bfloat16*>(Wb); p.bias = nullptr; p.Y = dX;
   p.nplanes = 4; p.flush_each = 1; p.group_bytes = 1280; p.dst_tab_off = -1;
   for (int t = 0; t < 7; ++t) {
@@ -871,10 +871,10 @@ inline bool cv2_seam_supported(const GinPxSide& px, int K, int N) {
   return px.ntiles > 0 && px.nslots <= cv2::MAX_PLANES && cv2_supported(GIN_TILE_M, px.ntiles, 1, K, N);
 }
 inline int launch_patch_conv2_seam(const int32_t* plan_dev, const GinPxSide& px, int group, int P_src, int P_dst, const void* dYb, const void* Wb,
-                                   float* dX, int B, int K, int N, cudaStream_t st) {
+                                   float* dX, int B, int K, int N, bool bf16, cudaStream_t st) {
   cv2::Params p{};
   p.mask_off = -1;
-  p.plan = plan_dev; p.fmt = operand_format_bits(); p.U = GIN_TILE_M; p.Q = 1; p.ntiles = px.ntiles; p.group = group; p.B = B; p.K = K; p.N = N; p.P_src = P_src; p.P_dst = P_dst;
+  p.plan = plan_dev; p.fmt = idesc_fmt_bits(bf16); p.U = GIN_TILE_M; p.Q = 1; p.ntiles = px.ntiles; p.group = group; p.B = B; p.K = K; p.N = N; p.P_src = P_src; p.P_dst = P_dst;
   p.X = reinterpret_cast<const __nv_bfloat16*>(dYb); p.Wt = reinterpret_cast<const __nv_bfloat16*>(Wb); p.bias = nullptr; p.Y = dX;
   p.nplanes = px.nslots; p.flush_each = 0; p.group_bytes = 1024; p.accumulate = 1; p.dst_tab_off = px.dst_off;
   for (int s = 0; s < px.nslots; ++s) { p.ntaps[s] = 1; p.tap_id[s][0] = px.tap[s]; p.tap_row[s][0] = 0; }

@@ -119,7 +119,7 @@ GIN_DEVINL uint64_t make_desc_kmajor_sw128(uint32_t smem_addr) {
   return d;
 }
 // kind::f16 instruction descriptor WITHOUT the operand-format bits (those come from Params::fmt, see gin_common.cuh
-// operand_format_bits): D = f32, M = 128, operands K-major unless flagged
+// idesc_fmt_bits): D = f32, M = 128, operands K-major unless flagged
 __host__ __device__ constexpr uint32_t make_idesc_f16kind(int n, int a_mn_major = 0, int b_mn_major = 0) {
   return (1u << 4) | ((uint32_t)a_mn_major << 15) | ((uint32_t)b_mn_major << 16) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(BM >> 4) << 24);
 }
@@ -169,7 +169,7 @@ GIN_DEVINL int resolve_row(int code, long long base, long long total_pix, int sa
 
 struct Params {
   const int32_t* plan;
-  uint32_t fmt;               // operand-format bits of the instruction descriptor (gin_common.cuh: operand_format_bits)
+  uint32_t fmt;               // operand-format bits of the instruction descriptor (gin_common.cuh: idesc_fmt_bits)
   GinSide side;
   int group, B, K, N;
   const __nv_bfloat16* X;    // [B*P_src + 2B][K] bf16 (pixels, then pole-mean rows)
@@ -354,9 +354,9 @@ int launch(const Params& p, int ntiles, cudaStream_t st) {
 inline bool tc_supported(int K, int N) { return K % 64 == 0 && N % 64 == 0 && K >= 64 && N >= 64; }
 
 inline int launch_gather_gemm_tc(const int32_t* plan_dev, const GinSide& side, int group, const void* Xb, const void* Wb,
-                                 const float* bias, float* Y, int B, int K, int N, int ntiles, cudaStream_t st, int accumulate = 0) {
+                                 const float* bias, float* Y, int B, int K, int N, int ntiles, bool bf16, cudaStream_t st, int accumulate = 0) {
   tc::Params p;
-  p.plan = plan_dev; p.fmt = operand_format_bits(); p.side = side; p.group = group; p.B = B; p.K = K; p.N = N;
+  p.plan = plan_dev; p.fmt = idesc_fmt_bits(bf16); p.side = side; p.group = group; p.B = B; p.K = K; p.N = N;
   p.X = reinterpret_cast<const __nv_bfloat16*>(Xb); p.W = reinterpret_cast<const __nv_bfloat16*>(Wb); p.bias = bias; p.Y = Y;
   p.accumulate = accumulate;
   if ((long long)B * side.P_src + 2LL * B >= 0x7fffffffLL) return -4;
@@ -379,7 +379,7 @@ using namespace tc;
 
 struct Params {
   const int32_t* plan;
-  uint32_t fmt;               // operand-format bits of the instruction descriptor (gin_common.cuh: operand_format_bits)
+  uint32_t fmt;               // operand-format bits of the instruction descriptor (gin_common.cuh: idesc_fmt_bits)
   GinSide side;
   int group, B, Cin, Cout;
   const __nv_bfloat16* X;     // [B*P_src + 2B][Cin]
@@ -602,9 +602,9 @@ int launch(Params p, cudaStream_t st) {
 inline bool tc_wgrad_supported(int Cin, int Cout) { return Cin % 64 == 0 && Cout % 64 == 0 && Cin >= 64 && Cout >= 64; }
 
 inline int launch_wgrad_tc(const int32_t* plan_dev, const GinSide& side, int group, const void* Xb, const void* dYb, float* dWp,
-                           int B, int Cin, int Cout, int total_tiles, cudaStream_t st) {
+                           int B, int Cin, int Cout, int total_tiles, bool bf16, cudaStream_t st) {
   tcw::Params p;
-  p.plan = plan_dev; p.fmt = operand_format_bits(); p.side = side; p.group = group; p.B = B; p.Cin = Cin; p.Cout = Cout;
+  p.plan = plan_dev; p.fmt = idesc_fmt_bits(bf16); p.side = side; p.group = group; p.B = B; p.Cin = Cin; p.Cout = Cout;
   p.X = reinterpret_cast<const __nv_bfloat16*>(Xb); p.dY = reinterpret_cast<const __nv_bfloat16*>(dYb); p.dWp = dWp;
   p.total_tiles = total_tiles; p.tiles_per_cta = 1; p.units_m = 1;
   if ((long long)B * side.P_src + 2LL * B >= 0x7fffffffLL) return -4;

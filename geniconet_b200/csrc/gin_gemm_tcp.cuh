@@ -28,7 +28,7 @@ constexpr int MAX_ITEMS = 8;                     // source rows per producer thr
 
 struct Params {
   const int32_t* plan;
-  uint32_t fmt;               // operand-format bits of the instruction descriptor (gin_common.cuh: operand_format_bits)
+  uint32_t fmt;               // operand-format bits of the instruction descriptor (gin_common.cuh: idesc_fmt_bits)
   GinPSide ps;
   int group, B, K, N, P;      // P = pixels per sample (stride 1: same on both sides)
   const __nv_bfloat16* X;     // [B*P + 2B][K] bf16 (pixels, then pole-mean rows)
@@ -242,9 +242,9 @@ inline bool tcp_supported(const GinPSide& ps, int K, int N) {
 }
 
 inline int launch_patch_gemm_tc(const int32_t* plan_dev, const GinPSide& ps, int group, int P, const void* Xb, const void* Wb,
-                                const float* bias, float* Y, int B, int K, int N, int mirror, cudaStream_t st) {
+                                const float* bias, float* Y, int B, int K, int N, int mirror, bool bf16, cudaStream_t st) {
   tcp::Params p;
-  p.plan = plan_dev; p.fmt = operand_format_bits(); p.ps = ps; p.group = group; p.B = B; p.K = K; p.N = N; p.P = P;
+  p.plan = plan_dev; p.fmt = idesc_fmt_bits(bf16); p.ps = ps; p.group = group; p.B = B; p.K = K; p.N = N; p.P = P;
   p.X = reinterpret_cast<const __nv_bfloat16*>(Xb); p.W = reinterpret_cast<const __nv_bfloat16*>(Wb); p.bias = bias; p.Y = Y; p.mirror = mirror;
   if ((long long)B * P + 2LL * B >= 0x7fffffffLL) return -4;
   const int groups = (B + group - 1) / group;

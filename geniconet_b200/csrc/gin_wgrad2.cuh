@@ -36,7 +36,7 @@ constexpr int MAX_CTAS = kMaxSMs;
 // parity plane of the fine input and ONE tap pair per plane (taps {1,2} {5,6} {0,0} {3,4}); either way four accumulators.
 struct Params {
   const int32_t* plan;
-  uint32_t fmt;               // operand-format bits of the instruction descriptor (gin_common.cuh: operand_format_bits)
+  uint32_t fmt;               // operand-format bits of the instruction descriptor (gin_common.cuh: idesc_fmt_bits)
   int U, Q, ntiles;
   int group, B, Cin, Cout;
   int P_src, P_dst;            // pixels per sample of the x map / of the dy map
@@ -339,10 +339,10 @@ inline int wg2_dispatch(wg2::Params& p, float* dW, cudaStream_t st) {
 // paired so that the second tap of a pair never starts before the first: (1,5) (3,0) (4,6) (2,2).
 // Writes dW[Cout][Cin][7] directly; `partial` needs wg2::partial_bytes(Cin, Cout) bytes.
 inline int launch_wgrad_patch2(const int32_t* plan_dev, const GinPSide& ps, int group, int P, const void* Xb, const void* dYb, float* partial,
-                               float* dW, int B, int Cin, int Cout, cudaStream_t st) {
+                               float* dW, int B, int Cin, int Cout, bool bf16, cudaStream_t st) {
   static const int pairs[4][2] = {{1, 5}, {3, 0}, {4, 6}, {2, 2}};
   wg2::Params p{};
-  p.plan = plan_dev; p.fmt = operand_format_bits(); p.U = ps.U; p.Q = ps.Q; p.ntiles = ps.ntiles; p.group = group; p.B = B; p.Cin = Cin; p.Cout = Cout; p.P_src = P; p.P_dst = P;
+  p.plan = plan_dev; p.fmt = idesc_fmt_bits(bf16); p.U = ps.U; p.Q = ps.Q; p.ntiles = ps.ntiles; p.group = group; p.B = B; p.Cin = Cin; p.Cout = Cout; p.P_src = P; p.P_dst = P;
   p.X = reinterpret_cast<const __nv_bfloat16*>(Xb); p.dY = reinterpret_cast<const __nv_bfloat16*>(dYb); p.partial = partial;
   p.nplanes = 1; p.npairs[0] = 4;
   for (int j = 0; j < 4; ++j) {
@@ -358,10 +358,10 @@ inline int launch_wgrad_patch2(const int32_t* plan_dev, const GinPSide& ps, int 
 
 // stride 2: one tap pair per parity plane of the fine input: plane 0 (1,2), plane 1 (5,6), plane 2 (0,0), plane 3 (3,4)
 inline int launch_wgrad_patch2_s2(const int32_t* plan_dev, const GinP2Side& ps, int group, int P_f, int P_c, const void* Xb, const void* dYb,
-                                  float* partial, float* dW, int B, int Cin, int Cout, cudaStream_t st) {
+                                  float* partial, float* dW, int B, int Cin, int Cout, bool bf16, cudaStream_t st) {
   static const int pairs[4][2] = {{1, 2}, {5, 6}, {0, 0}, {3, 4}};
   wg2::Params p{};
-  p.plan = plan_dev; p.fmt = operand_format_bits(); p.U = ps.U; p.Q = ps.Q; p.ntiles = ps.ntiles; p.group = group; p.B = B; p.Cin = Cin; p.Cout = Cout; p.P_src = P_f; p.P_dst = P_c;
+  p.plan = plan_dev; p.fmt = idesc_fmt_bits(bf16); p.U = ps.U; p.Q = ps.Q; p.ntiles = ps.ntiles; p.group = group; p.B = B; p.Cin = Cin; p.Cout = Cout; p.P_src = P_f; p.P_dst = P_c;
   p.X = reinterpret_cast<const __nv_bfloat16*>(Xb); p.dY = reinterpret_cast<const __nv_bfloat16*>(dYb); p.partial = partial;
   p.nplanes = 4;
   for (int pl = 0; pl < 4; ++pl) {

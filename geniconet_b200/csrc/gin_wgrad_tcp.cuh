@@ -23,7 +23,7 @@ constexpr int MAX_ITEMS = tcp::MAX_ITEMS;
 
 struct Params {
   const int32_t* plan;
-  uint32_t fmt;               // operand-format bits of the instruction descriptor (gin_common.cuh: operand_format_bits)
+  uint32_t fmt;               // operand-format bits of the instruction descriptor (gin_common.cuh: idesc_fmt_bits)
   GinPSide ps;
   int group, B, Cin, Cout, P;
   const __nv_bfloat16* X;      // [B*P + 2B][Cin] bf16
@@ -212,9 +212,9 @@ int launch(Params p, cudaStream_t st) {
 inline bool tcwp_supported(const GinPSide& ps, int Cin, int Cout) { return tcp_supported(ps, Cin, Cout); }
 
 inline int launch_wgrad_patch_tc(const int32_t* plan_dev, const GinPSide& ps, int group, int P, const void* Xb, const void* dYb,
-                                 float* dWp, int B, int Cin, int Cout, cudaStream_t st) {
+                                 float* dWp, int B, int Cin, int Cout, bool bf16, cudaStream_t st) {
   tcwp::Params p;
-  p.plan = plan_dev; p.fmt = operand_format_bits(); p.ps = ps; p.group = group; p.B = B; p.Cin = Cin; p.Cout = Cout; p.P = P;
+  p.plan = plan_dev; p.fmt = idesc_fmt_bits(bf16); p.ps = ps; p.group = group; p.B = B; p.Cin = Cin; p.Cout = Cout; p.P = P;
   p.X = reinterpret_cast<const __nv_bfloat16*>(Xb); p.dY = reinterpret_cast<const __nv_bfloat16*>(dYb); p.dWp = dWp;
   const int groups = (B + group - 1) / group;
   p.total_tiles = groups * ps.ntiles;
