@@ -102,6 +102,9 @@ _SIGS = {
     'gin_head_bwd': (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i64, _i, _i, _vp]),
     'gin_point_mesh_ws_bytes': (_sz, [_i, _i]),
     'gin_point_mesh_distance': (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp]),
+    'gin_chamfer_ws_bytes': (_sz, [_i, _i, _i]),
+    'gin_chamfer_fwd': (_i, [_vp, _i64, _i64, _i64, _vp, _i64, _i64, _i64, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _vp]),
+    'gin_chamfer_bwd': (_i, [_vp, _i64, _i64, _i64, _vp, _i64, _i64, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _vp]),
     'gin_vertex_normals_fwd': (_i, [_vp, _vp, _vp, _vp, _i, _vp]),
     'gin_laplacian_fwd': (_i, [_vp, _vp, _vp, _vp, _i, _vp]),
     'gin_ring_ops_ws_bytes': (_sz, [_i, _i]),

@@ -24,6 +24,7 @@
 #include "gin_bn.cuh"
 #include "gin_resample.cuh"
 #include "gin_dist.cuh"
+#include "gin_chamfer.cuh"
 #include "gin_head.cuh"
 
 static thread_local char g_err[512] = "";
@@ -672,6 +673,93 @@ int gin_point_mesh_distance(const float* points, const float* verts, const int32
   if (rc != GIN_OK) return rc;
   gin::dist::unpack_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>((const unsigned long long*)ws, dist, face_idx, (long long)n);
   return check_launch("point_mesh_unpack");
+}
+
+// ------------------------------------------------------------------ Chamfer distance (one nearest neighbour, both directions)
+size_t gin_chamfer_ws_bytes(int B, int N, int M) {
+  if (B <= 0 || N <= 0 || M <= 0) return 0;
+  return (size_t)B * (N > M ? N : M) * sizeof(gin::chamfer::Acc);     // >= the forward's 8 B * B * (N + M) of 64-bit keys
+}
+
+static int chamfer_args(const char* fn, const float* x, const float* y, void* ws, int B, int N, int M) {
+  if (B < 0) return fail(GIN_ERR_ARG, "%s: B=%d is negative", fn, B);
+  if (B == 0) return GIN_OK;
+  if (N < 1 || M < 1) return fail(GIN_ERR_ARG, "%s: empty point set (N=%d, M=%d)", fn, N, M);
+  if (B > 65535) return fail(GIN_ERR_ARG, "%s: B=%d exceeds 65535", fn, B);
+  if ((long long)B * (N > M ? N : M) > 0x7fffffffLL) return fail(GIN_ERR_ARG, "%s: B*max(N,M) exceeds 2^31-1", fn);
+  if (!x || !y || !ws) return fail(GIN_ERR_ARG, "%s: null pointer (x, y and ws are required)", fn);
+  return GIN_OK;
+}
+
+// best[b][i] over the queries q of their nearest candidate in c, then unpacked into d / idx
+static int chamfer_direction(gin::chamfer::Pts q, gin::chamfer::Pts c, int B, int Nq, int Nc, unsigned long long* keys, float* d,
+                             int32_t* idx, cudaStream_t st) {
+  namespace ch = gin::chamfer;
+  const long long n = (long long)B * Nq;
+  if (cudaMemsetAsync(keys, 0xFF, (size_t)n * sizeof(unsigned long long), st) != cudaSuccess) return fail(GIN_ERR_CUDA, "gin_chamfer_fwd: memset failed");
+  // Split the candidates when the queries alone give fewer than 4 CTAs per SM, down to one tile per split.
+  const int qblocks = (Nq + ch::kQueries - 1) / ch::kQueries;
+  const long long want = 4LL * gin::num_sms();
+  long long splits = (want + (long long)qblocks * B - 1) / ((long long)qblocks * B);
+  const long long max_splits = (Nc + ch::kTile - 1) / ch::kTile;
+  splits = splits < 1 ? 1 : (splits > max_splits ? max_splits : splits);
+  int split_len = (int)((Nc + splits - 1) / splits);
+  split_len = (split_len + ch::kChunk - 1) / ch::kChunk * ch::kChunk;
+  splits = (Nc + split_len - 1) / split_len;
+  ch::nn_kernel<<<dim3(qblocks, (unsigned)splits, B), ch::kThreads, 0, st>>>(q, c, Nq, Nc, split_len, keys);
+  int rc = check_launch("chamfer_nn");
+  if (rc != GIN_OK) return rc;
+  gin::dist::unpack_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(keys, d, idx, n);
+  return check_launch("chamfer_unpack");
+}
+
+int gin_chamfer_fwd(const float* x, int64_t xsb, int64_t xsn, int64_t xsc, const float* y, int64_t ysb, int64_t ysn, int64_t ysc,
+                    float* d_xy, int32_t* idx_xy, float* d_yx, int32_t* idx_yx, void* ws, int B, int N, int M, void* stream) {
+  int rc = chamfer_args("gin_chamfer_fwd", x, y, ws, B, N, M);
+  if (rc != GIN_OK || B == 0) return rc;
+  if ((idx_xy && !d_xy) || (idx_yx && !d_yx)) return fail(GIN_ERR_ARG, "gin_chamfer_fwd: an index output needs its distance output");
+  if (!d_xy && !d_yx) return fail(GIN_ERR_ARG, "gin_chamfer_fwd: null pointer (neither direction has an output)");
+  cudaStream_t st = (cudaStream_t)stream;
+  const gin::chamfer::Pts px{x, xsb, xsn, xsc}, py{y, ysb, ysn, ysc};
+  unsigned long long* keys = (unsigned long long*)ws;
+  if (d_xy && (rc = chamfer_direction(px, py, B, N, M, keys, d_xy, idx_xy, st)) != GIN_OK) return rc;
+  if (d_yx) rc = chamfer_direction(py, px, B, M, N, keys + (size_t)B * N, d_yx, idx_yx, st);
+  return rc;
+}
+
+// out = direct term of side D (g_d, idx_d: D's own direction, may be NULL) + scatter from the other side's entries (g_e, idx_e)
+static int chamfer_side(gin::chamfer::Pts D, gin::chamfer::Pts O, int B, int Nd, int No, const int32_t* idx_d, const float* g_d,
+                        const int32_t* idx_e, const float* g_e, float* out, void* ws, cudaStream_t st) {
+  namespace ch = gin::chamfer;
+  ch::Acc* acc = nullptr;
+  if (g_e) {
+    acc = (ch::Acc*)ws;
+    if (cudaMemsetAsync(acc, 0, (size_t)B * Nd * sizeof(ch::Acc), st) != cudaSuccess) return fail(GIN_ERR_CUDA, "gin_chamfer_bwd: memset failed");
+    const long long ne = (long long)B * No;
+    ch::scatter_stats_kernel<<<(unsigned)((ne + 255) / 256), 256, 0, st>>>(D, O, idx_e, g_e, acc, Nd, No, ne);
+    int rc = check_launch("chamfer_scatter_stats");
+    if (rc != GIN_OK) return rc;
+    ch::scatter_sum_kernel<<<(unsigned)((ne + 255) / 256), 256, 0, st>>>(D, O, idx_e, g_e, acc, Nd, No, ne);
+    if ((rc = check_launch("chamfer_scatter_sum")) != GIN_OK) return rc;
+  }
+  const long long nd = (long long)B * Nd;
+  ch::finish_kernel<<<(unsigned)((nd + 255) / 256), 256, 0, st>>>(D, O, idx_d, g_d, acc, out, Nd, nd);
+  return check_launch("chamfer_finish");
+}
+
+int gin_chamfer_bwd(const float* x, int64_t xsb, int64_t xsn, int64_t xsc, const float* y, int64_t ysb, int64_t ysn, int64_t ysc,
+                    const int32_t* idx_xy, const float* g_xy, const int32_t* idx_yx, const float* g_yx, float* dx, float* dy, void* ws,
+                    int B, int N, int M, void* stream) {
+  int rc = chamfer_args("gin_chamfer_bwd", x, y, ws, B, N, M);
+  if (rc != GIN_OK || B == 0) return rc;
+  if ((g_xy && !idx_xy) || (g_yx && !idx_yx)) return fail(GIN_ERR_ARG, "gin_chamfer_bwd: null pointer (a cotangent needs its indices)");
+  if (!g_xy && !g_yx) return fail(GIN_ERR_ARG, "gin_chamfer_bwd: null pointer (neither direction has a cotangent)");
+  if (!dx && !dy) return fail(GIN_ERR_ARG, "gin_chamfer_bwd: null pointer (neither dx nor dy is requested)");
+  cudaStream_t st = (cudaStream_t)stream;
+  const gin::chamfer::Pts px{x, xsb, xsn, xsc}, py{y, ysb, ysn, ysc};
+  if (dx && (rc = chamfer_side(px, py, B, N, M, g_xy ? idx_xy : nullptr, g_xy, idx_yx, g_yx, dx, ws, st)) != GIN_OK) return rc;
+  if (dy) rc = chamfer_side(py, px, B, M, N, g_yx ? idx_yx : nullptr, g_yx, idx_xy, g_xy, dy, ws, st);
+  return rc;
 }
 
 // ------------------------------------------------------------------ fused BatchNorm + activation + operand cast

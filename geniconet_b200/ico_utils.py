@@ -4,6 +4,8 @@ output2vertices     grid -> vertex list with averaged poles, on the GPU (gin_pol
 computeDistance     mode 'point2mesh': mean squared point-to-surface distance of the output vertices to the reference mesh
                     (ico_utils.py:26-44 over kaolin 0.9.1 point_to_mesh_distance), on the GPU (gin_point_mesh_distance)
 point_to_mesh_distance   the batched primitive underneath, same return convention as kaolin's (distance, face index)
+computeDistance     mode 'chamfer' (no counterpart in the reference): the symmetric mean squared Chamfer distance of the output and
+                    reference vertex sets, no correspondence needed (losses.chamfer_distance, gin_chamfer_fwd)
 
 The reference's logging / file helpers (saveDistance, getEpochNumber, save_to_file, get_*_shape; ico_utils.py:46-103) are host
 utilities outside the hot path (SURVEY 2.1 row 3) and are not provided.
@@ -14,7 +16,7 @@ import torch
 
 from . import _lib
 from .ico_conv import _stream
-from .losses import output2vertices  # noqa: F401  (ico_utils.py:10-24; the kernel-backed implementation lives with the losses)
+from .losses import chamfer_distance, output2vertices  # noqa: F401  (ico_utils.py:10-24; the kernel-backed implementation lives with the losses)
 
 
 def point_to_mesh_distance(pointclouds, vertices, faces):
@@ -59,10 +61,14 @@ def writeOffMesh(path, vertices, faces):
 
 def computeDistance(outvertices, refvertices, reffaces, f, mode='point2point', write_mesh=False, outfaces=None):
     """ico_utils.py:26-44.  outvertices [N,3], refvertices [V,3], reffaces [F,3]; 'point2mesh' -> numpy scalar, the mean
-    squared distance; any other mode -> None (as the reference)."""
+    squared distance; 'chamfer' -> numpy scalar, mean_i min_j |o_i - r_j|^2 + mean_j min_i |o_i - r_j|^2 (reffaces unused);
+    any other mode -> None (as the reference)."""
     if write_mesh:
         writeOffMesh(f, outvertices, reffaces if outfaces is None else outfaces)
     if mode == 'point2mesh':
         dist, _ = point_to_mesh_distance(outvertices[None, :, :], refvertices[None, :, :], reffaces)
         return torch.mean(dist).cpu().numpy()
+    if mode == 'chamfer':
+        d_xy, _, d_yx, _ = chamfer_distance(outvertices[None, :, :], refvertices[None, :, :])
+        return (torch.mean(d_xy) + torch.mean(d_yx)).cpu().numpy()
     return None

@@ -264,6 +264,25 @@ size_t gin_point_mesh_ws_bytes(int B, int N);
 int gin_point_mesh_distance(const float* points, const float* verts, const int32_t* faces, float* dist, int32_t* face_idx,
                             void* ws, int B, int N, int V, int F, void* stream);
 
+/* ------------------------------------------------------------------ device: Chamfer distance --- */
+/* One nearest neighbour between two batched fp32 point sets, x [B][N][3] and y [B][M][3], read with element strides (element (b, i, c)
+ * of x at x[b*xsb + i*xsn + c*xsc]; the xyz rows of a [B][9][V] target are (9*V, 1, V)).  Brute force on the fp32 CUDA cores.
+ * Forward: d_xy [B][N] = squared distance of x_i to its nearest point of y, idx_xy [B][N] = that point's index (int32; the lowest
+ * index among equal distances); d_yx / idx_yx [B][M] the same towards x.  A direction runs when its distance output is given;
+ * its index output may be NULL, an index output without its distance output is an error.  The distance is recomputed in
+ * difference form for the chosen pair.  Deterministic.
+ * Backward: dx [B][N][3] = 2 g_xy_i (x_i - y_idx_xy(i)) + sum_{j : idx_yx(j) = i} 2 g_yx_j (x_i - y_j), dy [B][M][3] symmetrically
+ * (both contiguous; either may be NULL, not both).  g_xy [B][N] / g_yx [B][M] are the cotangents of d_xy / d_yx; either may be NULL
+ * (one-sided loss), not both; a cotangent needs its indices.  The scatter sum is exact int64 fixed point: bit-reproducible, no
+ * floating-point atomics.
+ * ws: gin_chamfer_ws_bytes(B, N, M), contents irrelevant.  B = 0: no-op.  Needs N, M >= 1, B <= 65535, B*max(N, M) < 2^31. */
+size_t gin_chamfer_ws_bytes(int B, int N, int M);
+int gin_chamfer_fwd(const float* x, int64_t xsb, int64_t xsn, int64_t xsc, const float* y, int64_t ysb, int64_t ysn, int64_t ysc,
+                    float* d_xy, int32_t* idx_xy, float* d_yx, int32_t* idx_yx, void* ws, int B, int N, int M, void* stream);
+int gin_chamfer_bwd(const float* x, int64_t xsb, int64_t xsn, int64_t xsc, const float* y, int64_t ysb, int64_t ysn, int64_t ysc,
+                    const int32_t* idx_xy, const float* g_xy, const int32_t* idx_yx, const float* g_yx, float* dx, float* dy, void* ws,
+                    int B, int N, int M, void* stream);
+
 /* ------------------------------------------------------------------ device: optimizer step --- */
 /* The Adam step of the training loop (run.py:446 `torch.optim.Adam(model.parameters(), lr)`, run.py:250 `optimizer.step()`) over
  * a LIST of fp32 tensors in one launch; same arithmetic as torch.optim.Adam (amsgrad = maximize = False, L2 weight_decay):
