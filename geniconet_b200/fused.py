@@ -511,8 +511,10 @@ def _bn_table(pairs):
     buffer it fills: per entry scale [C], shift [C] (conv bias folded in), stat [4][C] (gin_bn_act_fwd layout, no bias).  Cached
     per set of parameter storages: the table holds pointers only, so in-place load_state_dict needs no rebuild, and a captured
     graph reads the current values at every replay."""
-    key = tuple((id(bn), bn.weight.data_ptr(), bn.bias.data_ptr(), bn.running_mean.data_ptr(), bn.running_var.data_ptr(), float(bn.eps),
-                 b.data_ptr() if b is not None else 0) for bn, b in pairs)
+    # num_features too: a BatchNorm created after another one died can get its id() and, from the caching allocator, the same
+    # storage addresses with a different width
+    key = tuple((id(bn), bn.num_features, bn.weight.data_ptr(), bn.bias.data_ptr(), bn.running_mean.data_ptr(), bn.running_var.data_ptr(),
+                 float(bn.eps), b.data_ptr() if b is not None else 0) for bn, b in pairs)
     hit = _EVAL_CACHE.get(key)
     if hit is not None:
         return hit

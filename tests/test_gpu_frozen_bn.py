@@ -87,6 +87,27 @@ def _consts(C, seed):
     return fused._eval_consts([(bn, None)])[0][2].clone().view(4, C)      # stat [4][C]
 
 
+def test_eval_consts_follow_the_width_at_the_same_addresses():
+    """The constants cache (fused._bn_table) must not hand a BatchNorm the table of another width that had the same id() and storage
+    addresses, as one created after another died can have (the caching allocator reuses the blocks).  Modelled here by one module
+    narrowed in place to the leading half of its own storages."""
+    bn = torch.nn.BatchNorm2d(128).cuda().eval()
+    g = torch.Generator().manual_seed(3)
+    with torch.no_grad():
+        bn.weight.copy_(1 + 0.3 * torch.randn(128, generator=g))
+        bn.bias.copy_(0.2 * torch.randn(128, generator=g))
+        bn.running_mean.copy_(0.3 * torch.randn(128, generator=g))
+        bn.running_var.copy_(0.5 + torch.rand(128, generator=g))
+    assert fused._eval_consts([(bn, None)])[0][2].numel() == 4 * 128
+    bn.weight, bn.bias = torch.nn.Parameter(bn.weight.data[:64]), torch.nn.Parameter(bn.bias.data[:64])
+    bn.running_mean, bn.running_var, bn.num_features = bn.running_mean[:64], bn.running_var[:64], 64
+    scale, shift, stat = fused._eval_consts([(bn, None)])[0]
+    assert (scale.numel(), shift.numel(), stat.numel()) == (64, 64, 4 * 64)
+    want = bn.weight.detach() / torch.sqrt(bn.running_var + bn.eps)
+    torch.testing.assert_close(scale, want, rtol=1e-5, atol=0)
+    torch.testing.assert_close(shift, bn.bias.detach() - bn.running_mean * want, rtol=1e-5, atol=1e-6)
+
+
 def _ptr(t, off=0):
     return t.data_ptr() + off if t is not None else None
 
