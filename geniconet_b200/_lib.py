@@ -105,6 +105,9 @@ _SIGS = {
     'gin_chamfer_ws_bytes': (_sz, [_i, _i, _i]),
     'gin_chamfer_fwd': (_i, [_vp, _i64, _i64, _i64, _vp, _i64, _i64, _i64, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _vp]),
     'gin_chamfer_bwd': (_i, [_vp, _i64, _i64, _i64, _vp, _i64, _i64, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _vp]),
+    'gin_chamfer_terms_ws_bytes': (_sz, [_i, _i, _i]),
+    'gin_chamfer_terms_fwd': (_i, [_vp, _vp, _vp, _vp, _i64, _i64, _i64, _vp, _i64, _i64, _i64, _vp, _vp, _vp, _vp, _i, _i, _vp]),
+    'gin_chamfer_terms_bwd': (_i, [_vp, _vp, _vp, _vp, _i64, _i64, _i64, _vp, _i64, _i64, _i64, _vp, _vp, _vp, _vp, _vp, _i, _i, _vp]),
     'gin_vertex_normals_fwd': (_i, [_vp, _vp, _vp, _vp, _i, _vp]),
     'gin_laplacian_fwd': (_i, [_vp, _vp, _vp, _vp, _i, _vp]),
     'gin_ring_ops_ws_bytes': (_sz, [_i, _i]),

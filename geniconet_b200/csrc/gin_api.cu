@@ -25,6 +25,7 @@
 #include "gin_resample.cuh"
 #include "gin_dist.cuh"
 #include "gin_chamfer.cuh"
+#include "gin_chamfer_terms.cuh"
 #include "gin_head.cuh"
 
 static thread_local char g_err[512] = "";
@@ -678,7 +679,7 @@ int gin_point_mesh_distance(const float* points, const float* verts, const int32
 // ------------------------------------------------------------------ Chamfer distance (one nearest neighbour, both directions)
 size_t gin_chamfer_ws_bytes(int B, int N, int M) {
   if (B <= 0 || N <= 0 || M <= 0) return 0;
-  return (size_t)B * (N > M ? N : M) * sizeof(gin::chamfer::Acc);     // >= the forward's 8 B * B * (N + M) of 64-bit keys
+  return (size_t)B * (N > M ? N : M) * sizeof(gin::fixsum::Acc);     // >= the forward's 8 B * B * (N + M) of 64-bit keys
 }
 
 static int chamfer_args(const char* fn, const float* x, const float* y, void* ws, int B, int N, int M) {
@@ -1093,6 +1094,90 @@ int gin_p2p_loss_bwd(const void* plan_host, const void* plan_dev, const float* x
   if ((rc = check_launch("p2p_bwd_gather"))) return rc;
   gin::pole_vertices_bwd_kernel<<<grid_for((long long)B * h->P * 3, 256), 256, 0, st>>>(plan_words(plan_dev), dv, dx, sb, sp, sc, B, 3);
   return check_launch("pole_vertices_bwd");
+}
+
+
+// ------------------------------------------------------------------ Chamfer normal and Laplacian terms (matched through the indices)
+// workspace layout: forward [partials: 1024*4 f64]; backward [g_n: B*V*3 f32][g_L: B*V*3 f32][acc_n: B*V Acc][acc_L: B*V Acc], the
+// gin_ring_ops_bwd workspace (B*V*6 f32) reusing acc_n once the cotangents are formed
+size_t gin_chamfer_terms_ws_bytes(int B, int level, int M) {
+  if (B <= 0 || level < 0 || level > 9 || M < 1) return 0;
+  const size_t BV = (size_t)B * ((size_t)(10 << (2 * level)) + 2);
+  const size_t bwd = BV * (2 * 3 * 4 + 2 * sizeof(gin::fixsum::Acc));
+  const size_t fwd = (size_t)gin::chamfer_terms::kMaxParts * 4 * 8;
+  return bwd > fwd ? bwd : fwd;
+}
+
+static int chamfer_terms_args(const char* fn, const void* plan_host, const void* plan_dev, const float* v, const float* tn, const float* tl,
+                              const int32_t* idx_xy, const int32_t* idx_yx, const void* out, void* ws, int B, int M,
+                              const GinLossPlanHdr** h) {
+  if (B < 0) return fail(GIN_ERR_ARG, "%s: B=%d is negative", fn, B);
+  if (M < 1) return fail(GIN_ERR_ARG, "%s: M=%d, the target needs at least one point", fn, M);
+  int rc = loss_hdr(plan_host, plan_dev, h);
+  if (rc) return rc;
+  if ((*h)->level < 0 || (*h)->level > 9) return fail(GIN_ERR_ARG, "%s: bad level %d", fn, (*h)->level);
+  if ((long long)B * ((*h)->V > M ? (*h)->V : M) > 0x7fffffffLL) return fail(GIN_ERR_ARG, "%s: B*max(V,M) exceeds 2^31-1", fn);
+  if (B == 0) return GIN_OK;
+  if (!v || !out || !ws) return fail(GIN_ERR_ARG, "%s: null pointer (v, the output and ws are required)", fn);
+  if (!tn && !tl) return fail(GIN_ERR_ARG, "%s: null pointer (neither target normals nor target Laplacians)", fn);
+  if (!idx_xy && !idx_yx) return fail(GIN_ERR_ARG, "%s: null pointer (neither direction has indices)", fn);
+  return GIN_OK;
+}
+
+int gin_chamfer_terms_fwd(const void* plan_host, const void* plan_dev, const float* v, const float* tn, int64_t tnsb, int64_t tnsn,
+                          int64_t tnsc, const float* tl, int64_t tlsb, int64_t tlsn, int64_t tlsc, const int32_t* idx_xy,
+                          const int32_t* idx_yx, float* out, void* ws, int B, int M, void* stream) {
+  namespace ct = gin::chamfer_terms;
+  const GinLossPlanHdr* h;
+  int rc = chamfer_terms_args("gin_chamfer_terms_fwd", plan_host, plan_dev, v, tn, tl, idx_xy, idx_yx, out, ws, B, M, &h);
+  if (rc != GIN_OK || B == 0) return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+  ct::Args a{};
+  a.plan = plan_words(plan_dev); a.v = v;
+  a.tn = gin::chamfer::Pts{tn, tnsb, tnsn, tnsc}; a.tl = gin::chamfer::Pts{tl, tlsb, tlsn, tlsc};
+  a.idx_xy = idx_xy; a.idx_yx = idx_yx;
+  a.partial = reinterpret_cast<double*>(ws);
+  a.B = B; a.M = M;
+  const long long BV = (long long)B * h->V, BM = (long long)B * M;
+  int parts = grid_for((idx_xy ? BV : 0) + (idx_yx ? BM : 0), ct::kThreads, 4);
+  if (parts > ct::kMaxParts) parts = ct::kMaxParts;
+  ct::fwd_kernel<<<parts, ct::kThreads, 0, st>>>(a);
+  if ((rc = check_launch("chamfer_terms_fwd"))) return rc;
+  ct::final_kernel<<<1, ct::kThreads, 0, st>>>(a.partial, parts, out, 1.0 / (double)BV, 1.0 / (double)BM);
+  return check_launch("chamfer_terms_final");
+}
+
+int gin_chamfer_terms_bwd(const void* plan_host, const void* plan_dev, const float* v, const float* tn, int64_t tnsb, int64_t tnsn,
+                          int64_t tnsc, const float* tl, int64_t tlsb, int64_t tlsn, int64_t tlsc, const int32_t* idx_xy,
+                          const int32_t* idx_yx, const float* dout, float* dv, void* ws, int B, int M, void* stream) {
+  namespace ct = gin::chamfer_terms;
+  const GinLossPlanHdr* h;
+  int rc = chamfer_terms_args("gin_chamfer_terms_bwd", plan_host, plan_dev, v, tn, tl, idx_xy, idx_yx, dv, ws, B, M, &h);
+  if (rc != GIN_OK || B == 0) return rc;
+  if (!dout) return fail(GIN_ERR_ARG, "gin_chamfer_terms_bwd: null pointer (dout is required)");
+  cudaStream_t st = (cudaStream_t)stream;
+  const long long BV = (long long)B * h->V, BM = (long long)B * M;
+  ct::Args a{};
+  a.plan = plan_words(plan_dev); a.v = v;
+  a.tn = gin::chamfer::Pts{tn, tnsb, tnsn, tnsc}; a.tl = gin::chamfer::Pts{tl, tlsb, tlsn, tlsc};
+  a.idx_xy = idx_xy; a.idx_yx = idx_yx; a.dout = dout;
+  a.g_n = reinterpret_cast<float*>(ws);
+  a.g_l = a.g_n + BV * 3;
+  a.acc_n = reinterpret_cast<gin::fixsum::Acc*>(a.g_l + BV * 3);
+  a.acc_l = a.acc_n + BV;
+  a.B = B; a.M = M;
+  if (idx_yx) {
+    if (cudaMemsetAsync(a.acc_n, 0, (size_t)BV * 2 * sizeof(gin::fixsum::Acc), st) != cudaSuccess)
+      return fail(GIN_ERR_CUDA, "gin_chamfer_terms_bwd: memset failed");
+    const unsigned blocks = (unsigned)((BM + ct::kThreads - 1) / ct::kThreads);
+    ct::scatter_kernel<false><<<blocks, ct::kThreads, 0, st>>>(a);
+    if ((rc = check_launch("chamfer_terms_scatter_stats"))) return rc;
+    ct::scatter_kernel<true><<<blocks, ct::kThreads, 0, st>>>(a);
+    if ((rc = check_launch("chamfer_terms_scatter_sum"))) return rc;
+  }
+  ct::cotangent_kernel<<<(unsigned)((BV + ct::kThreads - 1) / ct::kThreads), ct::kThreads, 0, st>>>(a);
+  if ((rc = check_launch("chamfer_terms_cotangents"))) return rc;
+  return gin_ring_ops_bwd(plan_host, plan_dev, v, tn ? a.g_n : nullptr, tl ? a.g_l : nullptr, dv, a.acc_n, B, stream);
 }
 
 }  // extern "C"

@@ -17,14 +17,12 @@
 // smallest distance and, among equal distances, the lowest index, whatever the order the CTAs finish in.
 //
 // Backward: dx_i = 2 g_xy_i (x_i - y_idx_xy(i))  +  sum_{j : idx_yx(j) = i} 2 g_yx_j (x_i - y_j), symmetrically for dy.  The first
-// term is a gather.  The second is a scatter, summed without floating-point atomics in exact int64 fixed point: a first pass takes,
-// per receiving point, the largest exponent of its terms and their count (integer atomicMax / atomicAdd); a second pass rounds
-// every term to the grid 2^-s of that point (s chosen so that count terms cannot overflow 62 bits) and adds the integers with
-// 64-bit integer atomics -- integer addition is associative, so the sum is the same bits whatever the order; the finishing pass
-// converts it back.  Every term within 2^-38 of its point's largest term keeps all of its fp32 bits.
+// term is a gather.  The second is a scatter, summed without floating-point atomics in exact int64 fixed point (gin_fixed_scatter.cuh):
+// scatter_stats_kernel is its first pass, scatter_sum_kernel its second, and finish_kernel reads the sums back.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include "gin_fixed_scatter.cuh"
 
 namespace gin {
 namespace chamfer {
@@ -140,23 +138,14 @@ __global__ void __launch_bounds__(kThreads) nn_kernel(Pts q, Pts c, int Nq, int 
 }
 
 // ---------------------------------------------------------------------------------------------------------------- backward
-// Scatter workspace, per receiving point r of one side: Acc {int64 sum[3]; int32 exponent; int32 count} (32 B), zeroed.
-struct Acc { long long s[3]; int e; int n; };
+// Scatter workspace, per receiving point r of one side: a fixsum::Acc (32 B), zeroed.
+using fixsum::Acc;
 
 // term of entry e (a point of the other side, whose nearest point on this side is r = idx[e]): 2 g_e (S_r - E_e)
 __device__ __forceinline__ void scatter_term(const Pts& S, const Pts& E, int b, int e, int r, float g, float t[3]) {
 #pragma unroll
   for (int k = 0; k < 3; ++k) t[k] = 2.f * g * (S.at(b, r, k) - E.at(b, e, k));
 }
-
-// biased fp32 exponent of the largest component (0 for zeros)
-__device__ __forceinline__ int max_exponent(const float t[3]) {
-  const unsigned m = max(max(__float_as_uint(t[0]) & 0x7fffffffu, __float_as_uint(t[1]) & 0x7fffffffu), __float_as_uint(t[2]) & 0x7fffffffu);
-  return (int)(m >> 23);
-}
-
-// 2^shift such that count terms below 2^(e - 126) (biased exponent e) sum to less than 2^62
-__device__ __forceinline__ int fixed_shift(const Acc& a) { return 61 - (a.e - 127) - (32 - __clz(max(a.n, 1))); }
 
 __global__ void scatter_stats_kernel(Pts S, Pts E, const int32_t* __restrict__ idx, const float* __restrict__ g, Acc* __restrict__ acc,
                                      int Ns, int Ne, long long n) {
@@ -166,9 +155,7 @@ __global__ void scatter_stats_kernel(Pts S, Pts E, const int32_t* __restrict__ i
   const int r = idx[t];
   float v[3];
   scatter_term(S, E, b, e, r, g[t], v);
-  Acc* a = acc + (long long)b * Ns + r;
-  atomicMax(&a->e, max_exponent(v));
-  atomicAdd(&a->n, 1);
+  fixsum::note(acc + (long long)b * Ns + r, v);
 }
 
 __global__ void scatter_sum_kernel(Pts S, Pts E, const int32_t* __restrict__ idx, const float* __restrict__ g, Acc* __restrict__ acc,
@@ -179,14 +166,7 @@ __global__ void scatter_sum_kernel(Pts S, Pts E, const int32_t* __restrict__ idx
   const int r = idx[t];
   float v[3];
   scatter_term(S, E, b, e, r, g[t], v);
-  Acc* a = acc + (long long)b * Ns + r;
-  if (a->e == 0) return;                         // every term of this point is zero
-  const int sh = fixed_shift(*a);
-#pragma unroll
-  for (int k = 0; k < 3; ++k) {
-    const long long q = __double2ll_rn(ldexp((double)v[k], sh));      // exact scaling, one rounding to the grid
-    atomicAdd(reinterpret_cast<unsigned long long*>(&a->s[k]), (unsigned long long)q);
-  }
+  fixsum::add(acc + (long long)b * Ns + r, v);
 }
 
 // out[b][d][3] = 2 g_d (D_d - O_idx(d))  (when g != NULL)  +  the fixed-point scatter sum of d (when acc != NULL)
@@ -202,14 +182,7 @@ __global__ void finish_kernel(Pts D, Pts O, const int32_t* __restrict__ idx, con
 #pragma unroll
     for (int k = 0; k < 3; ++k) v[k] = 2.f * gd * (D.at(b, d, k) - O.at(b, o, k));
   }
-  if (acc) {
-    const Acc a = acc[t];
-    if (a.e != 0) {
-      const int sh = fixed_shift(a);
-#pragma unroll
-      for (int k = 0; k < 3; ++k) v[k] += (float)ldexp((double)a.s[k], -sh);
-    }
-  }
+  if (acc) fixsum::read(acc[t], v);
 #pragma unroll
   for (int k = 0; k < 3; ++k) out[t * 3 + k] = v[k];
 }

@@ -7,7 +7,8 @@ Same class names, constructor arguments, forward contracts and ``get_last_losses
     P2PKLD_Loss                 (losses.py:131-145)
 
 and, with no counterpart in the reference (run.py:629-630 only names it as an option), the Chamfer reconstruction loss against a
-point set without vertex correspondence: chamfer_distance, Chamfer_Loss, ChamferKLD_Loss (csrc/gin_chamfer.cuh).
+point set without vertex correspondence: chamfer_distance, Chamfer_Loss, ChamferKLD_Loss (csrc/gin_chamfer.cuh), with optional
+normal and Laplacian terms matched through the nearest neighbours (csrc/gin_chamfer_terms.cuh).
 
 The pole averaging (losses.py:22-31,49-51), vertex normals, Laplacian and the three reductions run
 as one fused CUDA pipeline (csrc/gin_loss.cuh); the scalar read-backs the reference does with
@@ -220,49 +221,139 @@ def _target_points(target, what):
     raise ValueError('%s: expected a point set [B,M,3] or a target [B,9,V], got %s' % (what, tuple(target.shape)))
 
 
+def _target_rows(target, what):
+    """(points, normals, Laplacians) of a Chamfer target as [B,M,3] views (no copy); a part the target lacks is None.
+
+    [B,M,3] points; [B,M,6] points and normals; [B,M,9] points, normals and Laplacians; or the data-path target [B,9,V] (rows 0-2,
+    3-5, 6-8).  A [B,9,K] tensor with K != 3 is read as the data-path target, as _target_points reads it."""
+    if target.dim() == 3 and target.shape[-1] != 3 and target.shape[1] == 9:
+        return tuple(target[:, r:r + 3, :].transpose(1, 2) for r in (0, 3, 6))
+    if target.dim() == 3 and target.shape[-1] in (3, 6, 9):
+        return tuple(target[..., r:r + 3] if r < target.shape[-1] else None for r in (0, 3, 6))
+    raise ValueError('%s: expected a point set [B,M,3], [B,M,6] (with normals), [B,M,9] (with normals and Laplacians) or a target '
+                     '[B,9,V], got %s' % (what, tuple(target.shape)))
+
+
+class _ChamferTermsFn(torch.autograd.Function):
+    """(nor_xy, nor_yx, lap_xy, lap_yx) of the output vertices v [B,V,3] against the target normals tn / Laplacians tl [B,M,3]
+    (any strides; None: that term is 0) through the nearest-neighbour indices i_xy [B,V] / i_yx [B,M] (None: that direction is 0);
+    gin_chamfer_terms_fwd / _bwd.  Differentiable in v only."""
+
+    @staticmethod
+    def forward(ctx, v, tn, tl, i_xy, i_yx, level):
+        _require_cuda_f32(v, 'Chamfer_Loss')
+        for t in (tn, tl):
+            if t is not None:
+                _require_cuda_f32(t, 'Chamfer_Loss')
+        B, M = v.shape[0], (tn if tn is not None else tl).shape[1]
+        plan = get_plan(_lib.PLAN_LOSS, level, 1, 'average', v.device)
+        v = v.contiguous()
+        out = torch.empty(4, dtype=torch.float32, device=v.device)
+        ws = torch.empty(max(1, _lib.lib.gin_chamfer_terms_ws_bytes(B, level, M)), dtype=torch.uint8, device=v.device)
+        _lib.check(_lib.lib.gin_chamfer_terms_fwd(plan.host_ptr, plan.dev_ptr, v.data_ptr(), *_rows_arg(tn), *_rows_arg(tl), _ptr(i_xy),
+                                                  _ptr(i_yx), out.data_ptr(), ws.data_ptr(), B, M, _stream()), 'gin_chamfer_terms_fwd')
+        ctx.plan, ctx.level, ctx.M = plan, level, M
+        ctx.save_for_backward(v, tn, tl, i_xy, i_yx)
+        return out
+
+    @staticmethod
+    def backward(ctx, dout):
+        v, tn, tl, i_xy, i_yx = ctx.saved_tensors
+        B = v.shape[0]
+        dout = dout.contiguous().float()
+        dv = torch.empty_like(v)
+        ws = torch.empty(max(1, _lib.lib.gin_chamfer_terms_ws_bytes(B, ctx.level, ctx.M)), dtype=torch.uint8, device=v.device)
+        _lib.check(_lib.lib.gin_chamfer_terms_bwd(ctx.plan.host_ptr, ctx.plan.dev_ptr, v.data_ptr(), *_rows_arg(tn), *_rows_arg(tl),
+                                                  _ptr(i_xy), _ptr(i_yx), dout.data_ptr(), dv.data_ptr(), ws.data_ptr(), B, ctx.M,
+                                                  _stream()), 'gin_chamfer_terms_bwd')
+        return dv, None, None, None, None, None
+
+
+def _ptr(t):
+    return None if t is None else t.data_ptr()
+
+
+def _rows_arg(t):
+    return (None, 0, 0, 0) if t is None else (t.data_ptr(), *t.stride())
+
+
 class Chamfer_Loss(torch.nn.Module):
     """Chamfer reconstruction loss between the output vertices and a point set without vertex correspondence:
 
-        mean_b( factor_xy * mean_i d_xy  +  factor_yx * mean_j d_yx )
+        factor_xy * l_xy  +  factor_yx * l_yx  +  factor_nor * l_nor  +  factor_lap * l_lap
 
-    with d_xy the squared distance of output vertex i (output2vertices: the grid plus the two averaged poles) to its nearest target
-    point and d_yx that of target point j to its nearest output vertex.  `target` is a point set [B,M,3] (a scan, surface samples)
-    or the data-path target [B,9,P+2], whose xyz rows are used.  A direction whose factor is 0 is not computed (one-sided loss for
-    partial scans).  forward never synchronises with the host."""
+    v = output2vertices(s, out) [B,V,3] (the grid plus the two averaged poles, V = 10*4^s + 2); i_xy(i) is the nearest target point
+    of output vertex i and i_yx(j) the nearest output vertex of target point j (chamfer_distance), d_xy / d_yx their squared
+    distances, n_i / L_i the vertex normal and uniform Laplacian of v (exactly gin_vertex_normals_fwd / gin_laplacian_fwd on the
+    level-s loss plan), tn_j / tl_j the target's normal and Laplacian at point j:
 
-    def __init__(self, subdivisions, factor_xy=1.0, factor_yx=1.0):
+        l_xy = mean_{b,i} d_xy                                   l_yx = mean_{b,j} d_yx
+        nor_xy = mean_{b,i} (1 - cos(n_i, tn_{i_xy(i)}))        nor_yx = mean_{b,j} (1 - cos(tn_j, n_{i_yx(j)}))
+        lap_xy = mean_{b,i,c} (L_i - tl_{i_xy(i)})_c^2           lap_yx = mean_{b,j,c} (tl_j - L_{i_yx(j)})_c^2
+
+    cos takes the eps of P2P_Loss (kCosEps on each norm, kNormalEps inside the normal).  l_nor is the mean of nor_* over the enabled
+    directions, those whose position factor is non-zero; l_lap likewise.  The gradient flows into v through the distances, n and L;
+    the nearest-neighbour choice is piecewise constant and not differentiated, and the target gets no gradient.  When the target is
+    the output grid itself, i_xy is the identity and the xy direction alone gives exactly P2P_Loss's l_nor and l_lap.
+
+    `target` is a point set [B,M,3] (a scan, surface samples), [B,M,6] with normals, [B,M,9] with normals and Laplacians, or the
+    data-path target [B,9,P+2], read in place.  factor_nor != 0 needs target normals and factor_lap != 0 target Laplacians
+    (ValueError otherwise).  A direction whose factor is 0 is not computed (one-sided loss for partial scans), and with factor_nor =
+    factor_lap = 0 nothing beyond the position terms runs.  forward never synchronises with the host."""
+
+    def __init__(self, subdivisions, factor_xy=1.0, factor_yx=1.0, factor_nor=0.0, factor_lap=0.0):
         super().__init__()
         self.subdivisions = int(subdivisions)
         self.factor_xy, self.factor_yx = float(factor_xy), float(factor_yx)
+        self.factor_nor, self.factor_lap = float(factor_nor), float(factor_lap)
         if not (self.factor_xy or self.factor_yx):
             raise ValueError('Chamfer_Loss: factor_xy and factor_yx are both 0')
         self._last = None
 
     def forward(self, inputs, target):
         v = output2vertices(self.subdivisions, inputs)
-        y = _target_points(target, 'Chamfer_Loss')
+        y, tn, tl = _target_rows(target, 'Chamfer_Loss')
+        if self.factor_nor and tn is None:
+            raise ValueError('Chamfer_Loss: factor_nor=%g needs target normals ([B,M,6], [B,M,9] or [B,9,V]), got %s'
+                             % (self.factor_nor, tuple(target.shape)))
+        if self.factor_lap and tl is None:
+            raise ValueError('Chamfer_Loss: factor_lap=%g needs target Laplacians ([B,M,9] or [B,9,V]), got %s'
+                             % (self.factor_lap, tuple(target.shape)))
         if y.shape[0] != v.shape[0]:
             raise ValueError('Chamfer_Loss: batch sizes differ (%d vs %d)' % (v.shape[0], y.shape[0]))
-        d_xy, _, d_yx, _ = chamfer_distance(v, y, xy=self.factor_xy != 0, yx=self.factor_yx != 0)
+        d_xy, i_xy, d_yx, i_yx = chamfer_distance(v, y, xy=self.factor_xy != 0, yx=self.factor_yx != 0)
         zero = v.new_zeros(())
         l_xy = d_xy.mean() if d_xy is not None else zero
         l_yx = d_yx.mean() if d_yx is not None else zero
         loss = self.factor_xy * l_xy + self.factor_yx * l_yx
-        self._last = torch.stack([l_xy, l_yx, loss]).detach()
+        if not (self.factor_nor or self.factor_lap):
+            self._last = torch.stack([l_xy, l_yx, loss]).detach()
+            return loss
+        t = _ChamferTermsFn.apply(v, tn if self.factor_nor else None, tl if self.factor_lap else None, i_xy, i_yx, self.subdivisions)
+        if i_xy is not None and i_yx is not None:
+            l_nor, l_lap = 0.5 * (t[0] + t[1]), 0.5 * (t[2] + t[3])
+        else:
+            d = 0 if i_xy is not None else 1
+            l_nor, l_lap = t[d], t[2 + d]
+        loss = loss + self.factor_nor * l_nor + self.factor_lap * l_lap
+        self._last = torch.stack([l_xy, l_yx, l_nor, l_lap, loss]).detach()
         return loss
 
     def get_last_losses(self):
+        """(l_xy, l_yx, l_nor, l_lap, total); l_nor and l_lap are 0 when their factor is."""
         if self._last is None:
             return 0., 0., 0., 0., 0.
-        l_xy, l_yx, total = (float(v) for v in self._last.tolist())     # one device->host read
-        return l_xy, l_yx, 0., 0., total
+        last = [float(v) for v in self._last.tolist()]     # one device->host read
+        if len(last) == 3:
+            return last[0], last[1], 0., 0., last[2]
+        return tuple(last)
 
 
 class ChamferKLD_Loss(Chamfer_Loss, KLD_Loss):
     """Chamfer_Loss on the reconstruction plus factor_kl * KLD_Loss, composed as P2PKLD_Loss composes P2P_Loss."""
 
-    def __init__(self, subdivisions, factor_xy, factor_yx, factor_kl):
-        Chamfer_Loss.__init__(self, subdivisions, factor_xy, factor_yx)
+    def __init__(self, subdivisions, factor_xy, factor_yx, factor_kl, factor_nor=0.0, factor_lap=0.0):
+        Chamfer_Loss.__init__(self, subdivisions, factor_xy, factor_yx, factor_nor, factor_lap)
         self.factor_kl = factor_kl
 
     def forward(self, output, target):

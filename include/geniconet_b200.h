@@ -282,6 +282,25 @@ int gin_chamfer_fwd(const float* x, int64_t xsb, int64_t xsn, int64_t xsc, const
 int gin_chamfer_bwd(const float* x, int64_t xsb, int64_t xsn, int64_t xsc, const float* y, int64_t ysb, int64_t ysn, int64_t ysc,
                     const int32_t* idx_xy, const float* g_xy, const int32_t* idx_yx, const float* g_yx, float* dx, float* dy, void* ws,
                     int B, int N, int M, void* stream);
+/* Normal and Laplacian terms of the Chamfer loss, matched through the nearest-neighbour indices of gin_chamfer_fwd.  v [B][V][3]
+ * contiguous, V = P+2 of the level-s loss plan; n_i / L_i are its vertex normal and uniform Laplacian exactly as
+ * gin_vertex_normals_fwd / gin_laplacian_fwd compute them; tn / tl are the target's normals / Laplacians [B][M][3], read with
+ * element strides like gin_chamfer_fwd's inputs (rows 3-5 / 6-8 of a [B][9][V] target: (9*V, 1, V)); idx_xy [B][V], idx_yx [B][M]:
+ *   out[0] nor_xy = mean_{b,i} (1 - cos(n_i, tn_{idx_xy(i)}))      out[1] nor_yx = mean_{b,j} (1 - cos(tn_j, n_{idx_yx(j)}))
+ *   out[2] lap_xy = mean_{b,i,c} (L_i - tl_{idx_xy(i)})_c^2         out[3] lap_yx = mean_{b,j,c} (tl_j - L_{idx_yx(j)})_c^2
+ * cos with the eps of gin_p2p_loss_fwd.  A NULL tn / tl switches the normal / Laplacian terms off, a NULL idx_xy / idx_yx that
+ * direction; a term that is off reads 0 (at least one of tn, tl and one of idx_xy, idx_yx are needed).  Deterministic.
+ * Backward: dv [B][V][3] = the gradient of sum_k dout[k] out[k] (dout: device [4]) through n and L; the indices are not
+ * differentiated and the target gets no gradient.  The yx part is scattered in exact int64 fixed point: bit-reproducible, no
+ * floating-point atomics.
+ * ws: gin_chamfer_terms_ws_bytes(B, level, M), contents irrelevant.  B = 0: no-op.  Needs M >= 1, B*max(V, M) < 2^31. */
+size_t gin_chamfer_terms_ws_bytes(int B, int level, int M);
+int gin_chamfer_terms_fwd(const void* plan_host, const void* plan_dev, const float* v, const float* tn, int64_t tnsb, int64_t tnsn,
+                          int64_t tnsc, const float* tl, int64_t tlsb, int64_t tlsn, int64_t tlsc, const int32_t* idx_xy,
+                          const int32_t* idx_yx, float* out, void* ws, int B, int M, void* stream);
+int gin_chamfer_terms_bwd(const void* plan_host, const void* plan_dev, const float* v, const float* tn, int64_t tnsb, int64_t tnsn,
+                          int64_t tnsc, const float* tl, int64_t tlsb, int64_t tlsn, int64_t tlsc, const int32_t* idx_xy,
+                          const int32_t* idx_yx, const float* dout /* device [4] */, float* dv, void* ws, int B, int M, void* stream);
 
 /* ------------------------------------------------------------------ device: optimizer step --- */
 /* The Adam step of the training loop (run.py:446 `torch.optim.Adam(model.parameters(), lr)`, run.py:250 `optimizer.step()`) over
