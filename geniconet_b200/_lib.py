@@ -82,6 +82,15 @@ _SIGS = {
     'gin_bn_act_bwd': (_i, [_vp, _i64, _vp, _vp, _i64, _i, _vp, _vp, _vp, _i64, _vp, _i64, _vp, _i, _i, _i, _i, _vp]),
     'gin_bn_pair_ws_bytes': (_sz, [_i]),
     'gin_bn_act_bwd_pair': (_i, [_vp, _i64, _vp, _vp, _i64, _vp, _vp, _vp, _i64, _vp, _i64, _vp, _vp, _vp, _i64, _i, _vp, _i, _i, _i, _i, _vp]),
+    'gin_bn_sync_record_bytes': (_sz, [_i, _i]),
+    'gin_bn_sync_stats_total': (_i, [_vp, _i64, _i64, _i, _vp, _vp, _vp]),
+    'gin_bn_sync_stats_total_from_parts': (_i, [_vp, _i, _i64, _i64, _i, _i, _i, _vp, _vp]),
+    'gin_bn_sync_stats_final': (_i, [_vp, _i, _i, _vp, _vp, _f, _f, _vp, _vp, _vp, _vp, _vp, _vp, _f, _f, _vp, _vp, _vp, _vp, _vp]),
+    'gin_bn_sync_bwd_reduce': (_i, [_vp, _i64, _vp, _vp, _i64, _i, _vp, _vp, _vp, _i, _i, _i, _i, _vp]),
+    'gin_bn_sync_bwd_reduce_pair': (_i, [_vp, _i64, _vp, _vp, _i64, _vp, _vp, _i64, _vp, _i, _vp, _vp, _i, _i, _i, _i, _vp]),
+    'gin_bn_sync_bwd_final': (_i, [_vp, _i, _i, _i, _vp, _vp, _vp]),
+    'gin_bn_bwd_apply': (_i, [_vp, _i64, _vp, _vp, _i64, _i, _vp, _vp, _vp, _i64, _vp, _i64, _i, _i, _i, _i, _vp]),
+    'gin_bn_bwd_apply_pair': (_i, [_vp, _i64, _vp, _vp, _i64, _vp, _vp, _vp, _i64, _vp, _i64, _vp, _vp, _vp, _i64, _i, _i, _i, _i, _i, _vp]),
     'gin_bn_eval_bwd_ws_bytes': (_sz, [_i]),
     'gin_bn_eval_bwd': (_i, [_vp, _i64, _vp, _vp, _i64, _i, _vp, _vp, _vp, _i64, _vp, _i64, _vp, _i, _i, _i, _i, _vp]),
     'gin_bn_eval_bwd_pair': (_i, [_vp, _i64, _vp, _vp, _i64, _vp, _vp, _vp, _i64, _vp, _i64, _vp, _vp, _vp, _i64, _i, _vp, _i, _i, _i, _i, _vp]),

@@ -823,29 +823,82 @@ int gin_bn_act_fwd(const void* y1, int64_t ld1, const float* stat1, const void* 
   return check_launch("bn_act_fwd");
 }
 
-int gin_bn_act_bwd(const float* dout, int64_t ldg, const void* mask_b, const void* y, int64_t ld, int y_fp16, const float* stat, float* bstat, void* dy_b,
-                   int64_t ldo, float* dy_f, int64_t ldf, void* ws, int B, int level, int C, int relu_from_y, void* stream) {
-  cudaStream_t st = (cudaStream_t)stream;
-  if (!dout || !y || !stat || !bstat || !ws || (!dy_b && !dy_f) || B <= 0 || level < 0 || level > 9 || !bn_shape_ok(C))
-    return fail(GIN_ERR_ARG, "gin_bn_act_bwd: bad argument");
+// the apply pass of gin_bn_act_bwd / _pair (and of the synchronised backward) from finished bstat
+static int bn_bwd_apply(const float* dout, int64_t ldg, const void* mask_b, const void* y, int64_t ld, int y_fp16, const float* stat, const float* bstat,
+                        void* dy_b, int64_t ldo, float* dy_f, int64_t ldf, int B, int level, int C, int relu_from_y, cudaStream_t st) {
   const int n = 1 << level, P = 10 << (2 * level);
-  const long long rows = (long long)B * P;
   const gin::bn::Src sy{reinterpret_cast<const float*>(y), (long long)ld, y_fp16 ? 1 : 0};
   const __nv_bfloat16* mask = reinterpret_cast<const __nv_bfloat16*>(mask_b);
-  const int ctas = gin::bn::grid_for_rows(rows * (C >> 3));
+  const int ctas = gin::bn::grid_for_rows((long long)B * P * (C >> 3));
+  const bool smem = gin::bn::smem_consts(C);
+  const int from_y = (relu_from_y && mask && smem) ? 1 : 0;
+  __nv_bfloat16* dyb = reinterpret_cast<__nv_bfloat16*>(dy_b);
+  if (!smem) gin::launch_pdl(gin::bn::bwd_apply_anyc_kernel, dim3(ctas), dim3(256), 0, st, dout, ldg, mask, sy, stat, bstat, dyb, ldo, dy_f, ldf, n, B, P, C);
+  else gin::launch_pdl(y_fp16 ? gin::bn::bwd_apply_kernel<true> : gin::bn::bwd_apply_kernel<false>, dim3(ctas), dim3(256), 0, st, dout, ldg, mask, sy, stat, bstat, dyb, ldo, dy_f, ldf, n, B, P, C, from_y);
+  return check_launch("bn_bwd_apply");
+}
+
+static int bn_bwd_apply_pair(const float* dout, int64_t ldg, const void* mask_b, const void* yA, int64_t ldA, const float* statA, const float* bstatA,
+                             void* dyA_b, int64_t ldoA, const void* yB, int64_t ldB, const float* statB, const float* bstatB, void* dyB_b, int64_t ldoB,
+                             int y_fp16, int B, int level, int C, int relu_from_y, cudaStream_t st) {
+  const int n = 1 << level, P = 10 << (2 * level);
+  const gin::bn::Src sA{reinterpret_cast<const float*>(yA), (long long)ldA, y_fp16 ? 1 : 0}, sB{reinterpret_cast<const float*>(yB), (long long)ldB, y_fp16 ? 1 : 0};
+  const __nv_bfloat16* mask = reinterpret_cast<const __nv_bfloat16*>(mask_b);
+  const int ctas = gin::bn::grid_for_rows((long long)B * P * (C >> 3));
+  const bool smem = gin::bn::smem_consts(C);
+  const int from_y = (relu_from_y && mask && smem) ? 1 : 0;
+  __nv_bfloat16 *da = reinterpret_cast<__nv_bfloat16*>(dyA_b), *db = reinterpret_cast<__nv_bfloat16*>(dyB_b);
+  if (!smem) gin::launch_pdl(gin::bn::bwd_apply2_anyc_kernel, dim3(ctas), dim3(256), 0, st, dout, ldg, mask, sA, statA, bstatA, sB, statB, bstatB, da, ldoA, db, ldoB, n, B, P, C);
+  else gin::launch_pdl(y_fp16 ? gin::bn::bwd_apply2_kernel<true> : gin::bn::bwd_apply2_kernel<false>, dim3(ctas), dim3(256), 0, st, dout, ldg, mask, sA, statA, bstatA, sB, statB, bstatB, da, ldoA, db, ldoB, n, B, P, C, from_y);
+  return check_launch("bn_bwd_apply2");
+}
+
+// the reduce pass of gin_bn_act_bwd / _pair: per-CTA partials in ws; returns their count in *nparts
+static int bn_bwd_reduce(const float* dout, int64_t ldg, const void* mask_b, const void* y, int64_t ld, int y_fp16, const float* stat, void* ws,
+                         long long rows, int C, int relu_from_y, cudaStream_t st, int* nparts) {
+  const gin::bn::Src sy{reinterpret_cast<const float*>(y), (long long)ld, y_fp16 ? 1 : 0};
+  const __nv_bfloat16* mask = reinterpret_cast<const __nv_bfloat16*>(mask_b);
+  const int ctas = *nparts = gin::bn::grid_for_rows(rows * (C >> 3));
   const bool smem = gin::bn::smem_consts(C);
   const int from_y = (relu_from_y && mask && smem) ? 1 : 0;      // the register-constant kernels always read the mask
   float* part = reinterpret_cast<float*>(ws);
   if (!smem) gin::launch_pdl(gin::bn::bwd_reduce_kernel, dim3(ctas), dim3(256), 0, st, dout, ldg, mask, sy, stat, rows, C, part);
   else gin::launch_pdl(y_fp16 ? gin::bn::bwd_reduce_s_kernel<true> : gin::bn::bwd_reduce_s_kernel<false>, dim3(ctas), dim3(256), 0, st, dout, ldg, mask, sy, stat, rows, C, part, from_y);
-  int rc = check_launch("bn_bwd_reduce");
+  return check_launch("bn_bwd_reduce");
+}
+
+static int bn_bwd_reduce_pair(const float* dout, int64_t ldg, const void* mask_b, const void* yA, int64_t ldA, const float* statA, const void* yB,
+                              int64_t ldB, const float* statB, int y_fp16, void* ws, long long rows, int C, int relu_from_y, cudaStream_t st, int* nparts) {
+  const gin::bn::Src sA{reinterpret_cast<const float*>(yA), (long long)ldA, y_fp16 ? 1 : 0}, sB{reinterpret_cast<const float*>(yB), (long long)ldB, y_fp16 ? 1 : 0};
+  const __nv_bfloat16* mask = reinterpret_cast<const __nv_bfloat16*>(mask_b);
+  const int ctas = *nparts = gin::bn::grid_for_rows(rows * (C >> 3));
+  const bool smem = gin::bn::smem_consts(C);
+  const int from_y = (relu_from_y && mask && smem) ? 1 : 0;
+  float* part = reinterpret_cast<float*>(ws);
+  if (!smem) gin::launch_pdl(gin::bn::bwd_reduce2_anyc_kernel, dim3(ctas), dim3(256), 0, st, dout, ldg, mask, sA, statA, sB, statB, rows, C, part);
+  else gin::launch_pdl(y_fp16 ? gin::bn::bwd_reduce2_kernel<true> : gin::bn::bwd_reduce2_kernel<false>, dim3(ctas), dim3(256), 0, st, dout, ldg, mask, sA, statA, sB, statB, rows, C, part, from_y);
+  return check_launch("bn_bwd_reduce2");
+}
+
+static bool bn_bwd_args_ok(const float* dout, const void* y, const float* stat, const void* dy_b, const float* dy_f, int B, int level, int C) {
+  return dout && y && stat && (dy_b || dy_f) && B > 0 && level >= 0 && level <= 9 && bn_shape_ok(C);
+}
+
+static bool bn_bwd_pair_args_ok(const float* dout, const void* yA, const float* statA, const void* dyA_b, const void* yB, const float* statB,
+                                const void* dyB_b, int B, int level, int C) {
+  return dout && yA && yB && statA && statB && dyA_b && dyB_b && B > 0 && level >= 0 && level <= 9 && bn_shape_ok(C);
+}
+
+int gin_bn_act_bwd(const float* dout, int64_t ldg, const void* mask_b, const void* y, int64_t ld, int y_fp16, const float* stat, float* bstat, void* dy_b,
+                   int64_t ldo, float* dy_f, int64_t ldf, void* ws, int B, int level, int C, int relu_from_y, void* stream) {
+  cudaStream_t st = (cudaStream_t)stream;
+  if (!bstat || !ws || !bn_bwd_args_ok(dout, y, stat, dy_b, dy_f, B, level, C)) return fail(GIN_ERR_ARG, "gin_bn_act_bwd: bad argument");
+  const long long rows = (long long)B * (10 << (2 * level));
+  int ctas, rc = bn_bwd_reduce(dout, ldg, mask_b, y, ld, y_fp16, stat, ws, rows, C, relu_from_y, st, &ctas);
   if (rc) return rc;
   gin::launch_pdl(gin::bn::bwd_final_kernel, dim3(C / 8), dim3(256), 0, st, reinterpret_cast<const float*>(ws), ctas, rows, C, bstat);
   if ((rc = check_launch("bn_bwd_final"))) return rc;
-  __nv_bfloat16* dyb = reinterpret_cast<__nv_bfloat16*>(dy_b);
-  if (!smem) gin::launch_pdl(gin::bn::bwd_apply_anyc_kernel, dim3(ctas), dim3(256), 0, st, dout, ldg, mask, sy, stat, bstat, dyb, ldo, dy_f, ldf, n, B, P, C);
-  else gin::launch_pdl(y_fp16 ? gin::bn::bwd_apply_kernel<true> : gin::bn::bwd_apply_kernel<false>, dim3(ctas), dim3(256), 0, st, dout, ldg, mask, sy, stat, bstat, dyb, ldo, dy_f, ldf, n, B, P, C, from_y);
-  return check_launch("bn_bwd_apply");
+  return bn_bwd_apply(dout, ldg, mask_b, y, ld, y_fp16, stat, bstat, dy_b, ldo, dy_f, ldf, B, level, C, relu_from_y, st);
 }
 
 size_t gin_bn_pair_ws_bytes(int C) { return C <= 0 ? 0 : (size_t)gin::bn::MAX_CTAS * 4 * C * 4; }
@@ -854,26 +907,93 @@ int gin_bn_act_bwd_pair(const float* dout, int64_t ldg, const void* mask_b, cons
                         void* dyA_b, int64_t ldoA, const void* yB, int64_t ldB, const float* statB, float* bstatB, void* dyB_b, int64_t ldoB,
                         int y_fp16, void* ws, int B, int level, int C, int relu_from_y, void* stream) {
   cudaStream_t st = (cudaStream_t)stream;
-  if (!dout || !yA || !yB || !statA || !statB || !bstatA || !bstatB || !dyA_b || !dyB_b || !ws || B <= 0 || level < 0 || level > 9 || !bn_shape_ok(C))
+  if (!bstatA || !bstatB || !ws || !bn_bwd_pair_args_ok(dout, yA, statA, dyA_b, yB, statB, dyB_b, B, level, C))
     return fail(GIN_ERR_ARG, "gin_bn_act_bwd_pair: bad argument");
-  const int n = 1 << level, P = 10 << (2 * level);
-  const long long rows = (long long)B * P;
-  const gin::bn::Src sA{reinterpret_cast<const float*>(yA), (long long)ldA, y_fp16 ? 1 : 0}, sB{reinterpret_cast<const float*>(yB), (long long)ldB, y_fp16 ? 1 : 0};
-  const __nv_bfloat16* mask = reinterpret_cast<const __nv_bfloat16*>(mask_b);
-  const int ctas = gin::bn::grid_for_rows(rows * (C >> 3));
-  const bool smem = gin::bn::smem_consts(C);
-  const int from_y = (relu_from_y && mask && smem) ? 1 : 0;
-  float* part = reinterpret_cast<float*>(ws);
-  if (!smem) gin::launch_pdl(gin::bn::bwd_reduce2_anyc_kernel, dim3(ctas), dim3(256), 0, st, dout, ldg, mask, sA, statA, sB, statB, rows, C, part);
-  else gin::launch_pdl(y_fp16 ? gin::bn::bwd_reduce2_kernel<true> : gin::bn::bwd_reduce2_kernel<false>, dim3(ctas), dim3(256), 0, st, dout, ldg, mask, sA, statA, sB, statB, rows, C, part, from_y);
-  int rc = check_launch("bn_bwd_reduce2");
+  const long long rows = (long long)B * (10 << (2 * level));
+  int ctas, rc = bn_bwd_reduce_pair(dout, ldg, mask_b, yA, ldA, statA, yB, ldB, statB, y_fp16, ws, rows, C, relu_from_y, st, &ctas);
   if (rc) return rc;
   gin::launch_pdl(gin::bn::bwd_final2_kernel, dim3(C / 8), dim3(256), 0, st, reinterpret_cast<const float*>(ws), ctas, rows, C, bstatA, bstatB);
   if ((rc = check_launch("bn_bwd_final2"))) return rc;
-  __nv_bfloat16 *da = reinterpret_cast<__nv_bfloat16*>(dyA_b), *db = reinterpret_cast<__nv_bfloat16*>(dyB_b);
-  if (!smem) gin::launch_pdl(gin::bn::bwd_apply2_anyc_kernel, dim3(ctas), dim3(256), 0, st, dout, ldg, mask, sA, statA, bstatA, sB, statB, bstatB, da, ldoA, db, ldoB, n, B, P, C);
-  else gin::launch_pdl(y_fp16 ? gin::bn::bwd_apply2_kernel<true> : gin::bn::bwd_apply2_kernel<false>, dim3(ctas), dim3(256), 0, st, dout, ldg, mask, sA, statA, bstatA, sB, statB, bstatB, da, ldoA, db, ldoB, n, B, P, C, from_y);
-  return check_launch("bn_bwd_apply2");
+  return bn_bwd_apply_pair(dout, ldg, mask_b, yA, ldA, statA, bstatA, dyA_b, ldoA, yB, ldB, statB, bstatB, dyB_b, ldoB, y_fp16, B, level, C, relu_from_y, st);
+}
+
+// ------------------------------------------------------------------ synchronised BatchNorm (records all-gathered by the caller)
+size_t gin_bn_sync_record_bytes(int C, int pair) { return C <= 0 ? 0 : (size_t)8 * (pair ? 2 : 1) * (2 * (size_t)C + 1); }
+
+int gin_bn_sync_stats_total(const float* y, int64_t ld, int64_t rows, int C, double* rec, void* ws, void* stream) {
+  cudaStream_t st = (cudaStream_t)stream;
+  if (!y || !rec || !ws || rows <= 0 || !bn_shape_ok(C) || ld < C || (ld & 3)) return fail(GIN_ERR_ARG, "gin_bn_sync_stats_total: bad argument (C/8 must divide 256)");
+  const int ctas = gin::bn::grid_for_rows(rows * (C >> 3));
+  gin::launch_pdl(gin::bn::stats_kernel, dim3(ctas), dim3(256), 0, st, gin::bn::Src{y, (long long)ld, 0}, rows, C, reinterpret_cast<float*>(ws));
+  int rc = check_launch("bn_stats");
+  if (rc) return rc;
+  gin::launch_pdl(gin::bn::stats_total_kernel, dim3(C / 8), dim3(256), 0, st, reinterpret_cast<const float*>(ws), (const float*)nullptr, ctas, (long long)rows, C,
+                  (long long)C, rec);
+  return check_launch("bn_stats_total");
+}
+
+int gin_bn_sync_stats_total_from_parts(const float* parts, int nparts, int64_t ld, int64_t rows, int C, int colA, int colB, double* rec, void* stream) {
+  if (!parts || nparts <= 0 || nparts > gin::bn::MAX_CTAS || !rec || rows <= 0 || !bn_shape_ok(C) || colA < 0 || colB < -1 ||
+      ld < C + (colA > colB ? colA : colB))
+    return fail(GIN_ERR_ARG, "gin_bn_sync_stats_total_from_parts: bad argument");
+  const int nbn = colB >= 0 ? 2 : 1;
+  gin::launch_pdl(gin::bn::stats_total_kernel, dim3(nbn * (C / 8)), dim3(256), 0, (cudaStream_t)stream, parts + colA, colB >= 0 ? parts + colB : nullptr,
+                  nparts, (long long)rows, C, (long long)ld, rec);
+  return check_launch("bn_stats_total");
+}
+
+int gin_bn_sync_stats_final(const double* recs, int world, int C, const float* gammaA, const float* betaA, float epsA, float momentumA, float* rmeanA,
+                            float* rvarA, int64_t* nbtA, float* statA, const float* gammaB, const float* betaB, float epsB, float momentumB, float* rmeanB,
+                            float* rvarB, int64_t* nbtB, float* statB, void* stream) {
+  if (!recs || world <= 0 || !statA || !bn_shape_ok(C)) return fail(GIN_ERR_ARG, "gin_bn_sync_stats_final: bad argument");
+  const int nbn = statB ? 2 : 1;
+  gin::bn::StatsTarget a{nullptr, gammaA, betaA, rmeanA, rvarA, reinterpret_cast<long long*>(nbtA), statA, epsA, momentumA};
+  gin::bn::StatsTarget b{nullptr, gammaB, betaB, rmeanB, rvarB, reinterpret_cast<long long*>(nbtB), statB, epsB, momentumB};
+  gin::launch_pdl(gin::bn::stats_sync_final_kernel, dim3(nbn * (C / 8)), dim3(256), 0, (cudaStream_t)stream, recs, world, nbn, C, a, b);
+  return check_launch("bn_stats_sync_final");
+}
+
+int gin_bn_sync_bwd_reduce(const float* dout, int64_t ldg, const void* mask_b, const void* y, int64_t ld, int y_fp16, const float* stat, double* rec,
+                           void* ws, int B, int level, int C, int relu_from_y, void* stream) {
+  cudaStream_t st = (cudaStream_t)stream;
+  if (!rec || !ws || !bn_bwd_args_ok(dout, y, stat, rec, nullptr, B, level, C)) return fail(GIN_ERR_ARG, "gin_bn_sync_bwd_reduce: bad argument");
+  const long long rows = (long long)B * (10 << (2 * level));
+  int ctas, rc = bn_bwd_reduce(dout, ldg, mask_b, y, ld, y_fp16, stat, ws, rows, C, relu_from_y, st, &ctas);
+  if (rc) return rc;
+  gin::launch_pdl(gin::bn::bwd_total_kernel, dim3(C / 8), dim3(256), 0, st, reinterpret_cast<const float*>(ws), ctas, 1, rows, C, rec);
+  return check_launch("bn_bwd_total");
+}
+
+int gin_bn_sync_bwd_reduce_pair(const float* dout, int64_t ldg, const void* mask_b, const void* yA, int64_t ldA, const float* statA, const void* yB,
+                                int64_t ldB, const float* statB, int y_fp16, double* rec, void* ws, int B, int level, int C, int relu_from_y, void* stream) {
+  cudaStream_t st = (cudaStream_t)stream;
+  if (!rec || !ws || !bn_bwd_pair_args_ok(dout, yA, statA, rec, yB, statB, rec, B, level, C)) return fail(GIN_ERR_ARG, "gin_bn_sync_bwd_reduce_pair: bad argument");
+  const long long rows = (long long)B * (10 << (2 * level));
+  int ctas, rc = bn_bwd_reduce_pair(dout, ldg, mask_b, yA, ldA, statA, yB, ldB, statB, y_fp16, ws, rows, C, relu_from_y, st, &ctas);
+  if (rc) return rc;
+  gin::launch_pdl(gin::bn::bwd_total_kernel, dim3(C / 8), dim3(256), 0, st, reinterpret_cast<const float*>(ws), ctas, 2, rows, C, rec);
+  return check_launch("bn_bwd_total");
+}
+
+int gin_bn_sync_bwd_final(const double* recs, int world, int rank, int C, float* bstatA, float* bstatB, void* stream) {
+  if (!recs || world <= 0 || rank < 0 || rank >= world || !bstatA || !bn_shape_ok(C)) return fail(GIN_ERR_ARG, "gin_bn_sync_bwd_final: bad argument");
+  gin::launch_pdl(gin::bn::bwd_sync_final_kernel, dim3(C / 8), dim3(256), 0, (cudaStream_t)stream, recs, world, rank, bstatB ? 2 : 1, C, bstatA, bstatB);
+  return check_launch("bn_bwd_sync_final");
+}
+
+int gin_bn_bwd_apply(const float* dout, int64_t ldg, const void* mask_b, const void* y, int64_t ld, int y_fp16, const float* stat, const float* bstat,
+                     void* dy_b, int64_t ldo, float* dy_f, int64_t ldf, int B, int level, int C, int relu_from_y, void* stream) {
+  if (!bstat || !bn_bwd_args_ok(dout, y, stat, dy_b, dy_f, B, level, C)) return fail(GIN_ERR_ARG, "gin_bn_bwd_apply: bad argument");
+  return bn_bwd_apply(dout, ldg, mask_b, y, ld, y_fp16, stat, bstat, dy_b, ldo, dy_f, ldf, B, level, C, relu_from_y, (cudaStream_t)stream);
+}
+
+int gin_bn_bwd_apply_pair(const float* dout, int64_t ldg, const void* mask_b, const void* yA, int64_t ldA, const float* statA, const float* bstatA,
+                          void* dyA_b, int64_t ldoA, const void* yB, int64_t ldB, const float* statB, const float* bstatB, void* dyB_b, int64_t ldoB,
+                          int y_fp16, int B, int level, int C, int relu_from_y, void* stream) {
+  if (!bstatA || !bstatB || !bn_bwd_pair_args_ok(dout, yA, statA, dyA_b, yB, statB, dyB_b, B, level, C))
+    return fail(GIN_ERR_ARG, "gin_bn_bwd_apply_pair: bad argument");
+  return bn_bwd_apply_pair(dout, ldg, mask_b, yA, ldA, statA, bstatA, dyA_b, ldoA, yB, ldB, statB, bstatB, dyB_b, ldoB, y_fp16, B, level, C, relu_from_y,
+                           (cudaStream_t)stream);
 }
 
 // ------------------------------------------------------------------ eval-mode BatchNorm backward (frozen statistics)

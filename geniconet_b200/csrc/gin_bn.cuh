@@ -149,37 +149,8 @@ __global__ void __launch_bounds__(256) stats_kernel(Src y, long long rows, int C
   block_partials(s0, s1, C, partial);
 }
 
-// stat[0..3][C] = mean, invstd, scale = gamma*invstd, shift = beta - mean*scale; running statistics updated as torch does
-// (momentum, unbiased variance).  grid = C/8, block = 256.
-__global__ void __launch_bounds__(256)
-stats_final_kernel(const float* __restrict__ partial, int nblocks, long long rows, int C, const float* __restrict__ gamma,
-                   const float* __restrict__ beta, float eps, float momentum, float* __restrict__ running_mean, float* __restrict__ running_var,
-                   long long* __restrict__ num_batches_tracked, float* __restrict__ stat, long long ld) {
-  GIN_PDL_SYNC();
-  __shared__ double sums[16];
-  const double t = final_sum(partial, nblocks, C, ld);
-  if (threadIdx.x < 16) sums[threadIdx.x] = t;
-  __syncthreads();
-  const int c = blockIdx.x * 8 + threadIdx.x;
-  if (num_batches_tracked && blockIdx.x == 0 && threadIdx.x == 0) *num_batches_tracked += 1;
-  if (threadIdx.x < 8 && c < C) {
-    const double mean = sums[threadIdx.x] / (double)rows;
-    double var = sums[8 + threadIdx.x] / (double)rows - mean * mean;
-    if (var < 0.0) var = 0.0;
-    const float invstd = (float)(1.0 / sqrt(var + (double)eps));
-    const float g = gamma ? gamma[c] : 1.f, b = beta ? beta[c] : 0.f;
-    const float scale = g * invstd;
-    stat[c] = (float)mean; stat[C + c] = invstd; stat[2 * C + c] = scale; stat[3 * C + c] = b - (float)mean * scale;
-    if (running_mean) {
-      const double unbiased = rows > 1 ? var * (double)rows / (double)(rows - 1) : var;
-      running_mean[c] = (1.f - momentum) * running_mean[c] + momentum * (float)mean;
-      running_var[c] = (1.f - momentum) * running_var[c] + momentum * (float)unbiased;
-    }
-  }
-}
-
-// Two BatchNorms whose statistics come from column slices of the SAME partial-sum rows (the two sibling convolutions of a residual
-// block run as one GEMM): one launch, blockIdx.x < C/8 -> the first, else the second.
+// One BatchNorm whose statistics a final kernel writes.  The pair kernels take two: the sibling convolutions of a residual block
+// run as one GEMM, so their partial sums are column slices of the same rows.
 struct StatsTarget {
   const float* partial;      // first column of this BatchNorm inside the partial-sum rows
   const float* gamma;
@@ -190,18 +161,11 @@ struct StatsTarget {
   float* stat;
   float eps, momentum;
 };
-__global__ void __launch_bounds__(256)
-stats_final2_kernel(StatsTarget a, StatsTarget b, int nblocks, long long rows, int C, long long ld) {
-  GIN_PDL_SYNC();
-  __shared__ double sums[16];
-  const int nb = C / 8;
-  const bool second = (int)blockIdx.x >= nb;
-  const StatsTarget& t = second ? b : a;
-  const int blk = second ? blockIdx.x - nb : blockIdx.x;
-  // final_sum indexes channels by blockIdx.x: shift the base pointer instead
-  const double s = final_sum(t.partial - (second ? (size_t)nb * 8 : 0), nblocks, C + (second ? nb * 8 : 0), ld);
-  if (threadIdx.x < 16) sums[threadIdx.x] = s;
-  __syncthreads();
+
+// sums[0..7] = sum y, sums[8..15] = sum y^2 of the 8 channels of block blk (shared memory, written before a __syncthreads) ->
+// stat[0..3][C] = mean, invstd, scale = gamma*invstd, shift = beta - mean*scale; running statistics updated as torch does
+// (momentum, unbiased variance over `rows`).
+GIN_DEVINL void stats_write(const double* sums, int blk, long long rows, int C, const StatsTarget& t) {
   const int c = blk * 8 + threadIdx.x;
   if (t.num_batches_tracked && blk == 0 && threadIdx.x == 0) *t.num_batches_tracked += 1;
   if (threadIdx.x < 8 && c < C) {
@@ -218,6 +182,78 @@ stats_final2_kernel(StatsTarget a, StatsTarget b, int nblocks, long long rows, i
       t.running_var[c] = (1.f - t.momentum) * t.running_var[c] + t.momentum * (float)unbiased;
     }
   }
+}
+
+// stats_write from per-CTA partials.  grid = C/8, block = 256.
+__global__ void __launch_bounds__(256)
+stats_final_kernel(const float* __restrict__ partial, int nblocks, long long rows, int C, const float* __restrict__ gamma,
+                   const float* __restrict__ beta, float eps, float momentum, float* __restrict__ running_mean, float* __restrict__ running_var,
+                   long long* __restrict__ num_batches_tracked, float* __restrict__ stat, long long ld) {
+  GIN_PDL_SYNC();
+  __shared__ double sums[16];
+  const double t = final_sum(partial, nblocks, C, ld);
+  if (threadIdx.x < 16) sums[threadIdx.x] = t;
+  __syncthreads();
+  stats_write(sums, blockIdx.x, rows, C, StatsTarget{partial, gamma, beta, running_mean, running_var, num_batches_tracked, stat, eps, momentum});
+}
+
+// Two BatchNorms from column slices of the SAME partial-sum rows in one launch: blockIdx.x < C/8 -> the first, else the second.
+__global__ void __launch_bounds__(256)
+stats_final2_kernel(StatsTarget a, StatsTarget b, int nblocks, long long rows, int C, long long ld) {
+  GIN_PDL_SYNC();
+  __shared__ double sums[16];
+  const int nb = C / 8;
+  const bool second = (int)blockIdx.x >= nb;
+  const StatsTarget& t = second ? b : a;
+  const int blk = second ? blockIdx.x - nb : blockIdx.x;
+  // final_sum indexes channels by blockIdx.x: shift the base pointer instead
+  const double s = final_sum(t.partial - (second ? (size_t)nb * 8 : 0), nblocks, C + (second ? nb * 8 : 0), ld);
+  if (threadIdx.x < 16) sums[threadIdx.x] = s;
+  __syncthreads();
+  stats_write(sums, blk, rows, C, t);
+}
+
+// ------------------------------------------------------------------------------------------------ synchronised BatchNorm
+// A BatchNorm synchronised over W ranks splits each final above in two: this rank's fp64 totals go into a record, the records of
+// every rank are all-gathered (a copy), and a final kernel sums them in rank order 0..W-1.  Every rank therefore computes the
+// same bits, and with W = 1 the sum is the rank's own total: bit for bit the unsynchronised final.
+//   forward record of one BatchNorm: [sum y [C] | sum y^2 [C] | rows], 2C + 1 doubles; of a sibling pair: A's record, then B's
+//   backward record of one BatchNorm: [sum g [C] | sum g*yhat [C] | rows]; of a pair: A's record, then B's (sum g is the same in both)
+GIN_DEVINL double rank_sum(const double* __restrict__ recs, int world, long long stride, long long off) {
+  double s = recs[off];
+  for (int w = 1; w < world; ++w) s += recs[(long long)w * stride + off];
+  return s;
+}
+
+// forward records from per-CTA partials (final_sum's order); grid = nbn * C/8 (nbn = 1, or 2 for a pair: partB, the second record)
+__global__ void __launch_bounds__(256)
+stats_total_kernel(const float* __restrict__ partA, const float* __restrict__ partB, int nblocks, long long rows, int C, long long ld,
+                   double* __restrict__ rec) {
+  GIN_PDL_SYNC();
+  const int nb = C / 8;
+  const bool second = (int)blockIdx.x >= nb;
+  const int blk = second ? blockIdx.x - nb : blockIdx.x;
+  const double s = second ? final_sum(partB - (size_t)nb * 8, nblocks, C + nb * 8, ld) : final_sum(partA, nblocks, C, ld);
+  double* r = rec + (second ? 2LL * C + 1 : 0);
+  const int k = threadIdx.x >> 3, c = blk * 8 + (threadIdx.x & 7);
+  if (threadIdx.x < 16 && c < C) r[(long long)k * C + c] = s;
+  if (blk == 0 && threadIdx.x == 0) r[2LL * C] = (double)rows;
+}
+
+// stats_write from the gathered forward records recs[world][nbn * (2C + 1)] with the global row count; grid = nbn * C/8
+__global__ void __launch_bounds__(256) stats_sync_final_kernel(const double* __restrict__ recs, int world, int nbn, int C, StatsTarget a, StatsTarget b) {
+  GIN_PDL_SYNC();
+  __shared__ double sums[16];
+  __shared__ long long rows;
+  const int nb = C / 8;
+  const bool second = (int)blockIdx.x >= nb;
+  const int blk = second ? blockIdx.x - nb : blockIdx.x;
+  const long long stride = (long long)nbn * (2 * C + 1), base = second ? 2LL * C + 1 : 0;
+  const int k = threadIdx.x >> 3, c = blk * 8 + (threadIdx.x & 7);
+  if (threadIdx.x < 16) sums[threadIdx.x] = c < C ? rank_sum(recs, world, stride, base + (long long)k * C + c) : 0.0;
+  if (threadIdx.x == 16) rows = (long long)rank_sum(recs, world, stride, base + 2LL * C);
+  __syncthreads();
+  stats_write(sums, blk, rows, C, second ? b : a);
 }
 
 // ------------------------------------------------------------------------------------------------ forward apply
@@ -479,10 +515,8 @@ bwd_reduce2_anyc_kernel(const float* __restrict__ dout, long long ldg, const __n
   }
 }
 
-// bstatA / bstatB [4][C] from partial[nblocks][4][C]; grid = C/8, block = 256 (8 row groups x 32 (sum, channel) lanes)
-__global__ void __launch_bounds__(256)
-bwd_final2_kernel(const float* __restrict__ partial, int nblocks, long long rows, int C, float* __restrict__ bstatA, float* __restrict__ bstatB) {
-  GIN_PDL_SYNC();
+// final[k][c] (double) = sum_b partial[b][k][c] (k = 0..3) for the 8 channels of this CTA; returned to threads 0..31 (k = tid >> 3)
+GIN_DEVINL double final_sum4(const float* __restrict__ partial, int nblocks, int C) {
   __shared__ double red[8][33];
   const int j = threadIdx.x & 31, rg = threadIdx.x >> 5;
   const int k = j >> 3, c = blockIdx.x * 8 + (j & 7);
@@ -499,15 +533,52 @@ bwd_final2_kernel(const float* __restrict__ partial, int nblocks, long long rows
   }
   red[rg][j] = acc;
   __syncthreads();
-  if (threadIdx.x < 32 && c < C) {
-    double t = 0.0;
+  double t = 0.0;
+  if (threadIdx.x < 32)
 #pragma unroll
     for (int r = 0; r < 8; ++r) t += red[r][threadIdx.x];
+  return t;
+}
+
+// bstatA / bstatB [4][C] from partial[nblocks][4][C]; grid = C/8, block = 256 (8 row groups x 32 (sum, channel) lanes)
+__global__ void __launch_bounds__(256)
+bwd_final2_kernel(const float* __restrict__ partial, int nblocks, long long rows, int C, float* __restrict__ bstatA, float* __restrict__ bstatB) {
+  GIN_PDL_SYNC();
+  const double t = final_sum4(partial, nblocks, C);
+  const int k = (threadIdx.x & 31) >> 3, c = blockIdx.x * 8 + (threadIdx.x & 7);
+  if (threadIdx.x < 32 && c < C) {
     float* bs = k < 2 ? bstatA : bstatB;
     const int kk = k & 1;
     bs[kk * C + c] = (float)t;
     bs[(2 + kk) * C + c] = (float)(t / (double)rows);
   }
+}
+
+// backward records (layout: see stats_total_kernel) from the partials of bwd_reduce(_s)_kernel (nbn = 1, bwd_final_kernel's order)
+// or of bwd_reduce2(_anyc)_kernel (nbn = 2, bwd_final2_kernel's order).  grid = C/8.
+__global__ void __launch_bounds__(256)
+bwd_total_kernel(const float* __restrict__ partial, int nblocks, int nbn, long long rows, int C, double* __restrict__ rec) {
+  GIN_PDL_SYNC();
+  const double t = nbn == 1 ? final_sum(partial, nblocks, C) : final_sum4(partial, nblocks, C);
+  const int k = threadIdx.x >> 3, c = blockIdx.x * 8 + (threadIdx.x & 7);
+  const long long len = 2LL * C + 1;
+  if (threadIdx.x < 16 * nbn && c < C) rec[(k >> 1) * len + (k & 1) * C + c] = t;
+  if (blockIdx.x == 0 && threadIdx.x < nbn) rec[threadIdx.x * len + 2 * C] = (double)rows;
+}
+
+// bstatA (and bstatB of a pair, nbn = 2) from the gathered backward records recs[world][nbn * (2C + 1)]: dbeta, dgamma = the sums of
+// rank `rank`, mean(g), mean(g*yhat) = the sums over every rank / the global row count.  grid = C/8.
+__global__ void __launch_bounds__(256)
+bwd_sync_final_kernel(const double* __restrict__ recs, int world, int rank, int nbn, int C, float* __restrict__ bstatA, float* __restrict__ bstatB) {
+  GIN_PDL_SYNC();
+  const int k = threadIdx.x >> 3, c = blockIdx.x * 8 + (threadIdx.x & 7);
+  if (threadIdx.x >= 16 * nbn || c >= C) return;
+  const long long len = 2LL * C + 1, stride = nbn * len, base = (k >> 1) * len, off = base + (k & 1) * C + c;
+  const double t = recs[rank * stride + off], s = rank_sum(recs, world, stride, off), rows = rank_sum(recs, world, stride, base + 2 * C);
+  float* bs = k < 2 ? bstatA : bstatB;
+  const int kk = k & 1;
+  bs[kk * C + c] = (float)t;
+  bs[(2 + kk) * C + c] = (float)(s / rows);
 }
 
 // dyA, dyB as bf16 gradient copies (row strides ldoA / ldoB, pole-mean rows included)

@@ -23,6 +23,9 @@ the training chain's forward kernels with the running statistics, nothing update
 BatchNorm (gin_bn_eval_bwd / _pair) that computes weight gradients only for weights that need them.
 In train mode a conv bias that feeds a BatchNorm has a mathematically zero gradient and the training chain returns exactly zero
 for it; in eval mode its gradient is scale * sum(g), which the frozen chain returns.
+A chain of SyncBatchNorm (torch.nn.SyncBatchNorm.convert_sync_batchnorm) runs the same chains; in training, when torch would
+synchronise, every BatchNorm reduction all-gathers one fp64 record per rank and sums the records in rank order (sync_group,
+_exchange; DESIGN "Synchronised BatchNorm").
 """
 import torch
 
@@ -40,11 +43,17 @@ def _is_block(m):
     return hasattr(m, 'conv00') and hasattr(m, 'icobn10')
 
 
+# The BatchNorms a chain runs.  A SyncBatchNorm in eval mode is a plain BatchNorm; in train mode the training chain synchronises
+# its statistics over its process group (sync_group).
+_BN = (torch.nn.BatchNorm2d, torch.nn.SyncBatchNorm)
+
+
 def chain_supported(mods):
-    """True when `mods` is [IcoConvS2S(3->C), BatchNorm2d, ReLU]? + residual blocks with tensor-core channel widths."""
+    """True when `mods` is [IcoConvS2S(3->C), BatchNorm, ReLU]? + residual blocks with tensor-core channel widths, and its BatchNorms
+    are all BatchNorm2d or all SyncBatchNorm on one process group."""
     mods = list(mods)
     i = 0
-    if len(mods) >= 3 and isinstance(mods[0], IcoConvS2S) and isinstance(mods[1], torch.nn.BatchNorm2d) and isinstance(mods[2], torch.nn.ReLU):
+    if len(mods) >= 3 and isinstance(mods[0], IcoConvS2S) and isinstance(mods[1], _BN) and isinstance(mods[2], torch.nn.ReLU):
         if mods[0].in_features != 3 or mods[0].stride != 1 or mods[0].out_features % 64 or mods[0].bias is None:
             return False
         i = 3
@@ -59,9 +68,24 @@ def chain_supported(mods):
             if c.in_features % 64 or c.out_features % 64 or c.bias is None or 256 % (c.out_features // 8):
                 return False
         for b in (m.icobn00, m.icobn01, m.icobn10):
-            if not isinstance(b, torch.nn.BatchNorm2d) or not b.affine or not b.track_running_stats or b.momentum is None:
+            if not isinstance(b, _BN) or not b.affine or not b.track_running_stats or b.momentum is None:
                 return False
-    return True
+    bns = [bn for bn, _ in eval_pairs(mods)]
+    return len({isinstance(bn, torch.nn.SyncBatchNorm) for bn in bns}) == 1 and len({id(getattr(bn, 'process_group', None)) for bn in bns}) == 1
+
+
+def sync_group(mods):
+    """(process group, world size, rank in it) over which the training chain `mods` (see chain_supported) synchronises its BatchNorm
+    statistics, or None when it does not: BatchNorm2d, or SyncBatchNorm that torch would not synchronise either (torch.distributed
+    not initialised, or a group of one rank)."""
+    bn = mods[1] if isinstance(mods[0], IcoConvS2S) else mods[0].icobn00
+    if not isinstance(bn, torch.nn.SyncBatchNorm):
+        return None
+    import torch.distributed as dist
+    if not (dist.is_available() and dist.is_initialized()):
+        return None
+    world = dist.get_world_size(bn.process_group)
+    return (bn.process_group, world, dist.get_rank(bn.process_group)) if world > 1 else None
 
 
 def chain_params(mods):
@@ -69,7 +93,7 @@ def chain_params(mods):
     for m in mods:
         if isinstance(m, IcoConvS2S):
             out += [m.weight, m.bias]
-        elif isinstance(m, torch.nn.BatchNorm2d):
+        elif isinstance(m, _BN):
             out += [m.weight, m.bias]
         elif _is_block(m):
             for c, b in ((m.conv00, m.icobn00), (m.conv01, m.icobn01), (m.conv10, m.icobn10)):
@@ -184,8 +208,46 @@ def _dest(params, shape):
     return t.view(shape) if t is not None and t.numel() == int(torch.Size(shape).numel()) else None
 
 
-def _bn_stats(y, col0, ld, rows, C, bn, parts=None):
+def _exchange(rec, sync):
+    """All-gather of this rank's fp64 record over sync = (process group, world, rank): [world][record], in rank order.  Every rank
+    issues the chain's exchanges in the same order."""
+    out = torch.empty(sync[1] * rec.numel(), dtype=torch.float64, device=rec.device)      # flat: gloo takes no other shape
+    torch.distributed.all_gather_into_tensor(out, rec, group=sync[0])
+    return out
+
+
+def _bn_ptrs(bn, stat):
+    """gin_bn_sync_stats_final's arguments of one BatchNorm; (None, ...) for the absent second one"""
+    if bn is None:
+        return [None, None, 0.0, 0.0, None, None, None, None]
+    return [bn.weight.data_ptr(), bn.bias.data_ptr(), float(bn.eps), float(bn.momentum), bn.running_mean.data_ptr(), bn.running_var.data_ptr(),
+            bn.num_batches_tracked.data_ptr(), stat.data_ptr()]
+
+
+def _sync_stats(y, cols, ld, rows, C, parts, sync, targets):
+    """Synchronised batch statistics of the BatchNorms `targets` = [(bn, stat)] (one, or a sibling pair) whose inputs are columns
+    `cols` of y: this rank's record (from the epilogue partials, else from the fp32 map), one exchange, the final over every rank."""
+    dev = y.device
+    rec = _empty(L.gin_bn_sync_record_bytes(C, len(targets) - 1) // 8, torch.float64, dev)
+    if parts is not None:
+        _lib.check(L.gin_bn_sync_stats_total_from_parts(parts[0].data_ptr(), parts[1], ld, rows, C, cols[0], cols[1] if len(cols) > 1 else -1,
+                                                        rec.data_ptr(), _stream()), 'gin_bn_sync_stats_total_from_parts')
+    else:
+        assert y.dtype == torch.float32, 'gin_bn_sync_stats_total reads fp32 maps (fp16 conv outputs always come with epilogue statistics)'
+        ws = _empty(L.gin_bn_ws_bytes(C), torch.uint8, dev)
+        for q, col in enumerate(cols):
+            _lib.check(L.gin_bn_sync_stats_total(y.data_ptr() + 4 * col, ld, rows, C, rec.data_ptr() + 8 * q * (2 * C + 1), ws.data_ptr(), _stream()),
+                       'gin_bn_sync_stats_total')
+    recs = _exchange(rec, sync)
+    (bnA, statA), (bnB, statB) = targets[0], (targets[1] if len(targets) > 1 else (None, None))
+    _lib.check(L.gin_bn_sync_stats_final(recs.data_ptr(), sync[1], C, *_bn_ptrs(bnA, statA), *_bn_ptrs(bnB, statB), _stream()), 'gin_bn_sync_stats_final')
+
+
+def _bn_stats(y, col0, ld, rows, C, bn, parts=None, sync=None):
     stat = _empty(4 * C, torch.float32, y.device)
+    if sync is not None:
+        _sync_stats(y, (col0,), ld, rows, C, parts, sync, [(bn, stat)])
+        return stat
     if parts is not None:         # the conv epilogue already summed y and y^2 per CTA
         pbuf, n = parts
         _lib.check(L.gin_bn_stats_from_parts(pbuf.data_ptr() + 4 * col0, n, ld, rows, C, bn.weight.data_ptr(), bn.bias.data_ptr(), float(bn.eps),
@@ -221,15 +283,27 @@ def _bn_act(y1, col1, ld1, stat1, y2, col2, ld2, stat2, B, level, C, want_b=True
     return out_b, out_f, out_w
 
 
-def _bn_bwd(dout, mask_b, y, col0, ld, stat, B, level, C, dy_b=None, dy_b_col=0, ldo=0, want_f=False, mask_from_y=True):
+def _bn_bwd(dout, mask_b, y, col0, ld, stat, B, level, C, dy_b=None, dy_b_col=0, ldo=0, want_f=False, mask_from_y=True, sync=None):
     """Returns (bstat [4C]: dbeta, dgamma, ..., dy_f or None); writes the bf16 gradient copy into dy_b[:, dy_b_col:dy_b_col+C].
     mask_b must be the activation copy _bn_act produced from (y, stat) with ReLU.  With mask_from_y the kernel re-evaluates the
     mask from y and the BatchNorm constants instead of reading it (include/geniconet_b200.h: relu_from_y): 2 B / element less in
-    each pass, step 3.40 -> 3.27 ms on the same box (profiles/r02_ab_mask_*.json)."""
+    each pass, step 3.40 -> 3.27 ms on the same box (profiles/r02_ab_mask_*.json).  sync: see _walk; dbeta, dgamma are then this
+    rank's sums, the means are over every rank."""
     dev = dout.device
     bstat = _empty(4 * C, torch.float32, dev)
     ws = _empty(L.gin_bn_ws_bytes(C), torch.uint8, dev)
     dy_f = _empty((B * _P(level), C), torch.float32, dev) if want_f else None
+    mask, yp, yf16 = mask_b.data_ptr() if mask_b is not None else None, y.data_ptr() + y.element_size() * col0, 1 if y.dtype == torch.float16 else 0
+    dyb = (dy_b.data_ptr() + 2 * dy_b_col) if dy_b is not None else None
+    if sync is not None:
+        rec = _empty(L.gin_bn_sync_record_bytes(C, 0) // 8, torch.float64, dev)
+        _lib.check(L.gin_bn_sync_bwd_reduce(dout.data_ptr(), C, mask, yp, ld, yf16, stat.data_ptr(), rec.data_ptr(), ws.data_ptr(), B, level, C,
+                                            int(mask_from_y), _stream()), 'gin_bn_sync_bwd_reduce')
+        recs = _exchange(rec, sync)
+        _lib.check(L.gin_bn_sync_bwd_final(recs.data_ptr(), sync[1], sync[2], C, bstat.data_ptr(), None, _stream()), 'gin_bn_sync_bwd_final')
+        _lib.check(L.gin_bn_bwd_apply(dout.data_ptr(), C, mask, yp, ld, yf16, stat.data_ptr(), bstat.data_ptr(), dyb, ldo,
+                                      dy_f.data_ptr() if want_f else None, C, B, level, C, int(mask_from_y), _stream()), 'gin_bn_bwd_apply')
+        return bstat, dy_f
     _lib.check(L.gin_bn_act_bwd(dout.data_ptr(), C, mask_b.data_ptr() if mask_b is not None else None, y.data_ptr() + y.element_size() * col0, ld,
                                 1 if y.dtype == torch.float16 else 0, stat.data_ptr(), bstat.data_ptr(), (dy_b.data_ptr() + 2 * dy_b_col) if dy_b is not None else None, ldo,
                                 dy_f.data_ptr() if want_f else None, C, ws.data_ptr(), B, level, C,
@@ -261,10 +335,13 @@ def _stem_conv(x, conv):
     return plan, packed, xs, (sb, sp, sc), y, None
 
 
-def _block_stats(ycat, pcat, blk, rows, cout):
+def _block_stats(ycat, pcat, blk, rows, cout, sync=None):
     """Batch statistics of icobn00 / icobn10 (running statistics updated) from the sibling GEMM's output [rows][conv00 | conv10]."""
     dev = ycat.device
-    if pcat is not None:                 # both sibling BatchNorms from the same epilogue sums: one launch
+    if sync is not None:
+        stat00, stat10 = _empty(4 * cout, torch.float32, dev), _empty(4 * cout, torch.float32, dev)
+        _sync_stats(ycat, (0, cout), 2 * cout, rows, cout, pcat, sync, [(blk.icobn00, stat00), (blk.icobn10, stat10)])
+    elif pcat is not None:                 # both sibling BatchNorms from the same epilogue sums: one launch
         stat00, stat10 = _empty(4 * cout, torch.float32, dev), _empty(4 * cout, torch.float32, dev)
         bA, bB = blk.icobn00, blk.icobn10
         _lib.check(L.gin_bn_stats_from_parts2(pcat[0].data_ptr(), pcat[1], 2 * cout, rows, cout,
@@ -297,20 +374,21 @@ def _cat(blk):
 
 
 # ------------------------------------------------------------------------------------------------ the chain
-def _block(blk, plan_a, plan_b, a_b, pk_cat, pk01, B, lvl, consts, want_h_w, want_b, want_f, want_w):
+def _block(blk, plan_a, plan_b, a_b, pk_cat, pk01, B, lvl, consts, want_h_w, want_b, want_f, want_w, sync=None):
     """A residual block from the forward operand copy a_b of its input: the sibling GEMM conv00 | conv10, BatchNorm 00 / 10,
     relu(bn00) as conv01's operand, conv01, BatchNorm 01, relu(bn01 + bn10).  Batch statistics (running statistics updated) when
     consts is None, else the eval constants consts[bn].  Returns (out_b, out_f, what a backward needs: fp32 / fp16 conv outputs,
-    BatchNorm constants and the bf16 twins h_w of conv01's operand and out_w of the output, None where not wanted)."""
+    BatchNorm constants and the bf16 twins h_w of conv01's operand and out_w of the output, None where not wanted).  sync: see
+    _walk."""
     cin, cout, rows = blk.conv00.in_features, blk.conv00.out_features, B * _P(lvl)
     ycat, pcat = _conv_fwd(plan_a, a_b, pk_cat, blk.conv00.bias.detach(), B, cin, 2 * cout, _P(lvl), bias1=blk.conv10.bias.detach())   # [rows][conv00 | conv10]
     if consts is None:
-        stat00, stat10 = _block_stats(ycat, pcat, blk, rows, cout)
+        stat00, stat10 = _block_stats(ycat, pcat, blk, rows, cout, sync)
     else:
         stat00, stat10 = consts[blk.icobn00][2], consts[blk.icobn10][2]
     h_b, _, h_w = _bn_act(ycat, 0, 2 * cout, stat00, None, 0, 0, None, B, lvl, cout, want_w=want_h_w)
     y01, p01 = _conv_fwd(plan_b, h_b, pk01, blk.conv01.bias.detach(), B, cout, cout, _P(lvl))
-    stat01 = _bn_stats(y01, 0, cout, rows, cout, blk.icobn01, p01) if consts is None else consts[blk.icobn01][2]
+    stat01 = _bn_stats(y01, 0, cout, rows, cout, blk.icobn01, p01, sync) if consts is None else consts[blk.icobn01][2]
     out_b, out_f, out_w = _bn_act(y01, 0, cout, stat01, ycat, cout, 2 * cout, stat10, B, lvl, cout, want_b=want_b, want_f=want_f, want_w=want_w)
     return out_b, out_f, dict(ycat=ycat, y01=y01, h_w=h_w, out_w=out_w, stat00=stat00, stat01=stat01, stat10=stat10)
 
@@ -327,14 +405,14 @@ def _block_affine(blk, plan_a, plan_b, a_b, pk_cat, pk01, B, lvl, consts, want_b
     return (r[0], r[1]) if r is not None else None
 
 
-def _walk(x, mods, consts, twin, copy, record):
+def _walk(x, mods, consts, twin, copy, record, sync=None):
     """The forward of the chain `mods` (see chain_supported) on x, for the training, forward-only and frozen chains.
 
     consts: None for batch statistics that update the running statistics, else the eval constants of eval_pairs(mods) in that
     order (with record False the blocks then try the affine epilogue first).  twin(weights): whether to make the bf16 twin of an
     activation copy whose wgrad readers are `weights` (none for a block output that no Down block reads).  copy(nxt): whether to
     make the forward operand copy of the activation that the module nxt reads (None: the chain's output).  record: keep, per
-    stage, what a backward needs.  Returns (fp32 output map [B, C, H, W] with channels-last strides, its forward operand copy or
+    stage, what a backward needs.  sync: with consts None, sync_group(mods), whose ranks then share the batch statistics.  Returns (fp32 output map [B, C, H, W] with channels-last strides, its forward operand copy or
     None, the stages)."""
     dev, B = x.device, x.shape[0]
     if consts is not None:
@@ -344,7 +422,7 @@ def _walk(x, mods, consts, twin, copy, record):
         conv, bn = mods[0], mods[1]
         level, C = conv.subdivisions, conv.out_features
         plan, packed, xs, strides, y, parts = _stem_conv(x, conv)
-        stat = _bn_stats(y, 0, C, B * _P(level), C, bn, parts) if consts is None else consts[bn][2]
+        stat = _bn_stats(y, 0, C, B * _P(level), C, bn, parts, sync) if consts is None else consts[bn][2]
         act_b, _, act_w = _bn_act(y, 0, C, stat, None, 0, 0, None, B, level, C, want_b=copy(mods[3]), want_w=twin(_cat(mods[3])))
         if record:
             stages.append(dict(kind='stem', plan=plan, xs=xs, strides=strides, y=y, stat=stat, out_w=act_w, C=C, level=level, packed=packed, k=0))
@@ -396,7 +474,7 @@ def _walk(x, mods, consts, twin, copy, record):
         r = _block_affine(blk, plan_a, plan_b, a_b, pk_cat, pk01, B, lvl, consts, want_b, want_f) if consts is not None and not record else None
         if r is None:
             out_b, out_f, saved = _block(blk, plan_a, plan_b, a_b, pk_cat, pk01, B, lvl, consts, twin((blk.conv01.weight,)), want_b, want_f,
-                                         twin(_cat(nxt) if nxt is not None and nxt._down else ()))
+                                         twin(_cat(nxt) if nxt is not None and nxt._down else ()), sync)
             act_w = saved['out_w']
         else:
             (out_b, out_f), act_w = r, None
@@ -445,13 +523,14 @@ class _Chain(torch.autograd.Function):
     def forward(ctx, x, mods, *params):
         # every twin (the block outputs' are the ReLU masks of backward); the forward copy of every activation but the output, which
         # with bf16 forward operands is its own twin
-        out, _, ctx.stages = _walk(x, mods, None, lambda ws: True, lambda nxt: nxt is not None or not _DUAL, True)
+        ctx.sync = sync_group(mods)
+        out, _, ctx.stages = _walk(x, mods, None, lambda ws: True, lambda nxt: nxt is not None or not _DUAL, True, ctx.sync)
         ctx.mods, ctx.B, ctx.x_needs_grad = mods, x.shape[0], x.requires_grad
         return out
 
     @staticmethod
     def backward(ctx, d_out):
-        B, d, dx = ctx.B, _rows(d_out), None
+        B, d, dx, sync = ctx.B, _rows(d_out), None, ctx.sync
         plist = chain_params(ctx.mods)          # the Parameter objects, in the order of the gradients this function returns
         grads = [None] * len(plist)
         zmax = max([st['cout'] for st in ctx.stages if st['kind'] in ('down', 'up')] + [1])
@@ -469,13 +548,25 @@ class _Chain(torch.autograd.Function):
                 ws = _empty(L.gin_bn_pair_ws_bytes(cout), torch.uint8, dev)
                 ycat = st['ycat']
                 assert st['y01'].dtype == ycat.dtype
-                _lib.check(L.gin_bn_act_bwd_pair(d.data_ptr(), cout, st['out_w'].data_ptr(), st['y01'].data_ptr(), cout, st['stat01'].data_ptr(),
-                                                 bs01.data_ptr(), dy01_b.data_ptr(), cout, ycat.data_ptr() + ycat.element_size() * cout, 2 * cout,
-                                                 st['stat10'].data_ptr(), bs10.data_ptr(), dycat_b.data_ptr() + 2 * cout, 2 * cout,
-                                                 1 if ycat.dtype == torch.float16 else 0, ws.data_ptr(), B, lvl, cout, 1, _stream()), 'gin_bn_act_bwd_pair')
+                yA, statA, yB, statB = st['y01'].data_ptr(), st['stat01'].data_ptr(), ycat.data_ptr() + ycat.element_size() * cout, st['stat10'].data_ptr()
+                yf16 = 1 if ycat.dtype == torch.float16 else 0
+                if sync is None:
+                    _lib.check(L.gin_bn_act_bwd_pair(d.data_ptr(), cout, st['out_w'].data_ptr(), yA, cout, statA, bs01.data_ptr(), dy01_b.data_ptr(), cout,
+                                                     yB, 2 * cout, statB, bs10.data_ptr(), dycat_b.data_ptr() + 2 * cout, 2 * cout, yf16, ws.data_ptr(), B, lvl,
+                                                     cout, 1, _stream()), 'gin_bn_act_bwd_pair')
+                else:
+                    rec = _empty(L.gin_bn_sync_record_bytes(cout, 1) // 8, torch.float64, dev)
+                    _lib.check(L.gin_bn_sync_bwd_reduce_pair(d.data_ptr(), cout, st['out_w'].data_ptr(), yA, cout, statA, yB, 2 * cout, statB, yf16,
+                                                             rec.data_ptr(), ws.data_ptr(), B, lvl, cout, 1, _stream()), 'gin_bn_sync_bwd_reduce_pair')
+                    recs = _exchange(rec, sync)
+                    _lib.check(L.gin_bn_sync_bwd_final(recs.data_ptr(), sync[1], sync[2], cout, bs01.data_ptr(), bs10.data_ptr(), _stream()),
+                               'gin_bn_sync_bwd_final')
+                    _lib.check(L.gin_bn_bwd_apply_pair(d.data_ptr(), cout, st['out_w'].data_ptr(), yA, cout, statA, bs01.data_ptr(), dy01_b.data_ptr(), cout,
+                                                       yB, 2 * cout, statB, bs10.data_ptr(), dycat_b.data_ptr() + 2 * cout, 2 * cout, yf16, B, lvl, cout, 1,
+                                                       _stream()), 'gin_bn_bwd_apply_pair')
                 dW01 = _conv_wgrad(st['plan_b'], st['h_w'], dy01_b, B, cout, cout, out=_dest((blk.conv01.weight,), (cout, cout, 7)))
                 d_h = _conv_dgrad(st['plan_b'], dy01_b, st['pk01'], B, cout, cout, _P(lvl))
-                bs00, _ = _bn_bwd(d_h, st['h_w'], ycat, 0, 2 * cout, st['stat00'], B, lvl, cout, dycat_b, 0, 2 * cout)
+                bs00, _ = _bn_bwd(d_h, st['h_w'], ycat, 0, 2 * cout, st['stat00'], B, lvl, cout, dycat_b, 0, 2 * cout, sync=sync)
                 dWcat = _conv_wgrad(st['plan_a'], st['a_w'], dycat_b, B, cin, 2 * cout, out=_dest(_cat(blk), (2 * cout, cin, 7)))
                 d = _block_input_grad(st, dycat_b, B)
                 zero_b = zeros[:cout]
@@ -485,7 +576,7 @@ class _Chain(torch.autograd.Function):
                 n = 12
             elif st['kind'] == 'stem':
                 C = st['C']
-                bs, dy_f = _bn_bwd(d, st['out_w'], st['y'], 0, C, st['stat'], B, st['level'], C, want_f=True)
+                bs, dy_f = _bn_bwd(d, st['out_w'], st['y'], 0, C, st['stat'], B, st['level'], C, want_f=True, sync=sync)
                 dW, db, dx = _stem_bwd(st, dy_f, B, True, True, ctx.x_needs_grad)
                 grads[0:4] = [dW, db, bs[C:2 * C], bs[:C]]
                 n = 4
@@ -573,11 +664,11 @@ def _conv_affine(plan, xb, packed, B, cin, cout, level, scale, shift, relu_split
 
 
 def eval_pairs(mods):
-    """(BatchNorm2d, conv bias or None) of every BatchNorm of a chain, in the order infer_chain reads their constants; the stem's
+    """(BatchNorm, conv bias or None) of every BatchNorm of a chain, in the order infer_chain reads their constants; the stem's
     BatchNorm is applied by gin_bn_act_fwd to a map that already holds the conv bias."""
     pairs = []
     for m in mods:
-        if isinstance(m, torch.nn.BatchNorm2d):
+        if isinstance(m, _BN):
             pairs.append((m, None))
         elif _is_block(m):
             pairs += [(m.icobn00, m.conv00.bias), (m.icobn10, m.conv10.bias), (m.icobn01, m.conv01.bias)]
@@ -709,10 +800,10 @@ def run_frozen_chain(x, mods):
 
 
 def latent_supported(mu, logvar):
-    """The VAE's mu / logvar heads (IcoConvS2S stride 2 + BatchNorm2d, models.py _latent_head) in eval mode, without hooks."""
+    """The VAE's mu / logvar heads (IcoConvS2S stride 2 + BatchNorm, models.py _latent_head) in eval mode, without hooks."""
     for head in (mu, logvar):
         mods = list(head)
-        if len(mods) != 2 or not isinstance(mods[0], IcoConvS2S) or not isinstance(mods[1], torch.nn.BatchNorm2d):
+        if len(mods) != 2 or not isinstance(mods[0], IcoConvS2S) or not isinstance(mods[1], _BN):
             return False
         c, bn = mods
         if (c.stride != 2 or c.bias is None or getattr(c, 'impl', 0) != 0 or bn.training or not bn.affine or not bn.track_running_stats

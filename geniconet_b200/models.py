@@ -45,8 +45,8 @@ def set_fused(flag, head=None, inference=None, frozen=None):
 
 
 def _bn_modes(tops):
-    """The set of `training` flags of every BatchNorm2d inside the modules `tops`."""
-    return {m.training for t in tops for m in t.modules() if isinstance(m, torch.nn.BatchNorm2d)}
+    """The set of `training` flags of every BatchNorm2d or SyncBatchNorm inside the modules `tops`."""
+    return {m.training for t in tops for m in t.modules() if isinstance(m, _fused._BN)}
 
 
 def _route(mods, x, train_chain=True):
@@ -54,7 +54,8 @@ def _route(mods, x, train_chain=True):
     'train' (fused.run_chain), 'frozen' (fused.run_frozen_chain), or None (the caller runs the modules).  A chain needs a CUDA fp32 x,
     no forward (pre-)hook and no `impl` override inside, a supported module list, and every BatchNorm inside in the same mode.  With
     grad disabled that is the forward-only chain (when switched on); with grad enabled the BatchNorms decide: train mode -> the
-    training chain (unless train_chain is False: the split models never take it), eval mode -> the frozen chain (when switched on)."""
+    training chain (unless train_chain is False: the split models never take it), eval mode -> the frozen chain (when switched on).
+    SyncBatchNorm counts as BatchNorm; the training chain then synchronises the batch statistics (fused.sync_group)."""
     tops = [mods] if isinstance(mods, torch.nn.Module) else list(mods)
     mods = list(mods)
     if not (_FUSED and x.is_cuda and x.dtype == torch.float32):
@@ -64,7 +65,9 @@ def _route(mods, x, train_chain=True):
         return None
     modes = _bn_modes(tops)
     if not torch.is_grad_enabled():
-        return 'infer' if _INFER and len(modes) == 1 and _fused.chain_supported(mods) else None
+        # train-mode SyncBatchNorm that synchronises keeps the module path: the forward-only chain has no exchange
+        ok = _INFER and len(modes) == 1 and _fused.chain_supported(mods) and (modes == {False} or _fused.sync_group(mods) is None)
+        return 'infer' if ok else None
     if modes == {True}:
         return 'train' if train_chain and _fused.chain_supported(mods) else None
     return 'frozen' if _FROZEN and modes == {False} and _fused.frozen_supported(mods) else None

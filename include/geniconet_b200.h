@@ -197,6 +197,37 @@ size_t gin_bn_pair_ws_bytes(int C);
 int gin_bn_act_bwd_pair(const float* dout, int64_t ldg, const void* mask_b, const void* yA, int64_t ldA, const float* statA, float* bstatA,
                         void* dyA_b, int64_t ldoA, const void* yB, int64_t ldB, const float* statB, float* bstatB, void* dyB_b, int64_t ldoB,
                         int y_fp16, void* ws, int B, int level, int C, int relu_from_y, void* stream);
+/* Synchronised BatchNorm (torch.nn.SyncBatchNorm semantics over W ranks).  Each BatchNorm reduction is split at its fp64 total: a
+ * rank writes one fp64 record, the caller all-gathers the records of every rank into recs[W][record] (a copy), and the finals sum
+ * them in rank order 0..W-1.  With W = 1 every final is bit for bit the unsynchronised entry point's.  Records:
+ *   forward,  one BatchNorm: [sum y [C] | sum y^2 [C] | rows];
+ *   backward, one BatchNorm: [sum g [C] | sum g*yhat [C] | rows];
+ *   a pair (colB >= 0, statB / bstatB != NULL; the sibling BatchNorms of a residual block): A's record, then B's, one exchange.
+ * gin_bn_sync_record_bytes(C, pair): the size of one rank's record(s).  rows travels as a double (exact below 2^53). */
+size_t gin_bn_sync_record_bytes(int C, int pair);
+/* forward record from an fp32 map (ws: gin_bn_ws_bytes(C)), as gin_bn_stats sums it */
+int gin_bn_sync_stats_total(const float* y, int64_t ld, int64_t rows, int C, double* rec, void* ws, void* stream);
+/* forward record from per-CTA partials, as gin_bn_stats_from_parts (colB < 0) or gin_bn_stats_from_parts2 (colB >= 0: pair) sums them */
+int gin_bn_sync_stats_total_from_parts(const float* parts, int nparts, int64_t ld, int64_t rows, int C, int colA, int colB, double* rec, void* stream);
+/* stat[4][C] and the running statistics from recs[world][record] exactly as gin_bn_stats writes them, with the global row count
+ * (unbiased variance over it); statB == NULL: one BatchNorm, else a pair (the B arguments). */
+int gin_bn_sync_stats_final(const double* recs, int world, int C, const float* gammaA, const float* betaA, float epsA, float momentumA, float* rmeanA,
+                            float* rvarA, int64_t* nbtA, float* statA, const float* gammaB, const float* betaB, float epsB, float momentumB,
+                            float* rmeanB, float* rvarB, int64_t* nbtB, float* statB, void* stream);
+/* the reduce pass of gin_bn_act_bwd / gin_bn_act_bwd_pair, ending in this rank's backward record (ws as there) */
+int gin_bn_sync_bwd_reduce(const float* dout, int64_t ldg, const void* mask_b, const void* y, int64_t ld, int y_fp16, const float* stat, double* rec,
+                           void* ws, int B, int level, int C, int relu_from_y, void* stream);
+int gin_bn_sync_bwd_reduce_pair(const float* dout, int64_t ldg, const void* mask_b, const void* yA, int64_t ldA, const float* statA, const void* yB,
+                                int64_t ldB, const float* statB, int y_fp16, double* rec, void* ws, int B, int level, int C, int relu_from_y, void* stream);
+/* bstat[4][C] from recs[world][record]: dbeta, dgamma = rank `rank`'s own sums (as torch's SyncBatchNorm returns them; data-parallel
+ * averaging follows), mean(g), mean(g*yhat) over every rank.  bstatB == NULL: one BatchNorm, else a pair. */
+int gin_bn_sync_bwd_final(const double* recs, int world, int rank, int C, float* bstatA, float* bstatB, void* stream);
+/* the apply pass of gin_bn_act_bwd / gin_bn_act_bwd_pair from a finished bstat */
+int gin_bn_bwd_apply(const float* dout, int64_t ldg, const void* mask_b, const void* y, int64_t ld, int y_fp16, const float* stat, const float* bstat,
+                     void* dy_b, int64_t ldo, float* dy_f, int64_t ldf, int B, int level, int C, int relu_from_y, void* stream);
+int gin_bn_bwd_apply_pair(const float* dout, int64_t ldg, const void* mask_b, const void* yA, int64_t ldA, const float* statA, const float* bstatA,
+                          void* dyA_b, int64_t ldoA, const void* yB, int64_t ldB, const float* statB, const float* bstatB, void* dyB_b, int64_t ldoB,
+                          int y_fp16, int B, int level, int C, int relu_from_y, void* stream);
 /* IcoUpsampleS2S.forward whose result exists only as the next convolution's operand copy out_b = 16-bit [B*Pf + 2B][C] in the
  * forward operand format (upsample plan), plus (out_w, may be NULL) its bf16 twin for wgrad.  in: the fp32 coarse map
  * [B*Pc][C] (in_is_f32 = 1) or its forward-format operand copy [B*Pc + 2B][C] (0). */
